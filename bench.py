@@ -2,7 +2,7 @@
 """bench.py — filtered Gbases/s of the per-read filter/trim hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--config C] [--strong] [--reads R]
+                    [--config C] [--strong] [--reads R] [--dump-outputs DIR]
 
 One "step" = one pass of the whole hot path (K1 raw scan -> K3 adapter search -> K5 regions ->
 [K4] -> K1 clean scan) over the workload's batches.  Workload (`--config`, or TGSF_BENCH_CONFIG;
@@ -438,6 +438,43 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------------------
+# outputs of the timed path (--dump-outputs)
+# ------------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_SEED = 20261018
+READ_COLUMNS = ("sum_q", "status", "n_mid", "n_5p", "n_3p", "piece_begin", "n_pieces")
+PIECE_COLUMNS = ("sum_q", "read", "start", "len", "repeat_len", "status")
+
+
+def dump_outputs(out_dir: str, batch_ids, results, counters: np.ndarray, limit: int = DUMP_LIMIT_BYTES):
+    """What a caller of the timed path receives for one step, as float64 .npy files (every value is an integer below
+    2^53, so exactly):
+      batch<j>_reads.npy   one row per read of batch j: row index, then READ_COLUMNS (tgsf_read_result)
+      batch<j>_pieces.npy  one row per piece of batch j: row index, then PIECE_COLUMNS (tgsf_piece)
+      counters.npy         the QC counter block the step added (tgsf_counters: DropInfo, histograms, tables)
+    When the whole would exceed `limit` bytes, every per-row array keeps the same fraction of its rows, picked by a
+    generator with a fixed seed; the row index column says which rows they are."""
+    os.makedirs(out_dir, exist_ok=True)
+    tables = {}
+    for j, (reads, pieces) in zip(batch_ids, results):
+        tables[f"batch{j}_reads"] = (reads, READ_COLUMNS)
+        tables[f"batch{j}_pieces"] = (pieces, PIECE_COLUMNS)
+    row_bytes = sum(len(a) * (len(cols) + 1) * 8 for a, cols in tables.values())
+    frac = min(1.0, (limit - counters.size * 8) / max(row_bytes, 1))
+    for name, (a, cols) in tables.items():
+        rows = np.arange(len(a))
+        if frac < 1.0:
+            rng = np.random.default_rng([DUMP_SEED, len(a)])
+            rows = np.sort(rng.choice(len(a), int(len(a) * frac), replace=False))
+        out = np.empty((len(rows), len(cols) + 1), dtype=np.float64)
+        out[:, 0] = rows
+        for c, f in enumerate(cols, 1):
+            out[:, c] = a[f][rows]
+        np.save(os.path.join(out_dir, name + ".npy"), out)
+    np.save(os.path.join(out_dir, "counters.npy"), counters.astype(np.float64))
+
+
+# ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
 def main():
@@ -459,7 +496,11 @@ def main():
     ap.add_argument("--e2e-chunks", type=int, default=16)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-fed measurement (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (per-read results, pieces, QC counters) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
     if args.config not in CONFIG_READS:
         raise SystemExit(f"--config must be one of {sorted(CONFIG_READS)}")
@@ -586,13 +627,16 @@ def main():
         torch.cuda.synchronize()
     ar_ev = (torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True))
 
-    def step_resident(stage_acc):
-        """All local batches through the two slots; returns the step's device time in ms."""
+    def step_resident(stage_acc, keep=None):
+        """All local batches through the two slots; returns the step's device time in ms.  With a list as `keep`,
+        the (per-read results, pieces) of every batch are appended to it in batch order."""
         spans = []
         inflight = 0
 
         def retire():
-            eng.collect(want_results=False)
+            res = eng.collect(want_results=keep is not None)
+            if keep is not None:
+                keep.append(res)
             spans.append(eng.last_span())
             st = eng.last_stage_ms()
             for k in stage_acc:
@@ -775,17 +819,25 @@ def main():
     # ---- timed: resident
     launches0 = eng.launch_count()
     stage_sum = {k: 0.0 for k in _capi.STAGE_NAMES}
+    dump = args.dump_outputs is not None and rank == 0
+    last_results, cnt_before_last = [], None
     barrier()
     with ClockSampler(local_rank) as clk:
         wall0 = time.perf_counter()
         dev_ms = 0.0
-        for _ in range(args.steps):
-            dev_ms += step_resident(stage_sum)
+        for i in range(args.steps):
+            last = dump and i == args.steps - 1
+            if last:  # the counters accumulate over the steps: the last step's are the difference
+                cnt_before_last = eng.counters().flat.copy()
+            dev_ms += step_resident(stage_sum, last_results if last else None)
         barrier()
         wall_ms = (time.perf_counter() - wall0) * 1e3
     launches = eng.launch_count() - launches0
     clocks = clk.summary()
     cnt = eng.counters()
+    if dump:
+        dump_outputs(args.dump_outputs, [b.j for b in batches], last_results, cnt.flat - cnt_before_last)
+        del last_results
     # per-kernel times for the rooflines: one more pass with ONE batch in flight (stages of batches that overlap in
     # the two slots stretch each other, so their event times are not kernel times)
     # ... and with the end-window kernels on the batch's main stream (TGSF_FORK_ENDS=0: a second context), because the

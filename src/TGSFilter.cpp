@@ -541,6 +541,20 @@ int main(int argc, char **argv) {
     if (P.Infq == 0 && P.Outfq == 1) { cerr << "Error: Fasta format input file can't output fastq format file" << endl; return 1; }
     const bool has_qual = P.Infq == 1 || P.Infq == 2; // BAM/SAM records carry qualities (read_bam, T.cpp:1872-1916)
     const bool sambam = P.Infq == 2;
+#ifndef TGSF_HAVE_HTSLIB
+    if (sambam) { // CRAM is recognised by its content, as hts_open does; without htslib it cannot be decoded: fail loudly
+        char magic[4] = {0, 0, 0, 0};
+        if (FILE *f = fopen(P.InFile.c_str(), "rb")) {
+            if (fread(magic, 1, 4, f) != 4) magic[0] = 0;
+            fclose(f);
+        }
+        if (memcmp(magic, "CRAM", 4) == 0) {
+            cerr << "Error: CRAM input needs a build with htslib (make -C src HTS_DIR=<htslib prefix>); "
+                    "convert with `samtools fastq` or to BAM" << endl;
+            return 1;
+        }
+    }
+#endif
 
     // ---- pre-pass: read_fastx (T.cpp:949-982) + Get_qType (T.cpp:1042-1077) -----------------------
     int checkLen = std::max(std::max(P.EndLen, P.BCLen), 100);

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 import bench
@@ -35,6 +36,28 @@ def test_config_object_is_a_pure_function_of_the_command_line():
     a = bench.static_config(2, 200_000, False)
     assert a == bench.static_config(2, 200_000, False) and a != bench.static_config(2, 200_000, True)
     assert "config[1]" in a["workload"] and a["cli"] == "-x ont" and a["reads"] == 200_000
+
+
+def test_dump_outputs_writes_float64_and_samples_to_the_limit(tmp_path):
+    from tgsfilter_b200 import _capi
+    rng = np.random.default_rng(3)
+    reads = np.zeros(5000, dtype=_capi.READ_RESULT_DTYPE)
+    pieces = np.zeros(7000, dtype=_capi.PIECE_DTYPE)
+    reads["sum_q"] = rng.integers(0, 1 << 40, reads.size)
+    pieces["start"] = np.arange(pieces.size)
+    counters = np.arange(100, dtype=np.uint64)
+    bench.dump_outputs(str(tmp_path / "all"), [0], [(reads, pieces)], counters)
+    r = np.load(tmp_path / "all" / "batch0_reads.npy")
+    assert r.dtype == np.float64 and r.shape == (5000, 1 + len(bench.READ_COLUMNS))
+    assert np.array_equal(r[:, 1], reads["sum_q"].astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "all" / "counters.npy"), counters.astype(np.float64))
+    limit = 200_000
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), [0], [(reads, pieces)], counters, limit=limit)
+    assert sum(f.stat().st_size for f in (tmp_path / "s1").iterdir()) <= limit + 3 * 128  # + the .npy headers
+    p1, p2 = (np.load(tmp_path / d / "batch0_pieces.npy") for d in ("s1", "s2"))
+    assert 0 < len(p1) < pieces.size and np.array_equal(p1, p2)  # the same seeded sample every time
+    assert np.array_equal(p1[:, 0], p1[:, 3])  # row index column = the rows' own `start` here
 
 
 @pytest.mark.skipif(not ref_lib.available(), reason="oracle/_ref not present")
