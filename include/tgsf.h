@@ -97,13 +97,15 @@ typedef struct tgsf_piece {
     int32_t len;
     int32_t repeat_len; /* GetKmerCount result (T.cpp:1703-1753), -1 when MinRepeat == 0 */
     int32_t status;     /* TGSF_PIECE_* */
-    int32_t reserved;
+    int32_t contam_hits; /* windows whose canonical k-mer is in the contaminant set (tgsf_set_contaminants);
+                          * 0 without a set and for pieces that are not screened */
 } tgsf_piece;
 
 #define TGSF_PIECE_EMIT 0         /* becomes an output record */
 #define TGSF_PIECE_SHORT_REPEAT 1 /* DropInfo[15]/[16] (T.cpp:1982-1989) */
 #define TGSF_PIECE_LOWQ 2         /* DropInfo[13]/[14] (T.cpp:1995-2000) */
 #define TGSF_PIECE_QC_ONLY 3      /* --qc: region kept but nothing emitted (T.cpp:1976) */
+#define TGSF_PIECE_CONTAM 4       /* contaminant screen: hit share >= min_frac (tgsf_set_contaminants) */
 
 /* Layout (in uint64 words) of the cumulative counter block.  Every member is a sum, so blocks of
  * different GPUs combine with one allreduce(sum, u64).  [x][5] = {A,T,G,C,all} as in T.cpp:1462-1476. */
@@ -188,6 +190,21 @@ int tgsf_collect_gz(tgsf_ctx *ctx, uint8_t *blob, uint64_t blob_cap, uint64_t *b
  * only retire the batch (counters are still updated). */
 int tgsf_collect(tgsf_ctx *ctx, tgsf_read_result *reads, uint32_t n_reads, tgsf_piece *pieces,
                  uint32_t pieces_cap, uint32_t *n_pieces);
+/* Contaminant screen (an extension; the reference has none).  Installs on this context's device the set of every
+ * canonical k-mer (min of forward and reverse-complement code, A0 C1 G2 T3, 2 bits per base) of the records
+ * seq[offsets[i], offsets[i+1]), i < n_seqs (host buffers, offsets[0] == 0).  Bases are case-insensitive; a window
+ * with any other byte contributes nothing.  From the next batch on, every piece that is still TGSF_PIECE_EMIT after
+ * the repeat check (not with TGSF_FLAG_ONLY_QC) is screened: windows = len - k + 1, contam_hits = valid windows
+ * whose k-mer is in the set, and the piece becomes TGSF_PIECE_CONTAM iff windows >= 1 and
+ * contam_hits * 1000000 >= ppm * windows (u64), ppm = llround((double)min_frac * 1e6).  Contaminant pieces touch no
+ * counter; callers count them from the piece array.  k in [11, 31], ppm in [1, 1000000], otherwise TGSF_ERR_INVALID,
+ * as for a set without a valid k-mer; TGSF_ERR_STATE while a batch is outstanding; TGSF_ERR_NOMEM when the table
+ * (8 bytes x the next power of two >= 2 x set bytes) does not fit.  *n_kmers receives the number of distinct
+ * canonical k-mers.  A second call replaces the set; on error the previous set stays installed.  The screen's
+ * kernels are timed in TGSF_STAGE_KMER. */
+int tgsf_set_contaminants(tgsf_ctx *ctx, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs, int32_t k,
+                          float min_frac, uint64_t *n_kmers);
+
 /* Device time (ms, CUDA events on the slot's stream) of the batch retired by the last collect:
  * kernels only, and H2D+kernels+D2H. */
 int tgsf_last_timing(tgsf_ctx *ctx, float *kernel_ms, float *total_ms);
@@ -200,7 +217,7 @@ int tgsf_last_timing(tgsf_ctx *ctx, float *kernel_ms, float *total_ms);
 #define TGSF_STAGE_MID_SCAN 2    /* K3 k_mid_scan, all adapters (chunk table included) */
 #define TGSF_STAGE_RESOLVE 3     /* K3 k_mid_count + k_ends (start search, traceback, thresholds) */
 #define TGSF_STAGE_REGIONS 4     /* K3 k_mid_emit + K5 regions / piece compaction */
-#define TGSF_STAGE_KMER 5        /* K4 */
+#define TGSF_STAGE_KMER 5        /* K4 + the contaminant screen */
 #define TGSF_STAGE_CLEAN 6       /* K1 over the kept pieces + clean decisions + clean 5'/3' */
 int tgsf_last_stage_ms(tgsf_ctx *ctx, float *out, int n);
 

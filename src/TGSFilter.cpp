@@ -19,6 +19,7 @@
 #include <atomic>
 #include <cctype>
 #include <chrono>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -70,6 +71,9 @@ struct Params {
     bool OUTGZ = false;
     int compLevel = 6;
     int gpus = 1;                 // --gpus (extension; TGSF_GPUS env)
+    string ContamFile;            // --contam (extension): drop pieces that share k-mers with this FASTA
+    int ContamK = 17;             // --contam-k
+    float ContamFrac = 0.05f;     // --contam-frac
     uint64_t batch_bases = 64ull << 20; // bases per batch (TGSF_BATCH_MB)
 };
 
@@ -114,6 +118,10 @@ int usage() {
                  "   -c   <int>   compression level (0-9) for compressed output [6]\n"
                  "   -t   <int>   host threads for compressing/writing the output [16] (filtering runs on the GPU)\n"
                  "   --gpus <int> number of GPUs to shard batches over [1]\n"
+                 " Contaminant screen options:\n"
+                 "   --contam <str>        FASTA[.gz] of contaminant sequences; pieces sharing enough k-mers are discarded\n"
+                 "   --contam-k <int>      k-mer size of the contaminant screen, 11-31 [17]\n"
+                 "   --contam-frac <float> min fraction of a piece's k-mers found in the set to discard it [0.05]\n"
                  "   -h           show help [b200 host of v1.11]\n\n";
     return 1;
 }
@@ -182,11 +190,27 @@ int parse_cmd(int argc, char **argv, Params *P) {
         else if (flag == "f") { P->FastaOut = true; }
         else if (flag == "t") { if (!need()) return 1; P->n_thread = atoi(argv[i]); }
         else if (flag == "gpus") { if (!need()) return 1; P->gpus = std::max(1, atoi(argv[i])); }
+        else if (flag == "contam") { if (!need()) return 1; P->ContamFile = argv[i]; }
+        else if (flag == "contamk") { if (!need()) return 1; P->ContamK = atoi(argv[i]); }
+        else if (flag == "contamfrac") { if (!need()) return 1; P->ContamFrac = (float)atof(argv[i]); }
         else if (flag == "help" || flag == "h") { usage(); return 1; }
         else { cerr << "Error: UnKnow argument -" << flag << endl; return 1; }
     }
     if (P->InFile.empty()) { cerr << "Error: lack argument for the must: -i " << endl; exit(-1); }
     if (access(P->InFile.c_str(), 0) != 0) { cerr << "Error: Can't find this file for -i " << P->InFile << endl; exit(-1); }
+    if (P->ContamK < 11 || P->ContamK > 31) { cerr << "Error: --contam-k must be in [11,31]" << endl; exit(-1); }
+    const long long contam_ppm = llround((double)P->ContamFrac * 1e6); // as tgsf_set_contaminants computes it
+    if (!(P->ContamFrac == P->ContamFrac) || contam_ppm < 1 || contam_ppm > 1000000) {
+        cerr << "Error: --contam-frac must be in (0,1]" << endl;
+        exit(-1);
+    }
+    if (!P->ContamFile.empty()) {
+        if (P->OnlyQC || P->ONLYAD || !P->Filter) {
+            cerr << "Error: --contam screens filtered reads and cannot be combined with --qc, -A or -F" << endl;
+            exit(-1);
+        }
+        if (access(P->ContamFile.c_str(), R_OK) != 0) { cerr << "Error: Can't find this file for --contam " << P->ContamFile << endl; exit(-1); }
+    }
     if (P->OnlyQC) P->Filter = false;
     if (P->Filter) {
         if (P->readType.empty()) { cerr << "Error: lack argument for the must: -x " << endl; exit(-1); }
@@ -212,6 +236,37 @@ int parse_cmd(int argc, char **argv, Params *P) {
         exit(-1);
     }
     return 0;
+}
+
+// Contaminant FASTA (multi-line, plain or gzip): records back to back in seq, offs[i]..offs[i+1].
+bool load_contam_fasta(const string &path, std::vector<uint8_t> &seq, std::vector<uint64_t> &offs) {
+    gzFile f = gzopen(path.c_str(), "rb");
+    if (!f) return false;
+    gzbuffer(f, 1 << 20);
+    seq.clear();
+    offs.assign(1, 0);
+    std::vector<char> line(1 << 16);
+    bool in_rec = false, at_bol = true, header = false;
+    int n;
+    while ((n = gzread(f, line.data(), (unsigned)line.size())) > 0) {
+        for (int i = 0; i < n; ++i) {
+            const char ch = line[(size_t)i];
+            if (ch == '\n') { at_bol = true; header = false; continue; }
+            if (at_bol && ch == '>') {
+                if (in_rec) offs.push_back(seq.size());
+                in_rec = true;
+                header = true;
+            } else if (!header && ch != '\r' && ch != ' ' && ch != '\t') {
+                in_rec = true;
+                seq.push_back((uint8_t)ch);
+            }
+            at_bol = false;
+        }
+    }
+    const bool ok = n == 0;
+    gzclose(f);
+    if (in_rec) offs.push_back(seq.size());
+    return ok;
 }
 
 string file_ext(const string &p) { size_t d = p.rfind('.'); return d == string::npos ? "" : p.substr(d + 1); }
@@ -520,6 +575,12 @@ int main(int argc, char **argv) {
     const bool clean_exit = getenv("TGSF_CLEAN_EXIT") != nullptr; // destroy contexts / free buffers before returning
     if (const char *e = getenv("TGSF_GPUS")) P.gpus = std::max(1, atoi(e));
     if (parse_cmd(argc, argv, &P) == 1) return 1;
+    std::vector<uint8_t> contam_seq;
+    std::vector<uint64_t> contam_offs;
+    if (!P.ContamFile.empty()) {
+        if (!load_contam_fasta(P.ContamFile, contam_seq, contam_offs)) { cerr << "Error: Failed to read --contam " << P.ContamFile << endl; return 1; }
+        if (contam_offs.size() < 2 || contam_seq.empty()) { cerr << "Error: no sequence in --contam " << P.ContamFile << endl; return 1; }
+    }
     for (int i = 0; i < 256; i++) g_comp[i] = 'N';
     const char *pairs[] = {"AT", "GC", "CG", "TA", "at", "gc", "cg", "ta", "MK", "RY", "WW", "SS", "YR", "KM",
                            "mk", "ry", "ww", "ss", "yr", "km"};
@@ -770,6 +831,7 @@ int main(int argc, char **argv) {
     }
 
     uint64_t cleanNum = 0, cleanBases = 0, rawNum = 0, rawBases = 0;
+    uint64_t contamNum = 0, contamBases = 0; // pieces discarded by the contaminant screen (--contam)
     std::vector<int> rawLens, cleanLens;       // T.cpp:1794
     report::Side rawSide, cleanSide;
     string tmpPath;
@@ -816,6 +878,15 @@ int main(int argc, char **argv) {
     }
     for (int g = 0; g < P.gpus; g++)
         if (tgsf_create(g % n_dev, &tp, &ctx[(size_t)g]) != TGSF_OK) die_tgsf("tgsf_create");
+    if (!P.ContamFile.empty()) {
+        uint64_t n_kmers = 0;
+        for (int g = 0; g < P.gpus; g++)
+            if (tgsf_set_contaminants(ctx[(size_t)g], contam_seq.data(), contam_offs.data(), (uint32_t)(contam_offs.size() - 1),
+                                      P.ContamK, P.ContamFrac, &n_kmers) != TGSF_OK)
+                die_tgsf("tgsf_set_contaminants");
+        cerr << "INFO: " << n_kmers << " distinct " << P.ContamK << "-mers loaded from " << P.ContamFile << "." << endl;
+        std::vector<uint8_t>().swap(contam_seq);
+    }
 
     tlog("tgsf_create", T_ph.lap());
     // ---- main pass -----------------------------------------------------------------------------------
@@ -926,6 +997,7 @@ int main(int argc, char **argv) {
             for (size_t pi = 0; pi < job->pieces.size(); ++pi) { // T.cpp:1976-2059
                 const tgsf_piece &p = job->pieces[pi];
                 if ((uint32_t)p.read != last) { last = (uint32_t)p.read; pass = 1; }
+                if (p.status == TGSF_PIECE_CONTAM) { contamNum++; contamBases += (uint64_t)p.len; }
                 if (p.status != TGSF_PIECE_EMIT) continue;
                 emits.push_back(Emit{last, (uint32_t)p.start, (uint32_t)p.len, pass, (uint32_t)pi});
                 pass++;
@@ -1376,6 +1448,8 @@ int main(int argc, char **argv) {
         cerr << "INFO: " << D[13] << " reads were discarded with " << D[14] << " bases due to low quality after split." << endl;
         if (P.MinRepeat > 0)
             cerr << "INFO: " << D[15] << " reads were discarded with " << D[16] << " bases due to short repeat length." << endl;
+        if (!P.ContamFile.empty())
+            cerr << "INFO: " << contamNum << " reads were discarded with " << contamBases << " bases as contaminant." << endl;
         cerr << "INFO: " << cleanNum << " reads with a total of " << cleanBases << " bases after filtering." << endl;
         if (!P.Downsample && !P.OutFile.empty()) cerr << "INFO: Filtered reads were written to: " << P.OutFile << "." << endl;
     }

@@ -26,7 +26,7 @@ FLAG_GZ_BLOCKS = 8
 FLAG_GZ_FASTA = 16
 
 READ_EVALUATED, READ_LOWQ, READ_EMPTY = 0, 1, 2
-PIECE_EMIT, PIECE_SHORT_REPEAT, PIECE_LOWQ, PIECE_QC_ONLY = 0, 1, 2, 3
+PIECE_EMIT, PIECE_SHORT_REPEAT, PIECE_LOWQ, PIECE_QC_ONLY, PIECE_CONTAM = 0, 1, 2, 3, 4
 
 N_STAGES = 7
 STAGE_NAMES = ("raw_scan", "raw_final", "mid_scan", "resolve", "regions", "kmer", "clean")
@@ -83,7 +83,7 @@ class Piece(C.Structure):
         ("len", C.c_int32),
         ("repeat_len", C.c_int32),
         ("status", C.c_int32),
-        ("reserved", C.c_int32),
+        ("contam_hits", C.c_int32),
     ]
 
 
@@ -105,7 +105,7 @@ class AlignResult(C.Structure):
 READ_RESULT_DTYPE = [("sum_q", "<u8"), ("status", "<i4"), ("n_mid", "<i4"), ("n_5p", "<i4"),
                      ("n_3p", "<i4"), ("piece_begin", "<i4"), ("n_pieces", "<i4")]
 PIECE_DTYPE = [("sum_q", "<u8"), ("read", "<i4"), ("start", "<i4"), ("len", "<i4"),
-               ("repeat_len", "<i4"), ("status", "<i4"), ("reserved", "<i4")]
+               ("repeat_len", "<i4"), ("status", "<i4"), ("contam_hits", "<i4")]
 ALIGN_RESULT_DTYPE = [("edit_distance", "<i4"), ("n_locations", "<i4"), ("align_len", "<i4"),
                       ("first_start", "<i4"), ("first_end", "<i4"), ("last_start", "<i4"),
                       ("last_end", "<i4"), ("loc_hash", "<u4")]
@@ -115,7 +115,7 @@ EXPORTED_SYMBOLS = (
     "tgsf_version", "tgsf_last_error", "tgsf_create", "tgsf_destroy", "tgsf_device_count", "tgsf_host_alloc",
     "tgsf_host_free", "tgsf_submit", "tgsf_submit_packed", "tgsf_pack_bases", "tgsf_submit_device", "tgsf_collect", "tgsf_collect_gz", "tgsf_last_timing", "tgsf_last_span", "tgsf_last_stage_ms",
     "tgsf_counter_layout_get", "tgsf_counters", "tgsf_counters_reset", "tgsf_counters_device",
-    "tgsf_launch_count", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw",
+    "tgsf_launch_count", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw", "tgsf_set_contaminants",
 )
 
 _lib = None
@@ -161,6 +161,7 @@ def load() -> C.CDLL:
                                  C.POINTER(C.c_char_p), C.POINTER(C.c_int32), C.c_int32, C.c_float,
                                  vp, vp, vp, vp]
     lib.tgsf_align_hw.argtypes = [C.c_int, u8p, vp, u8p, vp, vp, C.c_uint32, vp]
+    lib.tgsf_set_contaminants.argtypes = [vp, u8p, u64p, C.c_uint32, C.c_int32, C.c_float, C.POINTER(C.c_uint64)]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)
         if fn.restype is C.c_int and name not in ("tgsf_version", "tgsf_last_error",

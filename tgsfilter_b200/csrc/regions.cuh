@@ -214,7 +214,7 @@ __global__ void k_place_pieces(const TmpPiece *__restrict__ tmp, const u32 *__re
     p.len = t.len;
     p.repeat_len = -1;
     p.status = only_qc ? TGSF_PIECE_QC_ONLY : TGSF_PIECE_EMIT;
-    p.reserved = 0;
+    p.contam_hits = 0;
     pieces[piece_begin[t.read] + (u32)t.idx] = p;
 }
 

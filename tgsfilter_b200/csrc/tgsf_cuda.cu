@@ -14,6 +14,7 @@
 
 #include "adapters.cuh"
 #include "common.cuh"
+#include "contam.cuh"
 #include "kmer.cuh"
 #include "kmer16.cuh"
 #include "gzenc.cuh"
@@ -223,12 +224,24 @@ struct Slot {
     int chunk_shift = MID_CHUNK_SHIFT_MIN;
     DBuf best_mid, mid_n, mid_off, end_n, end_pos, pool, sortbuf, tmp, pieces, res, header;
     DBuf scan_tmp, kmer_bitmaps, kmer_long_list, mid_work, gz_blob, gz_spans;
+    DBuf contam_cnt, contam_off, contam_chunks; // contaminant screen (only with a set installed)
     Scratch scratch, scratch2; // traceback stores: main stream (k_mid_count) / side stream (k_ends)
     u32 pool_cap = 0, pieces_cap = 0, chunks_cap = 0, tiles_cap = 0;
     // host results
     HBuf h_res, h_pieces, h_header;
     u32 h_pieces_copied = 0;
     float kernel_ms = 0, total_ms = 0;
+};
+
+// Contaminant k-mer set (tgsf_set_contaminants).
+struct ContamSet {
+    DBuf table, pf_bits; // pf_bits: prefilter bitmap, only for sets of <= CONTAM_PF_MAX_KEYS keys
+    u64 mask = 0;        // table capacity - 1
+    u64 n_keys = 0;
+    u64 ppm = 0;
+    int k = 0;
+    bool installed() const { return table.p != nullptr; }
+    void release() { table.release(); pf_bits.release(); n_keys = 0; }
 };
 
 }  // namespace
@@ -238,6 +251,7 @@ struct tgsf_ctx {
     int sm_count = TGSF_SM_COUNT_FALLBACK;
     DevParams P{};
     AdapterSet ads;
+    ContamSet contam;
     DBuf counters;
     std::vector<Slot> slots;
     u32 head = 0, tail = 0, outstanding = 0; // ring: submit at head, collect at tail
@@ -302,7 +316,8 @@ void slot_release(Slot &s) {
                     &s.seg_flag, &s.tile_cnt, &s.tile_off, &s.tiles, &s.read_active, &s.piece_cnt,
                     &s.piece_begin, &s.chunk_cnt, &s.chunk_off, &s.chunks, &s.chunk_min, &s.chunk_hits, &s.chunk_first, &s.chunk_perm, &s.chunk_hist,
                     &s.best_mid, &s.mid_n, &s.mid_off, &s.end_n, &s.end_pos, &s.pool, &s.sortbuf,
-                    &s.tmp, &s.pieces, &s.res, &s.header, &s.scan_tmp, &s.kmer_bitmaps, &s.kmer_long_list, &s.mid_work, &s.gz_blob, &s.gz_spans, &s.scratch.buf, &s.scratch2.buf};
+                    &s.tmp, &s.pieces, &s.res, &s.header, &s.scan_tmp, &s.kmer_bitmaps, &s.kmer_long_list, &s.mid_work, &s.gz_blob, &s.gz_spans, &s.scratch.buf, &s.scratch2.buf,
+                    &s.contam_cnt, &s.contam_off, &s.contam_chunks};
     for (DBuf *b : bufs) b->release();
     s.h_res.release();
     s.h_pieces.release();
@@ -639,6 +654,40 @@ int launch_head(tgsf_ctx *c, Slot &s) {
     return check_launch("head");
 }
 
+// Contaminant screen over the pieces still emitted after K4; writes piece fields only.
+int launch_contam(tgsf_ctx *c, Slot &s) {
+    cudaStream_t st = s.stream;
+    const ContamSet &cs = c->contam;
+    DevHeader *H = s.header.as<DevHeader>();
+    const u32 cap = s.pieces_cap;
+    // pieces are disjoint parts of the reads: at most n_bases / CHUNK full chunks plus one partial chunk per piece
+    const size_t chunks_cap = (size_t)(s.n_bases / CONTAM_CHUNK) + cap + 16;
+    TRY(s.contam_cnt.ensure((size_t)cap * sizeof(u32)));
+    TRY(s.contam_off.ensure(((size_t)cap + 1) * sizeof(u32)));
+    TRY(s.contam_chunks.ensure(chunks_cap * sizeof(ContamChunk)));
+    k_contam_count<<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap, cs.k,
+                                                   s.contam_cnt.as<u32>(), &H->status);
+    c->launches++;
+    TRY(exclusive_scan(c, st, s.contam_cnt.as<u32>(), s.contam_off.as<u32>(), cap, s.scan_tmp.as<u32>(),
+                       s.scan_tmp.cap / sizeof(u32)));
+    k_contam_fill<<<cdiv(cap, 256), 256, 0, st>>>(s.B, s.pieces.as<tgsf_piece>(), s.contam_off.as<u32>(), cap, cs.k,
+                                                  s.contam_chunks.as<ContamChunk>());
+    c->launches++;
+    if (cs.pf_bits.p)
+        k_contam_screen<true><<<c->sm_count, CONTAM_THREADS, CONTAM_PF_SMEM_BYTES, st>>>(
+            s.B.bases, s.contam_chunks.as<ContamChunk>(), s.contam_off.as<u32>() + cap, cs.k, cs.table.as<u64>(), cs.mask,
+            cs.pf_bits.as<u32>(), s.pieces.as<tgsf_piece>(), &H->status);
+    else
+        k_contam_screen<false><<<c->sm_count * 4, CONTAM_THREADS, 0, st>>>(
+            s.B.bases, s.contam_chunks.as<ContamChunk>(), s.contam_off.as<u32>() + cap, cs.k, cs.table.as<u64>(), cs.mask,
+            nullptr, s.pieces.as<tgsf_piece>(), &H->status);
+    c->launches++;
+    k_contam_decide<<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap, cs.k, cs.ppm,
+                                                    &H->status);
+    c->launches++;
+    return check_launch("contam");
+}
+
 // From the region pool onwards; re-runnable after a pool overflow (touches no counter before the
 // overflow check has passed).
 int launch_tail(tgsf_ctx *c, Slot &s) {
@@ -740,6 +789,7 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
                                                                             &H->tmp_cursor, C, &H->status, nullptr);
             c->launches++;
         }
+        if (c->contam.installed()) TRY(launch_contam(c, s));
         CU(cudaEventRecord(s.ev_stage[6], st));
         // clean pass over the kept pieces (T.cpp:1991-2009); piece count is device-side, the
         // kernels are launched over the capacity and bound themselves by the header.
@@ -912,6 +962,7 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
         cudaError_t e4 = cudaFuncSetAttribute(k_kmer<u64>, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SMEM_BYTES);
         if (e4 == cudaSuccess) e4 = cudaFuncSetAttribute(k_kmer_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SB_SMEM_BYTES);
         if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_kmer_tag16, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER16_SMEM_BYTES);
+        if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_contam_screen<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, CONTAM_PF_SMEM_BYTES);
         if (e3 == cudaSuccess) {
             int occ = 0;
             if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_kmer_tag16, KMER16_THREADS, KMER16_SMEM_BYTES) == cudaSuccess && occ >= 1)
@@ -937,8 +988,79 @@ int tgsf_destroy(tgsf_ctx *c) {
     for (auto &s : c->slots) slot_release(s);
     if (c->ev_epoch) cudaEventDestroy(c->ev_epoch);
     c->ads.release();
+    c->contam.release();
     c->counters.release();
     delete c;
+    return TGSF_OK;
+}
+
+int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs, int32_t k,
+                          float min_frac, uint64_t *n_kmers) {
+    if (!c || !offsets || !n_kmers || n_seqs == 0) { set_err("tgsf_set_contaminants: missing argument"); return TGSF_ERR_INVALID; }
+    if (c->outstanding) { set_err("tgsf_set_contaminants with %u batch(es) outstanding", c->outstanding); return TGSF_ERR_STATE; }
+    if (k < CONTAM_K_MIN || k > CONTAM_K_MAX) { set_err("contaminant k must be in [%d,%d], got %d", CONTAM_K_MIN, CONTAM_K_MAX, k); return TGSF_ERR_INVALID; }
+    const double fd = (double)min_frac;
+    const long long ppm = fd == fd && fd >= 0.0 && fd <= 2.0 ? llround(fd * 1e6) : -1;
+    if (ppm < 1 || ppm > 1000000) { set_err("contaminant min_frac must give ppm in [1,1000000], got %g", fd); return TGSF_ERR_INVALID; }
+    if (offsets[0] != 0) { set_err("contaminant offsets[0] must be 0"); return TGSF_ERR_INVALID; }
+    for (uint32_t i = 0; i < n_seqs; ++i)
+        if (offsets[i + 1] < offsets[i]) { set_err("contaminant offsets not ascending at %u", i); return TGSF_ERR_INVALID; }
+    const u64 n_bytes = offsets[n_seqs];
+    if (n_bytes < (u64)k || !seq) { set_err("contaminant set has no valid %d-mer", k); return TGSF_ERR_INVALID; }
+    if (n_bytes > (1ull << 36)) { set_err("contaminant set of %llu bytes is too large", (unsigned long long)n_bytes); return TGSF_ERR_NOMEM; }
+    CU(cudaSetDevice(c->device));
+    // distinct keys <= windows < n_bytes, so a capacity >= 2 x n_bytes keeps the load <= 0.5
+    u64 cap = 1024;
+    while (cap < 2 * n_bytes) cap <<= 1;
+    cudaStream_t st = c->slots[0].stream;
+    ContamSet next;
+    DBuf d_seq, d_off, d_cnt;
+    auto build = [&]() -> int {
+        TRY(next.table.ensure(cap * sizeof(u64)));
+        TRY(d_seq.ensure(n_bytes));
+        TRY(d_off.ensure(((size_t)n_seqs + 1) * sizeof(u64)));
+        TRY(d_cnt.ensure(sizeof(unsigned long long)));
+        CU(cudaMemsetAsync(next.table.p, 0xFF, cap * sizeof(u64), st));
+        CU(cudaMemsetAsync(d_cnt.p, 0, sizeof(unsigned long long), st));
+        CU(cudaMemcpyAsync(d_seq.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n_seqs + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
+        const u64 threads = (n_bytes + CONTAM_BUILD_SEG - 1) / CONTAM_BUILD_SEG;
+        const u32 grid = (u32)std::min<u64>((threads + 255) / 256, (u64)c->sm_count * 16);
+        k_contam_build<<<grid, 256, 0, st>>>(d_seq.as<uint8_t>(), d_off.as<u64>(), n_seqs, k, next.table.as<u64>(),
+                                             cap - 1, d_cnt.as<unsigned long long>());
+        c->launches++;
+        TRY(check_launch("k_contam_build"));
+        unsigned long long n = 0;
+        CU(cudaMemcpyAsync(&n, d_cnt.p, sizeof(n), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        next.n_keys = n;
+        if (n == 0) { set_err("contaminant set has no valid %d-mer", k); return TGSF_ERR_INVALID; }
+        if (n <= CONTAM_PF_MAX_KEYS) {
+            TRY(next.pf_bits.ensure(CONTAM_PF_SMEM_BYTES));
+            CU(cudaMemsetAsync(next.pf_bits.p, 0, CONTAM_PF_SMEM_BYTES, st));
+            k_contam_bitmap<<<(u32)std::min<u64>(cap / 256 + 1, (u64)c->sm_count * 8), 256, 0, st>>>(
+                next.table.as<u64>(), cap, next.pf_bits.as<u32>());
+            c->launches++;
+            TRY(check_launch("k_contam_bitmap"));
+            CU(cudaStreamSynchronize(st));
+        }
+        return TGSF_OK;
+    };
+    const int rc = build();
+    d_seq.release();
+    d_off.release();
+    d_cnt.release();
+    if (rc != TGSF_OK) {
+        next.release();
+        return rc;
+    }
+    next.mask = cap - 1;
+    next.ppm = (u64)ppm;
+    next.k = k;
+    c->contam.release();
+    c->contam = next; // takes over the buffers
+    next.table.p = next.pf_bits.p = nullptr;
+    *n_kmers = c->contam.n_keys;
     return TGSF_OK;
 }
 

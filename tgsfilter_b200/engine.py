@@ -73,6 +73,19 @@ class FilterEngine:
         except Exception:
             pass
 
+    # -- contaminant screen ---------------------------------------------------------------------
+    def set_contaminants(self, seqs, k: int = 17, min_frac: float = 0.05) -> int:
+        """tgsf_set_contaminants: screen every later batch against the canonical k-mers of ``seqs``
+        (bytes / str records).  Returns the number of distinct canonical k-mers."""
+        recs = [s.encode() if isinstance(s, str) else bytes(s) for s in seqs]
+        offs = np.zeros(len(recs) + 1, dtype=np.uint64)
+        np.cumsum([len(r) for r in recs], out=offs[1:])
+        buf = np.frombuffer(b"".join(recs) + b"\0", dtype=np.uint8)
+        n = C.c_uint64(0)
+        _capi.check(self._lib.tgsf_set_contaminants(self._ctx, buf.ctypes.data, offs.ctypes.data, len(recs), k,
+                                                     min_frac, C.byref(n)), "tgsf_set_contaminants")
+        return int(n.value)
+
     # -- batches --------------------------------------------------------------------------------
     def submit(self, batch) -> None:
         bases = np.ascontiguousarray(batch.bases, dtype=np.uint8)

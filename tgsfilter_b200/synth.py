@@ -236,3 +236,70 @@ def config_params(config: int) -> FilterParams:
         raise ValueError(config)
     p.head_trim = p.tail_trim = 0
     return p
+
+
+# ---- contaminant sets (tgsf_set_contaminants) --------------------------------------------------------
+def make_contaminant(length: int, seed: int = SEED0 + 100) -> bytes:
+    """A random uppercase contaminant genome of ``length`` bases (e.g. 48_502 for a lambda-sized set)."""
+    return _ACGT[np.random.default_rng(seed).integers(0, 4, length, dtype=np.uint8)].tobytes()
+
+
+_COMP = np.zeros(256, dtype=np.uint8)
+_COMP[np.frombuffer(b"ACGT", dtype=np.uint8)] = np.frombuffer(b"TGCA", dtype=np.uint8)
+
+
+def mutate_array(seq: np.ndarray, err: float, rng: np.random.Generator) -> np.ndarray:
+    """``mutate`` on a uint8 array, vectorised: substitutions, insertions and deletions at err / 3 each."""
+    r = rng.random(len(seq))
+    sub = r < err / 3
+    ins = (r >= err / 3) & (r < 2 * err / 3)
+    keep = (r >= err) | sub | ins  # err * 2/3 <= r < err: deleted
+    out = seq.copy()
+    out[sub] = _ACGT[rng.integers(0, 4, int(sub.sum()), dtype=np.uint8)]
+    reps = keep.astype(np.int64) + ins  # an insertion takes a second slot after its base
+    res = np.repeat(out, reps)
+    # the second slot of every insertion becomes a random base
+    ins_pos = np.cumsum(reps)[ins] - 1
+    res[ins_pos] = _ACGT[rng.integers(0, 4, len(ins_pos), dtype=np.uint8)]
+    return res
+
+
+def contaminant_read(genome: bytes, length: int, err: float, rng: np.random.Generator) -> np.ndarray:
+    """``length`` bases drawn from a random position and strand of the (circular) genome, with errors at
+    rate ``err``."""
+    g = np.frombuffer(genome, dtype=np.uint8)
+    want = length + length // 8 + 64  # room for net deletions
+    start = int(rng.integers(0, len(g)))
+    seg = np.take(g, np.arange(start, start + want) % len(g))
+    if rng.random() < 0.5:
+        seg = _COMP[seg[::-1]]
+    out = mutate_array(seg, err, rng)
+    while len(out) < length:  # pragma: no cover - only at extreme deletion rates
+        out = np.concatenate([out, mutate_array(seg, err, rng)])
+    return out[:length]
+
+
+def mix_contaminants(batch: ReadBatch, genome: bytes, frac: float, err: float, *, chimeras: float = 0.0,
+                     chimera_share=(0.3, 0.6), chimera_err: Optional[float] = None, seed: int = SEED0 + 101):
+    """Copy of a ``make_config`` batch in which a fraction ``frac`` of the reads is replaced by reads drawn
+    from ``genome`` (same lengths, so qualities and offsets stay), and a further fraction ``chimeras`` carries
+    one contaminant segment covering a share in ``chimera_share`` of the read at error rate ``chimera_err``
+    (default ``err``).  Returns (batch, planted read indices, chimera read indices)."""
+    rng = np.random.default_rng(seed)
+    bases = batch.bases.copy()
+    u = rng.random(batch.n_reads)
+    planted = np.nonzero(u < frac)[0]
+    chim = np.nonzero((u >= frac) & (u < frac + chimeras))[0]
+    off = batch.offsets.astype(np.int64)
+    for r in planted:
+        s, e = int(off[r]), int(off[r + 1])
+        bases[s:e] = contaminant_read(genome, e - s, err, rng)
+    cerr = err if chimera_err is None else chimera_err
+    for r in chim:
+        s, e = int(off[r]), int(off[r + 1])
+        n = int(round((e - s) * rng.uniform(*chimera_share)))
+        if n < 1:
+            continue
+        pos = s + int(rng.integers(0, e - s - n + 1))
+        bases[pos:pos + n] = contaminant_read(genome, n, cerr, rng)
+    return ReadBatch(bases, batch.quals, batch.offsets, batch.names), planted, chim
