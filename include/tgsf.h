@@ -241,6 +241,11 @@ int tgsf_counters_device(tgsf_ctx *ctx, void **d_ptr, uint32_t *n_u64);
 int tgsf_allreduce(tgsf_ctx **ctxs, int n);
 /* Number of kernels launched by this context since create (bench.py's gpu_launches). */
 uint64_t tgsf_launch_count(const tgsf_ctx *ctx);
+/* The SM count every grid of this context is sized by (the device's, or TGSF_SM_COUNT=n at create,
+ * clamped to [1, device SM count]) and the middle-scan chunk shift (log2 of the chunk length in
+ * bases, chosen per batch from its size and that SM count) of the last collected batch (0 before
+ * the first).  Lets tests check which launch regime a batch ran in. */
+int tgsf_launch_shape(const tgsf_ctx *ctx, int32_t *sm_count, int32_t *last_chunk_shift);
 
 /* Replaces: the compute of the pre-pass, CheckBaseContent's counting loop (T.cpp:1080-1095) and
  * adapterSearch's edlib loop (T.cpp:1156-1176), for both read ends.  ends5p / ends3p: n rows of

@@ -16,9 +16,10 @@ from tgsfilter_b200.params import ADAPTER_LIB, FilterParams, rev_comp
 pytestmark = pytest.mark.gpu
 
 
-def _compare(params, batch, n_batches=1):
-    """Engine vs oracle: per-read results, pieces, all counters."""
-    o_reads, o_pieces, o_cnt = oracle_lib.run(params, batch)
+def _compare(params, batch, n_batches=1, oracle=None, on_engine=None):
+    """Engine vs oracle: per-read results, pieces, all counters.  ``oracle``: the oracle's (reads, pieces,
+    counters) for this input if already computed; ``on_engine(eng)`` is called after the last collect."""
+    o_reads, o_pieces, o_cnt = oracle if oracle is not None else oracle_lib.run(params, batch)
     with FilterEngine(params) as eng:
         if n_batches == 1:
             reads, pieces = eng.run(batch)
@@ -47,6 +48,8 @@ def _compare(params, batch, n_batches=1):
                 rb += len(r)
         cnt = eng.counters().flat
         assert eng.launch_count() > 0
+        if on_engine is not None:
+            on_engine(eng)
     for f in reads.dtype.names:
         np.testing.assert_array_equal(reads[f], o_reads[f], err_msg=f"reads.{f}")
     assert len(pieces) == len(o_pieces)
@@ -202,6 +205,12 @@ def test_qc_only_mode():
 def test_region_pool_overflow_is_retried():
     # -M 10 / -S 0.8 on low-complexity reads: every read has hundreds of equal-score middle
     # locations, far beyond the initial pool; collect() must grow the pool and re-run the tail.
+    reads, _, _ = _compare(*_pool_overflow_case())
+    assert int(reads["n_mid"].sum()) > 65536
+
+
+def _pool_overflow_case():
+    """(params, batch) whose middle locations overflow the initial region pool of 65 536."""
     rng = np.random.default_rng(8)
     ad = b"ACACACACACACACACACACAC"
     seqs, quals = [], []
@@ -212,8 +221,7 @@ def test_region_pool_overflow_is_retried():
     batch = synth.pack_reads(seqs, quals)
     params = FilterParams(min_len=100, min_q=1.0, head_trim=0, tail_trim=0, mid_match_len=10,
                           extra_len=0, adapters=[ad]).apply_read_type("ont")
-    reads, _, _ = _compare(params, batch)
-    assert int(reads["n_mid"].sum()) > 65536
+    return params, batch
 
 
 def test_submit_device_resident_inputs():
@@ -462,6 +470,11 @@ def test_tgsf_allreduce_sums_context_blocks():
 def test_randomised_parameters_vs_oracle(seed):
     """Parameter fuzz: adapter sets with mixed word counts, every threshold, both k-mer key widths,
     the wide (global-atomic) 5'/3' tables, FASTA input, discard, tiny and huge trims."""
+    _compare(*_fuzz_case(seed))
+
+
+def _fuzz_case(seed):
+    """(params, batch) of test_randomised_parameters_vs_oracle for one seed."""
     rng = np.random.default_rng(1000 + seed)
     acgt = np.frombuffer(b"ACGT", dtype=np.uint8)
 
@@ -504,7 +517,7 @@ def test_randomised_parameters_vs_oracle(seed):
         extra_len=int(rng.choice([0, 50, 200])), end_sim=end_sim, mid_sim=mid_sim,
         kmer=int(rng.choice([5, 9, 11, 12, 13, 15, 16, 21, 31])), min_repeat=int(rng.choice([0, 0, 3, 30, 300])),
         qtype=0 if fasta else 33, discard=bool(rng.random() < 0.3), adapters=ads, max_read_len=10000)
-    _compare(params, batch)
+    return params, batch
 
 
 def test_packed_2bit_submit_is_byte_identical():

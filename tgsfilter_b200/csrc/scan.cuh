@@ -11,6 +11,12 @@
 // stride of 25 words: bank-conflict free), classifies 4 bases per 32-bit word with SWAR masks and
 // accumulates counts / quality sums with dp4a.  Bins below SCAN_SMEM_BINS are privatised per CTA in
 // shared memory and flushed once; deeper bins (reads > 102 kb) go to L2 atomics.
+//
+// The privatised quality sums are 32-bit when no CTA can reach 2^31 in one bin: a tile adds at most
+// 100 x (128 + |qtype|) to a bin, and the host knows how many tiles a CTA can take (scan_needs_wide).
+// Otherwise (few CTAs over very many reads: one CTA, 100-bp reads at Q93 pass 2^31 after ~230 k
+// reads) the WIDE kernel keeps them in 64 bits.  The counts stay 32-bit: at most 100 per tile, so
+// they hold for < 42.9 M tiles per CTA, more than any batch has.
 #pragma once
 #include "common.cuh"
 
@@ -21,6 +27,15 @@
 #define SCAN_SMEM_BINS 1024
 #define SCAN_SMEM_BYTES \
     (SCAN_WARPS * SCAN_STAGES * 2 * SCAN_BUF + SCAN_SMEM_BINS * 10 * 4 + SCAN_WARPS * SCAN_STAGES * 8)
+#define SCAN_SMEM_BYTES_WIDE (SCAN_SMEM_BYTES + SCAN_SMEM_BINS * 5 * 4) /* quality sums in 64 bits */
+
+// Whether k_scan_tiles_dyn must keep its shared quality sums in 64 bits for a launch of `grid` CTAs over
+// at most `max_tiles` tiles.
+static inline bool scan_needs_wide(u64 max_tiles, int grid, int qtype) {
+    const u64 per_cta = max_tiles / (u64)grid + SCAN_WARPS; // tiles are dealt to warps round-robin
+    const u64 per_tile = (u64)SCAN_BIN * (u64)(128 + (qtype < 0 ? -(i64)qtype : (i64)qtype));
+    return per_cta * per_tile >= (1ull << 31);
+}
 
 static __device__ __forceinline__ u32 smem_u32(const void *p) {
     return (u32)__cvta_generic_to_shared(p);
@@ -98,7 +113,7 @@ static __device__ __forceinline__ void scan_word(BinAcc &a, u32 bw, u32 qw) {
 // bases/quals: whole batch streams (16-byte aligned, readable up to the next 16-byte boundary
 // past the last segment).  tiles: self-contained records (reads in the raw pass, kept pieces in
 // the clean pass).  seg_sum[seg] += sum(q - qtype).
-template <bool HAS_QUAL>
+template <bool HAS_QUAL, bool WIDE>
 __global__ void __launch_bounds__(SCAN_THREADS, 1)
 k_scan_tiles_dyn(const uint8_t *__restrict__ bases, const uint8_t *__restrict__ quals,
                  const TileEntry *__restrict__ tiles, const u32 *__restrict__ n_tiles_ptr,
@@ -107,11 +122,13 @@ k_scan_tiles_dyn(const uint8_t *__restrict__ bases, const uint8_t *__restrict__ 
     extern __shared__ __align__(128) uint8_t smem[];
     const u32 n_tiles = *n_tiles_ptr; // device-side total (tile_off[n_seg])
     uint8_t *stage_base = smem;
+    // narrow: [bin][10] u32 = 5 counts, 5 quality sums.  WIDE: [bin][5] u32 counts, then [bin][5] u64 sums.
     u32 *sbins = (u32 *)(smem + SCAN_WARPS * SCAN_STAGES * 2 * SCAN_BUF);
-    u64 *bars = (u64 *)(sbins + SCAN_SMEM_BINS * 10);
+    u64 *squal = (u64 *)(sbins + SCAN_SMEM_BINS * 5);
+    u64 *bars = (u64 *)(sbins + SCAN_SMEM_BINS * (WIDE ? 15 : 10));
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    for (int i = threadIdx.x; i < SCAN_SMEM_BINS * 10; i += SCAN_THREADS) sbins[i] = 0;
+    for (int i = threadIdx.x; i < SCAN_SMEM_BINS * (WIDE ? 15 : 10); i += SCAN_THREADS) sbins[i] = 0;
     if (threadIdx.x < SCAN_WARPS * SCAN_STAGES) mbar_init(smem_u32(&bars[threadIdx.x]), 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     __syncthreads();
@@ -210,11 +227,14 @@ k_scan_tiles_dyn(const uint8_t *__restrict__ bases, const uint8_t *__restrict__ 
         if (nvalid > 0) {
             const u32 gb = tile_idx * SCAN_TILE_BINS + lane;
             if (gb < SCAN_SMEM_BINS) {
-                u32 *p = sbins + gb * 10;
+                u32 *p = sbins + gb * (WIDE ? 5 : 10);
 #pragma unroll
                 for (int c = 0; c < 5; ++c) {
                     if (cnt[c]) atomicAdd(p + c, cnt[c]);
-                    if (HAS_QUAL && qs[c]) atomicAdd(p + 5 + c, (u32)qs[c]);
+                    if (HAS_QUAL && qs[c]) {
+                        if constexpr (WIDE) atomicAdd(squal + gb * 5 + c, (u64)(i64)qs[c]);
+                        else atomicAdd(p + 5 + c, (u32)qs[c]);
+                    }
                 }
             } else if (gb < max_bins) {
 #pragma unroll
@@ -240,11 +260,11 @@ k_scan_tiles_dyn(const uint8_t *__restrict__ bases, const uint8_t *__restrict__ 
     for (int i = threadIdx.x; i < SCAN_SMEM_BINS * 5; i += SCAN_THREADS) {
         const int b = i / 5, c = i % 5;
         if ((u32)b >= max_bins) continue;
-        const u32 vc = sbins[b * 10 + c];
+        const u32 vc = sbins[b * (WIDE ? 5 : 10) + c];
         if (vc) atomic_add_u64(bin_cnt + (u64)b * 5 + c, (u64)vc);
         if (HAS_QUAL) {
-            const int vq = (int)sbins[b * 10 + 5 + c];
-            if (vq) atomic_add_u64(bin_qual + (u64)b * 5 + c, (u64)(i64)vq);
+            const u64 vq = WIDE ? squal[i] : (u64)(i64)(int)sbins[b * 10 + 5 + c];
+            if (vq) atomic_add_u64(bin_qual + (u64)b * 5 + c, vq);
         }
     }
 }
@@ -314,6 +334,9 @@ k_ends_qc(const uint8_t *__restrict__ bases, const uint8_t *__restrict__ quals, 
             }
         }
     }
+    // The shared sums are 32-bit, which is enough: one CTA takes every (4 x sm_count)-th segment of a launch,
+    // and a row adds at most |qv| <= 192 per segment, so a sum stays below 2^31 up to 11.1 M segments per CTA,
+    // i.e. 44.7 M x sm_count segments per launch (a batch has at most 2^24 reads).
     if (use_smem) {
         __syncthreads();
         for (int i = threadIdx.x; i < 2 * bc_len * 5; i += ENDS_THREADS) {

@@ -267,6 +267,7 @@ struct tgsf_ctx {
     u32 kmer16_list_cap = KMER16_LIST_CAP; // TGSF_KMER16_LIST_CAP=n: smaller pending list (tests of the retry path)
     float last_kernel_ms = 0, last_total_ms = 0;
     float last_stage_ms[TGSF_N_STAGES] = {};
+    int last_chunk_shift = 0; // middle-scan chunk shift of the last collected batch (tgsf_launch_shape)
     cudaEvent_t ev_epoch = nullptr; // recorded at creation: origin of tgsf_last_span
     float last_span_start = 0, last_span_end = 0;
 };
@@ -446,15 +447,13 @@ int launch_scan_pass(tgsf_ctx *c, Slot &s, u32 n_seg, u64 *bin_cnt, u64 *bin_qua
     u32 *status = &s.header.as<DevHeader>()->status;
     // n_tiles is passed by value through a tiny indirection kernel-free trick: tiles_cap bounds it,
     // and the kernel takes the device-side total.
-    if (s.has_qual) {
-        k_scan_tiles_dyn<true><<<grid, SCAN_THREADS, SCAN_SMEM_BYTES, st>>>(
-            s.B.bases, s.B.quals, s.tiles.as<TileEntry>(), s.tile_off.as<u32>() + n_seg,
-            s.seg_sum.as<u64>(), bin_cnt, bin_qual, c->P.qtype, c->P.L.max_bins, status);
-    } else {
-        k_scan_tiles_dyn<false><<<grid, SCAN_THREADS, SCAN_SMEM_BYTES, st>>>(
-            s.B.bases, s.B.quals, s.tiles.as<TileEntry>(), s.tile_off.as<u32>() + n_seg,
-            s.seg_sum.as<u64>(), bin_cnt, bin_qual, c->P.qtype, c->P.L.max_bins, status);
-    }
+    auto launch = [&](auto kern, size_t smem) {
+        kern<<<grid, SCAN_THREADS, smem, st>>>(s.B.bases, s.B.quals, s.tiles.as<TileEntry>(), s.tile_off.as<u32>() + n_seg,
+                                               s.seg_sum.as<u64>(), bin_cnt, bin_qual, c->P.qtype, c->P.L.max_bins, status);
+    };
+    if (!s.has_qual) launch(k_scan_tiles_dyn<false, false>, SCAN_SMEM_BYTES); // counts only
+    else if (scan_needs_wide(s.tiles_cap, grid, c->P.qtype)) launch(k_scan_tiles_dyn<true, true>, SCAN_SMEM_BYTES_WIDE);
+    else launch(k_scan_tiles_dyn<true, false>, SCAN_SMEM_BYTES);
     c->launches++;
     return check_launch("k_scan_tiles");
 }
@@ -948,8 +947,9 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
         rc = TGSF_ERR_CUDA;
     }
     if (rc == TGSF_OK) {
-        cudaError_t e1 = cudaFuncSetAttribute(k_scan_tiles_dyn<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
-        cudaError_t e2 = cudaFuncSetAttribute(k_scan_tiles_dyn<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
+        cudaError_t e1 = cudaFuncSetAttribute(k_scan_tiles_dyn<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
+        cudaError_t e2 = cudaFuncSetAttribute(k_scan_tiles_dyn<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
+        if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(k_scan_tiles_dyn<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES_WIDE);
         c->kmer_force_l2 = getenv("TGSF_KMER_L2") != nullptr;
         c->kmer_force_bitmap = getenv("TGSF_KMER_BITMAP") != nullptr;
         c->kmer_force_tag32 = getenv("TGSF_KMER_TAG32") != nullptr;
@@ -957,6 +957,9 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
         if (const char *e = getenv("TGSF_CARVEOUT")) c->max_carveout = atoi(e) != 0;
         if (const char *e = getenv("TGSF_FORK_ENDS")) c->fork_ends = atoi(e) != 0;
         if (const char *e = getenv("TGSF_RES_CTAS")) c->res_ctas_per_sm = std::max(1, std::min(16, atoi(e)));
+        // TGSF_SM_COUNT=n: size every grid and the chunk-shift rule as if the device had n SMs (clamped to
+        // [1, real count]), so that tests reach the launch shapes of multi-Gbase batches with small batches
+        if (const char *e = getenv("TGSF_SM_COUNT")) c->sm_count = std::max(1, std::min(c->sm_count, atoi(e)));
         if (const char *e = getenv("TGSF_KMER16_LIST_CAP")) c->kmer16_list_cap = (u32)std::min<long>(std::max<long>(atol(e), 32), (long)KMER16_LIST_CAP);
         cudaError_t e3 = cudaFuncSetAttribute(k_kmer<u32>, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SMEM_BYTES);
         cudaError_t e4 = cudaFuncSetAttribute(k_kmer<u64>, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SMEM_BYTES);
@@ -1342,6 +1345,7 @@ int tgsf_collect(tgsf_ctx *c, tgsf_read_result *reads, uint32_t n_reads, tgsf_pi
         cudaEventElapsedTime(&ms, s.ev_stage[i], s.ev_stage[i + 1]);
         c->last_stage_ms[i] = ms;
     }
+    c->last_chunk_shift = s.chunk_shift;
 
     auto retire = [&]() {
         s.busy = false;
@@ -1427,6 +1431,13 @@ int tgsf_counters_device(tgsf_ctx *c, void **d_ptr, uint32_t *n_u64) {
 }
 
 uint64_t tgsf_launch_count(const tgsf_ctx *c) { return c ? c->launches : 0; }
+
+int tgsf_launch_shape(const tgsf_ctx *c, int32_t *sm_count, int32_t *last_chunk_shift) {
+    if (!c) { set_err("ctx is NULL"); return TGSF_ERR_INVALID; }
+    if (sm_count) *sm_count = c->sm_count;
+    if (last_chunk_shift) *last_chunk_shift = c->last_chunk_shift;
+    return TGSF_OK;
+}
 
 
 int tgsf_allreduce(tgsf_ctx **ctxs, int n) {

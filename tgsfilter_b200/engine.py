@@ -234,6 +234,12 @@ class FilterEngine:
     def launch_count(self) -> int:
         return int(self._lib.tgsf_launch_count(self._ctx))
 
+    def launch_shape(self) -> Tuple[int, int]:
+        """(SM count the grids are sized by, middle-scan chunk shift of the last collected batch)."""
+        sm, shift = C.c_int32(0), C.c_int32(0)
+        _capi.check(self._lib.tgsf_launch_shape(self._ctx, C.byref(sm), C.byref(shift)), "tgsf_launch_shape")
+        return sm.value, shift.value
+
 
 def align_hw(pairs, device: int = 0) -> np.ndarray:
     """tgsf_align_hw on [(query, target, k)]: edlib HW+PATH semantics, one result per pair."""
