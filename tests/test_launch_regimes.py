@@ -487,13 +487,12 @@ def test_slot_ring_sequence_vs_oracle(n_slots):
     assert n_slots == 1 or seen == {"pool_overflow", "long_read"}
 
 
-def test_kept_clean_bitmap_over_consecutive_batches(monkeypatch):
-    """k = 13 on the global bitmap kernel (TGSF_KMER_L2): the per-CTA maps are zeroed once and must be left clean
-    by every batch; three batches through one slot."""
-    monkeypatch.setenv("TGSF_KMER_L2", "1")
+def test_kmer_long_list_over_consecutive_batches():
+    """k = 13 with one read per batch above the 65 000 k-mers of k_kmer_tag16: its work counter, the long-list
+    counter and the long list must start over with every batch; three batches through one slot."""
     params = FilterParams(min_len=50, min_q=0.0, kmer=13, min_repeat=200, qtype=33, adapters=[],
                           max_read_len=500000, n_slots=1)
-    batches = [_repeat_batch(500 + i, n=60) for i in range(3)]
+    batches = [_repeat_batch(500 + i, n=60, long_read=[70000]) for i in range(3)]
     o_cnt = None
     with FilterEngine(params) as eng:
         for b in batches:

@@ -223,7 +223,7 @@ struct Slot {
     DBuf read_active, piece_cnt, piece_begin, chunk_cnt, chunk_off, chunks, chunk_min, chunk_hits, chunk_first, chunk_perm, chunk_hist;
     int chunk_shift = MID_CHUNK_SHIFT_MIN;
     DBuf best_mid, mid_n, mid_off, end_n, end_pos, pool, sortbuf, tmp, pieces, res, header;
-    DBuf scan_tmp, kmer_bitmaps, kmer_long_list, mid_work, gz_blob, gz_spans;
+    DBuf scan_tmp, kmer_long_list, mid_work, gz_blob, gz_spans;
     DBuf contam_cnt, contam_off, contam_chunks; // contaminant screen (only with a set installed)
     Scratch scratch, scratch2; // traceback stores: main stream (k_mid_count) / side stream (k_ends)
     u32 pool_cap = 0, pieces_cap = 0, chunks_cap = 0, tiles_cap = 0;
@@ -256,14 +256,10 @@ struct tgsf_ctx {
     std::vector<Slot> slots;
     u32 head = 0, tail = 0, outstanding = 0; // ring: submit at head, collect at tail
     u64 launches = 0;
-    bool kmer_force_l2 = false; // TGSF_KMER_L2=1: keep k <= 12 on the global-memory bitmap kernel (A/B, tests)
-    bool kmer_force_bitmap = false; // TGSF_KMER_BITMAP=1: shared-memory bitmap passes also for single-tile pieces
-    bool kmer_force_tag32 = false;  // TGSF_KMER_TAG32=1: k <= 12 stays on k_kmer_smem alone (round-1 kernel; A/B, tests)
     int kmer16_ctas_per_sm = 2;
     int mid_ctas_per_sm = 0; // TGSF_MID_CTAS=n: cap on resident k_mid_scan CTAs per SM (0 = as many as fit)
     int res_ctas_per_sm = 6; // grid of the resolve kernels (k_ends, k_mid_count, k_mid_emit) in CTAs per SM; TGSF_RES_CTAS
     bool fork_ends = true; // TGSF_FORK_ENDS=0: k_ends on the batch's main stream after the middle scan (A/B)
-    bool max_carveout = false; // TGSF_CARVEOUT=1 (measured: no gain, see want_max_carveout)
     u32 kmer16_list_cap = KMER16_LIST_CAP; // TGSF_KMER16_LIST_CAP=n: smaller pending list (tests of the retry path)
     float last_kernel_ms = 0, last_total_ms = 0;
     float last_stage_ms[TGSF_N_STAGES] = {};
@@ -317,7 +313,7 @@ void slot_release(Slot &s) {
                     &s.seg_flag, &s.tile_cnt, &s.tile_off, &s.tiles, &s.read_active, &s.piece_cnt,
                     &s.piece_begin, &s.chunk_cnt, &s.chunk_off, &s.chunks, &s.chunk_min, &s.chunk_hits, &s.chunk_first, &s.chunk_perm, &s.chunk_hist,
                     &s.best_mid, &s.mid_n, &s.mid_off, &s.end_n, &s.end_pos, &s.pool, &s.sortbuf,
-                    &s.tmp, &s.pieces, &s.res, &s.header, &s.scan_tmp, &s.kmer_bitmaps, &s.kmer_long_list, &s.mid_work, &s.gz_blob, &s.gz_spans, &s.scratch.buf, &s.scratch2.buf,
+                    &s.tmp, &s.pieces, &s.res, &s.header, &s.scan_tmp, &s.kmer_long_list, &s.mid_work, &s.gz_blob, &s.gz_spans, &s.scratch.buf, &s.scratch2.buf,
                     &s.contam_cnt, &s.contam_off, &s.contam_chunks};
     for (DBuf *b : bufs) b->release();
     s.h_res.release();
@@ -410,18 +406,6 @@ int for_nw(int nw, F f) {
         case 32: return f(std::integral_constant<int, 32>());
         default: set_err("adapter longer than %d", TGSF_MAX_ADAPTER_LEN); return TGSF_ERR_INVALID;
     }
-}
-
-// Kernels that want different shared-memory carve-outs cannot be resident on one SM at the same time (the SM has to
-// drain before its L1 / shared split changes).  The K1 scan needs the maximum carve-out (197 KB of tiles and bins), so
-// every kernel that should be able to run NEXT to it (another batch's adapter scan, resolve and region kernels in the
-// other slot) would have to ask for the same split.  Measured on config[1] with two batches in flight (round 2):
-// 14.31 ms with the common carve-out vs 14.25 ms without, also when k_mid_scan leaves room (TGSF_MID_CTAS 3..5:
-// 15.4 / 14.5 / 14.4 ms) — the tails of one batch do not get under the other batch's scan this way either, so the
-// driver's choice stays the default; TGSF_CARVEOUT=1 turns the common split on (A/B).
-template <typename K>
-void want_max_carveout(const tgsf_ctx *c, K kern) {
-    if (c->max_carveout) cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
 }
 
 int check_launch(const char *what) {
@@ -535,8 +519,6 @@ int launch_head(tgsf_ctx *c, Slot &s) {
                 const u64 stride_a = (u64)grid_a * RES_THREADS;
                 TRY(for_nw(nw, [&](auto nwc) {
                     constexpr int NW = decltype(nwc)::value;
-                    want_max_carveout(c, k_ends<NW, 1>);
-                    if constexpr (NW <= 2) want_max_carveout(c, k_ends<NW, 2>);
                     if constexpr (NW <= 2) {
                         if (a1 != a0)
                             k_ends<NW, 2><<<grid_a, RES_THREADS, 2 * 4 * 256 * NW * sizeof(u64), es>>>(
@@ -603,7 +585,6 @@ int launch_head(tgsf_ctx *c, Slot &s) {
                 TRY(for_nw(nw, [&](auto nwc) {
                     constexpr int NW = decltype(nwc)::value;
                     auto launch = [&](auto kern, size_t smem) {
-                        want_max_carveout(c, kern);
                         int occ = 0; // persistent grid: exactly the resident CTA count
                         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, MID_THREADS, smem) != cudaSuccess || occ < 1) occ = 4;
                         if (c->mid_ctas_per_sm > 0) occ = std::min(occ, c->mid_ctas_per_sm);
@@ -631,7 +612,6 @@ int launch_head(tgsf_ctx *c, Slot &s) {
             const int grid_a = Scratch::grid_for(res_grid, RES_THREADS, 2 * Ah.qlen + 2, Ah.nw);
             TRY(for_nw(Ah.nw, [&](auto nwc) {
                 constexpr int NW = decltype(nwc)::value;
-                want_max_carveout(c, k_mid_count<NW>);
                 k_mid_count<NW><<<grid_a, RES_THREADS, 0, st>>>(
                     s.B, AC, a, P.end_len, A, s.best_mid.as<u32>(), s.chunk_off.as<u32>(), s.chunks_cap,
                     s.chunk_min.as<uint8_t>(), s.chunk_hits.as<u32>(), s.chunk_first.as<u64>(),
@@ -651,6 +631,34 @@ int launch_head(tgsf_ctx *c, Slot &s) {
     }
     CU(cudaEventRecord(s.ev_stage[4], st));
     return check_launch("head");
+}
+
+// K4, the -p repeat check.  k <= 16: k_kmer_tag16 over all pieces, as many CTAs per SM as fit; it hands the pieces too
+// long for its 16-bit positions to a long list, which k_kmer_smem (k <= 12) or the hash kernel k_kmer (k = 13 .. 16)
+// works through next.  k > 16: k_kmer over all pieces.
+int launch_kmer(tgsf_ctx *c, Slot &s, const DevParams &P) {
+    cudaStream_t st = s.stream;
+    DevHeader *H = s.header.as<DevHeader>();
+    u64 *C = c->counters.as<u64>();
+    tgsf_piece *pieces = s.pieces.as<tgsf_piece>();
+    if (P.kmer > 16) {
+        k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->tmp_cursor, C, &H->status, nullptr);
+        c->launches++;
+        return check_launch("k_kmer");
+    }
+    TRY(s.kmer_long_list.ensure((size_t)s.pieces_cap * sizeof(u32)));
+    u32 *long_list = s.kmer_long_list.as<u32>();
+    k_kmer_tag16<<<c->sm_count * c->kmer16_ctas_per_sm, KMER16_THREADS, KMER16_SMEM_BYTES, st>>>(
+        s.B, P, pieces, &H->tmp_cursor, C, &H->status, &H->kmer_work, long_list, &H->kmer_long, c->kmer16_list_cap);
+    if (P.kmer <= 12)
+        k_kmer_smem<<<c->sm_count, KMER_SB_THREADS, KMER_SB_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status,
+                                                                             long_list);
+    else if (P.kmer <= 15)
+        k_kmer<u32><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status, long_list);
+    else
+        k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status, long_list);
+    c->launches += 2;
+    return check_launch("k_kmer");
 }
 
 // Contaminant screen over the pieces still emitted after K4; writes piece fields only.
@@ -711,7 +719,6 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
             if (Ah.k_mid <= 0) continue;
             TRY(for_nw(Ah.nw, [&](auto nwc) {
                 constexpr int NW = decltype(nwc)::value;
-                want_max_carveout(c, k_mid_emit<NW>);
                 k_mid_emit<NW><<<res_grid, RES_THREADS, 0, st>>>(
                     s.B, AC, a, P.end_len, s.chunk_shift, P.extra_len, A, s.best_mid.as<u32>(), s.chunk_off.as<u32>(),
                     s.chunks.as<ChunkEntry>(), s.chunks_cap, s.chunk_min.as<uint8_t>(), s.chunk_hits.as<u32>(),
@@ -726,7 +733,6 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
     }
     // the host copies an optimistic prefix of the piece array before the count is known (enqueue_d2h): define it
     CU(cudaMemsetAsync(s.pieces.p, 0, (size_t)std::min<u32>(s.pieces_cap, n + 4096) * sizeof(tgsf_piece), st));
-    want_max_carveout(c, k_regions);
     k_regions<<<cdiv(n, REG_THREADS), REG_THREADS, 0, st>>>(
         s.B, P, s.read_active.as<int>(), s.end_n.as<int>(), s.end_pos.as<int>(), s.mid_n.as<u32>(),
         s.mid_off.as<u32>(), s.pool.as<Region>(), s.sortbuf.as<Region>(), s.pool_cap * 5, &H->sort_cursor,
@@ -743,51 +749,7 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
     c->launches++;
     CU(cudaEventRecord(s.ev_stage[5], st));
     if (!(P.flags & TGSF_FLAG_ONLY_QC)) {
-        if (P.min_repeat > 0 && P.kmer <= 16 && !c->kmer_force_l2 && !c->kmer_force_bitmap && !c->kmer_force_tag32) {
-            // owner-entry rounds, two CTAs per SM; pieces too long for 16-bit positions go to k_kmer_smem (k <= 12) or
-            // to the hash kernel (k = 13 .. 16) through the long list
-            TRY(s.kmer_long_list.ensure((size_t)s.pieces_cap * sizeof(u32)));
-            k_kmer_tag16<<<c->sm_count * c->kmer16_ctas_per_sm, KMER16_THREADS, KMER16_SMEM_BYTES, st>>>(
-                s.B, P, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, C, &H->status, &H->kmer_work,
-                s.kmer_long_list.as<u32>(), &H->kmer_long, c->kmer16_list_cap);
-            if (P.kmer <= 12)
-                k_kmer_smem<<<c->sm_count, KMER_SB_THREADS, KMER_SB_SMEM_BYTES, st>>>(s.B, P, s.pieces.as<tgsf_piece>(),
-                                                                                     &H->kmer_long, C, &H->status, 0,
-                                                                                     s.kmer_long_list.as<u32>());
-            else if (P.kmer <= 15)
-                k_kmer<u32><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, s.pieces.as<tgsf_piece>(), &H->kmer_long, C,
-                                                                            &H->status, s.kmer_long_list.as<u32>());
-            else
-                k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, s.pieces.as<tgsf_piece>(), &H->kmer_long, C,
-                                                                            &H->status, s.kmer_long_list.as<u32>());
-            c->launches += 2;
-        } else if (P.min_repeat > 0 && P.kmer <= 12 && !c->kmer_force_l2) {
-            // round-1 path: 32-bit tag rounds / shared-memory bitmap in key-range passes, one CTA per SM
-            k_kmer_smem<<<c->sm_count, KMER_SB_THREADS, KMER_SB_SMEM_BYTES, st>>>(s.B, P, s.pieces.as<tgsf_piece>(),
-                                                                                 &H->tmp_cursor, C, &H->status, c->kmer_force_bitmap ? 1 : 0,
-                                                                                 nullptr);
-            c->launches++;
-        } else if (P.min_repeat > 0 && P.kmer <= 13) {
-            // bitmap path: one 4^k-bit map per CTA, zeroed once and kept clean by the kernel
-            const u64 words = (1ull << (2 * P.kmer)) / 32 + 1;
-            const int grid = P.kmer <= 11 ? c->sm_count : std::max(1, c->sm_count / (1 << (2 * (P.kmer - 11))));
-            const size_t bytes = (size_t)grid * words * sizeof(u32);
-            if (s.kmer_bitmaps.cap < bytes) {
-                TRY(s.kmer_bitmaps.ensure(bytes));
-                CU(cudaMemsetAsync(s.kmer_bitmaps.p, 0, s.kmer_bitmaps.cap, st));
-            }
-            k_kmer_bitmap<<<grid, KMER_BM_THREADS, 0, st>>>(s.B, P, s.pieces.as<tgsf_piece>(), &H->tmp_cursor,
-                                                            s.kmer_bitmaps.as<u32>(), words, C, &H->status);
-            c->launches++;
-        } else if (P.min_repeat > 0) {
-            if (P.kmer <= 15)
-                k_kmer<u32><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, s.pieces.as<tgsf_piece>(),
-                                                                            &H->tmp_cursor, C, &H->status, nullptr);
-            else
-                k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, s.pieces.as<tgsf_piece>(),
-                                                                            &H->tmp_cursor, C, &H->status, nullptr);
-            c->launches++;
-        }
+        if (P.min_repeat > 0) TRY(launch_kmer(c, s, P));
         if (c->contam.installed()) TRY(launch_contam(c, s));
         CU(cudaEventRecord(s.ev_stage[6], st));
         // clean pass over the kept pieces (T.cpp:1991-2009); piece count is device-side, the
@@ -947,14 +909,11 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
         rc = TGSF_ERR_CUDA;
     }
     if (rc == TGSF_OK) {
+        // dynamic shared-memory limits only: no kernel asks for a carve-out (measured, DESIGN §8)
         cudaError_t e1 = cudaFuncSetAttribute(k_scan_tiles_dyn<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
         cudaError_t e2 = cudaFuncSetAttribute(k_scan_tiles_dyn<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
         if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(k_scan_tiles_dyn<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES_WIDE);
-        c->kmer_force_l2 = getenv("TGSF_KMER_L2") != nullptr;
-        c->kmer_force_bitmap = getenv("TGSF_KMER_BITMAP") != nullptr;
-        c->kmer_force_tag32 = getenv("TGSF_KMER_TAG32") != nullptr;
         if (const char *e = getenv("TGSF_MID_CTAS")) c->mid_ctas_per_sm = atoi(e);
-        if (const char *e = getenv("TGSF_CARVEOUT")) c->max_carveout = atoi(e) != 0;
         if (const char *e = getenv("TGSF_FORK_ENDS")) c->fork_ends = atoi(e) != 0;
         if (const char *e = getenv("TGSF_RES_CTAS")) c->res_ctas_per_sm = std::max(1, std::min(16, atoi(e)));
         // TGSF_SM_COUNT=n: size every grid and the chunk-shift rule as if the device had n SMs (clamped to
