@@ -252,7 +252,9 @@ int tgsf_launch_shape(const tgsf_ctx *ctx, int32_t *sm_count, int32_t *last_chun
  * row_len bytes (seq[0:checkLen] and revcomp(seq[-checkLen:]), T.cpp:966-969).  Outputs:
  * bases_num5p/3p [row_len][4] int32 in A,T,G,C order; map5p/3p [n_lib] int64 = sum of
  * (alignmentLength - editDistance) over the rows where the library adapter aligned with
- * k = int((1-minSim)*qLen)+1.  lib == NULL skips the adapter search (AdapterFile given). */
+ * k = int((1-minSim)*qLen)+1.  lib == NULL skips the adapter search (AdapterFile given).  Any row_len >= 1;
+ * 1 <= n_lib <= 1024 and library adapters of 1..TGSF_MAX_ADAPTER_LEN bases, otherwise TGSF_ERR_INVALID before
+ * the device is touched. */
 int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint32_t n,
                  uint32_t row_len, const uint8_t *const *lib_seq, const int32_t *lib_len,
                  int32_t n_lib, float min_sim, int32_t *bases_num5p, int32_t *bases_num3p,

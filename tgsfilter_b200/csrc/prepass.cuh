@@ -8,25 +8,32 @@
 #include "scan.cuh"
 
 #define PRE_THREADS 256
+// Columns per k_base_content tile: a [3072][4] u32 table is 48 KB, the dynamic shared memory a launch gets without
+// an opt-in, so any row length is counted with the same table.
+#define PRE_TILE_COLS 3072
 
-// rows: [n][row_len] bytes; out: [row_len][4] int32 (A,T,G,C).  Shared-memory histogram per CTA.
+// rows: [n][row_len] bytes; out: [row_len][4] int32 (A,T,G,C).  blockIdx.y picks a tile of PRE_TILE_COLS columns
+// (the last one shorter); each CTA counts its rows over that tile in a shared-memory table and adds it to out.
 __global__ void __launch_bounds__(PRE_THREADS)
 k_base_content(const uint8_t *__restrict__ rows, u32 n, u32 row_len, int *__restrict__ out) {
-    extern __shared__ u32 hist[]; // [row_len][4]
-    for (u32 i = threadIdx.x; i < row_len * 4; i += PRE_THREADS) hist[i] = 0;
+    extern __shared__ u32 hist[]; // [cols][4]
+    const u32 col0 = blockIdx.y * PRE_TILE_COLS;
+    const u32 cols = min(row_len - col0, (u32)PRE_TILE_COLS);
+    for (u32 i = threadIdx.x; i < cols * 4; i += PRE_THREADS) hist[i] = 0;
     __syncthreads();
     const int lane = threadIdx.x & 31;
     const u32 wpb = PRE_THREADS / 32;
     for (u32 r = blockIdx.x * wpb + (threadIdx.x >> 5); r < n; r += gridDim.x * wpb) {
-        const uint8_t *row = rows + (u64)r * row_len;
-        for (u32 i = lane; i < row_len; i += 32) {
+        const uint8_t *row = rows + (u64)r * row_len + col0;
+        for (u32 i = lane; i < cols; i += 32) {
             const int c = base_cat(row[i]);
             if (c >= 0) atomicAdd(&hist[i * 4 + c], 1u);
         }
     }
     __syncthreads();
-    for (u32 i = threadIdx.x; i < row_len * 4; i += PRE_THREADS)
-        if (hist[i]) atomicAdd(out + i, (int)hist[i]);
+    int *tile_out = out + (u64)col0 * 4;
+    for (u32 i = threadIdx.x; i < cols * 4; i += PRE_THREADS)
+        if (hist[i]) atomicAdd(tile_out + i, (int)hist[i]);
 }
 
 // One thread per (row, library adapter).  k per adapter is DevAdapter::k_end (the host stores

@@ -1451,11 +1451,16 @@ int tgsf_allreduce(tgsf_ctx **ctxs, int n) {
 int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint32_t n, uint32_t row_len,
                  const uint8_t *const *lib_seq, const int32_t *lib_len, int32_t n_lib, float min_sim,
                  int32_t *bases_num5p, int32_t *bases_num3p, int64_t *map5p, int64_t *map3p) {
-    if (!ends5p || !ends3p || !bases_num5p || !bases_num3p || row_len == 0 || row_len > 8192) {
+    if (!ends5p || !ends3p || !bases_num5p || !bases_num3p || row_len == 0) {
         set_err("prepass: bad arguments");
         return TGSF_ERR_INVALID;
     }
     if (lib_seq && (n_lib <= 0 || n_lib > 1024 || !lib_len || !map5p || !map3p)) { set_err("prepass: bad library"); return TGSF_ERR_INVALID; }
+    for (int32_t a = 0; lib_seq && a < n_lib; ++a)
+        if (!lib_seq[a] || lib_len[a] <= 0 || lib_len[a] > TGSF_MAX_ADAPTER_LEN) {
+            set_err("prepass: library adapter %d: length %d outside [1, %d]", a, lib_len[a], TGSF_MAX_ADAPTER_LEN);
+            return TGSF_ERR_INVALID;
+        }
     CU(cudaSetDevice(device));
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
@@ -1478,16 +1483,20 @@ int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint3
     if (e != cudaSuccess) { set_err("prepass upload: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
     int *c5 = d_cnt.as<int>(), *c3 = c5 + (size_t)row_len * 4;
     if (n) {
-        const int grid = std::min<u32>((u32)sms * 4, cdiv(n, PRE_THREADS / 32));
-        k_base_content<<<grid, PRE_THREADS, (size_t)row_len * 4 * sizeof(u32)>>>(r5, n, row_len, c5);
-        k_base_content<<<grid, PRE_THREADS, (size_t)row_len * 4 * sizeof(u32)>>>(r3, n, row_len, c3);
+        // column tiles on y; about 4 CTAs per SM in all, so the flush of the per-CTA tables does not grow with row_len
+        const u32 tiles = cdiv(row_len, PRE_TILE_COLS);
+        const dim3 grid(std::max<u32>(1, std::min<u32>(cdiv((u64)sms * 4, tiles), cdiv(n, PRE_THREADS / 32))), tiles);
+        const size_t smem = (size_t)std::min<u32>(row_len, PRE_TILE_COLS) * 4 * sizeof(u32);
+        k_base_content<<<grid, PRE_THREADS, smem>>>(r5, n, row_len, c5);
+        k_base_content<<<grid, PRE_THREADS, smem>>>(r3, n, row_len, c3);
+        rc = check_launch("k_base_content");
+        if (rc != TGSF_OK) { cleanup(); return rc; }
     }
     if (lib_seq) {
         rc = ads.build(lib_seq, lib_len, n_lib);
         if (rc == TGSF_OK) {
             if (min_sim < 0.9) min_sim = 0.9; // T.cpp:1151-1154 (float compared against a double literal)
             for (auto &A : ads.host) {
-                if (A.qlen <= 0 || A.qlen > TGSF_MAX_ADAPTER_LEN) { rc = TGSF_ERR_INVALID; set_err("library adapter length"); break; }
                 int minK = static_cast<int>((1 - min_sim) * A.qlen) + 1; // T.cpp:1161
                 A.k_end = std::min(minK, A.qlen - 1);
             }
@@ -1496,7 +1505,8 @@ int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint3
         if (rc == TGSF_OK) rc = d_maps.ensure((size_t)2 * n_lib * sizeof(long long));
         if (rc == TGSF_OK) rc = scratch.ensure(ads.host, sms * 4, RES_THREADS);
         if (rc != TGSF_OK) { cleanup(); return rc; }
-        cudaMemset(d_maps.p, 0, (size_t)2 * n_lib * sizeof(long long));
+        e = cudaMemset(d_maps.p, 0, (size_t)2 * n_lib * sizeof(long long));
+        if (e != cudaSuccess) { set_err("prepass maps: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
         long long *m5 = d_maps.as<long long>(), *m3 = m5 + n_lib;
         const AdapterCtx AC = ads.ctx();
         for (int a = 0; a < n_lib && n; ++a) {
