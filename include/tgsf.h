@@ -246,6 +246,9 @@ uint64_t tgsf_launch_count(const tgsf_ctx *ctx);
  * bases, chosen per batch from its size and that SM count) of the last collected batch (0 before
  * the first).  Lets tests check which launch regime a batch ran in. */
 int tgsf_launch_shape(const tgsf_ctx *ctx, int32_t *sm_count, int32_t *last_chunk_shift);
+/* log2 of the number of chunks per middle-scan run (the scan restarts a halo once per run) of the last collected
+ * batch, chosen per batch like the chunk shift (0 before the first). */
+int tgsf_mid_run_shift(const tgsf_ctx *ctx, int32_t *last_run_shift);
 
 /* Replaces: the compute of the pre-pass, CheckBaseContent's counting loop (T.cpp:1080-1095) and
  * adapterSearch's edlib loop (T.cpp:1156-1176), for both read ends.  ends5p / ends3p: n rows of

@@ -115,7 +115,7 @@ EXPORTED_SYMBOLS = (
     "tgsf_version", "tgsf_last_error", "tgsf_create", "tgsf_destroy", "tgsf_device_count", "tgsf_host_alloc",
     "tgsf_host_free", "tgsf_submit", "tgsf_submit_packed", "tgsf_pack_bases", "tgsf_submit_device", "tgsf_collect", "tgsf_collect_gz", "tgsf_last_timing", "tgsf_last_span", "tgsf_last_stage_ms",
     "tgsf_counter_layout_get", "tgsf_counters", "tgsf_counters_reset", "tgsf_counters_device",
-    "tgsf_launch_count", "tgsf_launch_shape", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw", "tgsf_set_contaminants",
+    "tgsf_launch_count", "tgsf_launch_shape", "tgsf_mid_run_shift", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw", "tgsf_set_contaminants",
 )
 
 _lib = None
@@ -157,6 +157,7 @@ def load() -> C.CDLL:
     lib.tgsf_launch_count.restype = C.c_uint64
     lib.tgsf_launch_count.argtypes = [vp]
     lib.tgsf_launch_shape.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+    lib.tgsf_mid_run_shift.argtypes = [vp, C.POINTER(C.c_int32)]
     lib.tgsf_allreduce.argtypes = [C.POINTER(vp), C.c_int]
     lib.tgsf_prepass.argtypes = [C.c_int, u8p, u8p, C.c_uint32, C.c_uint32,
                                  C.POINTER(C.c_char_p), C.POINTER(C.c_int32), C.c_int32, C.c_float,

@@ -1,8 +1,9 @@
 // K3: adapter search kernels.  Replaces GetEditDistance (T.cpp:1218-1322) = three edlibAlign
 // (HW, PATH) calls per (read, adapter): middle window, 5' window, 3' window.
 //
-//   k_mid_scan    one thread per (1024-column absolute chunk of a read's middle window, adapter):
-//                 HW scan with a q+k-1 column halo, chunk minimum + atomicMin per (read, adapter).
+//   k_mid_scan    one thread per run of consecutive 1024-column absolute chunks of a read's middle window and
+//                 adapter: HW scan with a q+k-1 column halo before the run, chunk minima + atomicMin per
+//                 (read, adapter).
 //                 This is the kernel that dominates the pipeline (INT-ALU bound).
 //   k_mid_count   one thread per (read, adapter) whose best distance is <= k: enumerates the end
 //                 columns (only chunks whose minimum equals the best), runs edlib's PATH step on
@@ -34,12 +35,18 @@ static __device__ __forceinline__ AdapterTables adapter_tables(const AdapterCtx 
 // ---------------------------------------------------------------------------------------------
 // k_mid_scan
 // ---------------------------------------------------------------------------------------------
-// One thread per chunk of a read's middle window; the thread scans the chunk for AP adapters of the
-// same word count at once: one LDS (64*AP*NW bits) per column serves all of them and the
-// independent Myers chains interleave.  The bottom-row score is not kept per column: Ph/Mh top bits
-// go into 32-bit histories and are folded every 16 columns; the exact per-column minimum is only
-// evaluated for a group when score - popc(minus bits) could reach k (otherwise no column of the
-// group can score <= k, and scores > k are never reported).
+// One thread per run: up to 2^run_shift consecutive chunks of a read's middle window (the absolute block
+// [run << (chunk_shift + run_shift), +2^(chunk_shift + run_shift)) clipped to the window).  The thread restarts a
+// q+k-1 column halo before the run's first chunk only and carries the Myers state across the later chunk
+// boundaries, where the state is the exact DP column; at each boundary it closes the finished chunk and starts
+// the next one's minimum.  The per-chunk results are what a halo restart per chunk gives: a chunk minimum is only
+// reported when it is <= k, and every column scoring <= k is exact after a halo of q+k-1 columns.
+//
+// The thread scans the run for AP adapters of the same word count at once: one LDS (64*AP*NW bits) per column
+// serves all of them and the independent Myers chains interleave.  The bottom-row score is not kept per column:
+// it is read off the state (popcounts) every 8 columns; the exact per-column minimum is only evaluated for a
+// group when score - popc(minus bits) could reach k (otherwise no column of the group can score <= k, and scores
+// > k are never reported).
 //
 // chunk_min : [n_adapters][chunk_stride] u8 (255 = nothing <= min(k,254) / window too short)
 // chunk_cnt / chunk_first : [n_adapters][chunk_stride], written only where chunk_min != 255:
@@ -50,8 +57,10 @@ struct MidScanArgs {
     int a[2];            // adapter indices handled by this launch (a[1] unused when AP == 1)
     int end_len;
     int chunk_shift;     // log2(chunk length)
+    int run_shift;       // log2(chunks per run)
     u32 chunk_stride;
     int n_adapters;
+    u32 byte_mul[4];     // {2^24, 2^16, 2^8, 8 * AP * NW}: see mid_row_off
 };
 
 template <int NW>
@@ -71,11 +80,13 @@ static __device__ void mid_chunk_record(const u64 *__restrict__ tab, int tab_str
     }
 }
 
-// Rare path of k_mid_scan: exact column-by-column minimum of one 8-column group, replayed from
-// the state saved at the group start.  Kept out of line so that it costs the hot loop no registers.
+// Rare path of k_mid_scan: exact column-by-column minimum of one 8-column group, replayed from the state saved at
+// the group start, folded into the replay threshold (see k_mid_scan_dyn).  Kept out of line so that it costs the
+// hot loop no registers.
 template <int NW>
 static __device__ __noinline__ int mid_replay_group(const u64 *P0, const u64 *M0, u32 w0, u32 w1,
-                                                    const u64 *tab, int tab_stride, int best) {
+                                                    const u64 *tab, int tab_stride, int thr) {
+    int best = 0x7fffffff;
     u64 tP[NW], tM[NW];
 #pragma unroll
     for (int w = 0; w < NW; ++w) { tP[w] = P0[w]; tM[w] = M0[w]; }
@@ -86,17 +97,27 @@ static __device__ __noinline__ int mid_replay_group(const u64 *P0, const u64 *M0
         myers_step_state<NW>(tP, tM, tab + byte * tab_stride);
         best = min(best, myers_score<NW>(tP, tM));
     }
-    return best;
+    return min(thr, 2 * best + 6);
+}
+
+// Byte offset of the table row of base j of a 16-byte group, computed on the FMA pipe: the ALU pipe is the limiter
+// of the scan, and a shift-and-mask costs it two instructions per base.  w * 2^(24-8j) puts byte j at the top,
+// mulhi(., 2^8) brings it down alone and * row_bytes scales it.  The multipliers come from the kernel arguments
+// (MidScanArgs::byte_mul = {2^24, 2^16, 2^8, row bytes}) so that ptxas cannot turn the multiplies back into shifts.
+static __device__ __forceinline__ u32 mid_row_off(const u32 (&wd)[4], int j, const u32 (&mul)[4]) {
+    const u32 w = wd[j >> 2];
+    const u32 top = (j & 3) == 3 ? w : w * mul[j & 3];
+    return __umulhi(top, mul[2]) * mul[3];
 }
 
 template <int NW, int AP>
 __global__ void __launch_bounds__(MID_THREADS, (NW * AP <= 2) ? 6 : 3)
-k_mid_scan_dyn(DevBatch B, AdapterCtx C, MidScanArgs M, const ChunkEntry *__restrict__ chunks,
-               const u32 *__restrict__ perm, const u32 *__restrict__ n_chunks_ptr,
-               uint8_t *__restrict__ chunk_min,
+k_mid_scan_dyn(DevBatch B, AdapterCtx C, MidScanArgs M, const u32 *__restrict__ chunk_off,
+               const ChunkEntry *__restrict__ runs, const u32 *__restrict__ perm,
+               const u32 *__restrict__ n_runs_ptr, uint8_t *__restrict__ chunk_min,
                u32 *__restrict__ chunk_cnt, u64 *__restrict__ chunk_first,
                u32 *__restrict__ best_mid, u32 *__restrict__ work_ctr) {
-    const u32 n_chunks = *n_chunks_ptr; // device-side total (chunk_off[n_reads])
+    const u32 n_runs = *n_runs_ptr; // device-side total (run_off[n_reads])
     extern __shared__ __align__(16) u64 s_peq_smem[]; // [256][AP][NW] top-padded tables
     DevAdapter A[AP];
 #pragma unroll
@@ -116,7 +137,8 @@ k_mid_scan_dyn(DevBatch B, AdapterCtx C, MidScanArgs M, const ChunkEntry *__rest
         __syncthreads();
     }
     constexpr int TS = AP * NW; // table stride per byte value (in u64)
-    const u64 chunk_len = 1ull << M.chunk_shift;
+    const int cs = M.chunk_shift;
+    const u64 chunk_len = 1ull << cs;
     int halo = 0, qmin = 0x7fffffff;
 #pragma unroll
     for (int x = 0; x < AP; ++x) {
@@ -124,31 +146,37 @@ k_mid_scan_dyn(DevBatch B, AdapterCtx C, MidScanArgs M, const ChunkEntry *__rest
         qmin = min(qmin, A[x].qlen);
     }
     const uint4 *__restrict__ b16 = (const uint4 *)B.bases;
+    // The chunk minimum so far is kept as the replay threshold thr = 2 * min(k, best - 1) + 8 = min(2k + 8,
+    // 2 * best + 6).  An 8-column group that starts at score s_0 and ends at s_8 has a minimum
+    // >= floor((s_0 + s_8 - 7) / 2) (adjacent columns differ by at most 1), which can only reach min(k, best - 1)
+    // when s_0 + s_8 <= thr: one add and one compare per group.  The chunk minimum is <= k exactly when
+    // thr < thr0 = 2k + 8, and it is then (thr - 6) / 2; a larger one is never reported.
+    int thr0[AP];
+#pragma unroll
+    for (int x = 0; x < AP; ++x) thr0[x] = 2 * A[x].k_mid + 8;
 
     // Work is handed out dynamically, 32 consecutive entries of the length-descending order per warp and fetch
-    // (zeroed counter per launch): longest chunks first, and CTAs that become resident late (another batch's
-    // kernels occupied the SM when this launch started) simply take fewer chunks instead of stretching the tail.
+    // (zeroed counter per launch): longest runs first, and CTAs that become resident late (another batch's
+    // kernels occupied the SM when this launch started) simply take fewer runs instead of stretching the tail.
     const u32 lane = threadIdx.x & 31u;
     for (;;) {
         u32 it = 0;
         if (lane == 0) it = atomicAdd(work_ctr, 32u);
         it = __shfl_sync(0xffffffffu, it, 0);
-        if (it >= n_chunks) break;
+        if (it >= n_runs) break;
         it += lane;
-        if (it >= n_chunks) continue; // (the warp's next fetch ends the loop)
-        const u32 ci = perm[it]; // length-descending order: a warp's 32 chunks have the same length
-        const ChunkEntry ce = chunks[ci];
-        const u64 rs = B.offsets[ce.read];
-        const u64 re = B.offsets[ce.read + 1];
-        const i64 tsm = (i64)(re - rs) - 2 * (i64)M.end_len;
-        const u64 mb = rs + (u64)M.end_len, me = re - (u64)M.end_len; // middle window
-        const u64 cb = (u64)ce.chunk << M.chunk_shift;
-        const u64 ob = max(cb, mb), oe = min(cb + chunk_len, me);     // columns this chunk reports
-        u64 sb = ob > (u64)halo ? ob - (u64)halo : 0;                   // restart point
-        if (sb < mb) sb = mb;
+        if (it >= n_runs) continue; // (the warp's next fetch ends the loop)
+        const ChunkEntry re = runs[perm[it]]; // length-descending order: a warp's 32 runs have the same length
+        const u64 rs = B.offsets[re.read];
+        const i64 tsm = (i64)(B.offsets[re.read + 1] - rs) - 2 * (i64)M.end_len;
+        const u64 mb = rs + (u64)M.end_len, me = B.offsets[re.read + 1] - (u64)M.end_len; // middle window
+        const u32 c_first = (u32)(mb >> cs);                                               // window's first chunk
+        u32 c = max(re.chunk << M.run_shift, c_first);                                     // run's first chunk
+        const u32 c_last = min(((re.chunk + 1) << M.run_shift) - 1u, (u32)((me - 1) >> cs));
+        u32 ci = chunk_off[re.read] + (c - c_first);                                       // its chunk table index
 
         u64 Pv[AP][NW], Mv[AP][NW];
-        int score[AP], best[AP];
+        int score[AP], thr[AP];
         bool on[AP];
 #pragma unroll
         for (int x = 0; x < AP; ++x) {
@@ -157,85 +185,123 @@ k_mid_scan_dyn(DevBatch B, AdapterCtx C, MidScanArgs M, const ChunkEntry *__rest
 #pragma unroll
             for (int w = 0; w < NW; ++w) { Pv[x][w] = s0.Pv[w]; Mv[x][w] = s0.Mv[w]; }
             score[x] = A[x].qlen;
-            best[x] = 0x7fffffff;
+            thr[x] = thr0[x];
             on[x] = A[x].k_mid > 0 && tsm >= (i64)A[x].qlen; // tsmLen >= qLen, T.cpp:1237
         }
-        if (tsm >= (i64)qmin) {
-            u64 p = sb;
+        const bool scan = tsm >= (i64)qmin;
+        u64 ob = max((u64)c << cs, mb);                               // first column the run reports
+        u64 sb = ob > (u64)halo ? ob - (u64)halo : 0;                  // restart point
+        if (sb < mb) sb = mb;
+        u64 p = sb;
+        if (scan) {
             // head: single bytes up to the next 16-byte boundary (first chunk of a window only)
-            while (p < oe && (p & 15ull)) {
+            const u64 oe0 = min(((u64)c << cs) + chunk_len, me);
+            while (p < oe0 && (p & 15ull)) {
                 const u64 *eq = s_peq + (u32)B.bases[p] * TS;
 #pragma unroll
                 for (int x = 0; x < AP; ++x) {
                     myers_step_state<NW>(Pv[x], Mv[x], eq + x * NW);
                     score[x] = myers_score<NW>(Pv[x], Mv[x]);
-                    if (p >= ob) best[x] = min(best[x], score[x]);
+                    if (p >= ob) thr[x] = min(thr[x], 2 * score[x] + 6);
                 }
                 ++p;
             }
-            // whole 16-byte groups: halo groups end at ob (16-aligned whenever a halo exists)
-            for (; p + 16 <= oe; p += 16) {
+            // halo: whole 16-byte groups up to ob (16-aligned whenever a halo exists), nothing tracked
+            for (; p < ob; p += 16) {
                 const uint4 v = __ldg(b16 + (p >> 4));
                 const u32 wd[4] = {v.x, v.y, v.z, v.w};
-                const bool tracked = p >= ob;
 #pragma unroll
-                for (int h = 0; h < 2; ++h) { // two 8-column groups per 16-byte load
-                    u64 Pv0[AP][NW], Mv0[AP][NW]; // state at the group start (only read on the rare path)
+                for (int j = 0; j < 16; ++j) {
+                    const u64 *eq = s_peq + ((wd[j >> 2] >> (8 * (j & 3))) & 0xffu) * TS;
 #pragma unroll
-                    for (int x = 0; x < AP; ++x)
+                    for (int x = 0; x < AP; ++x) myers_step_state<NW>(Pv[x], Mv[x], eq + x * NW);
+                }
+            }
 #pragma unroll
-                        for (int w = 0; w < NW; ++w) { Pv0[x][w] = Pv[x][w]; Mv0[x][w] = Mv[x][w]; }
+            for (int x = 0; x < AP; ++x) score[x] = myers_score<NW>(Pv[x], Mv[x]);
+        }
+        for (;;) { // the run's chunks; p >= ob here
+            const u64 cb = (u64)c << cs;
+            const u64 oe = min(cb + chunk_len, me); // the chunk reports [max(cb, mb), oe)
+            if (scan && p < oe) {
+                // whole 16-byte groups (p is 16-aligned: the head only stops short of a boundary at oe)
+                const uint4 *q = b16 + (p >> 4);
+                for (u32 g = (u32)((oe - p) >> 4); g; --g, ++q) {
+                    const uint4 v = __ldg(q);
+                    const u32 wd[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-                    for (int j = 8 * h; j < 8 * h + 8; ++j) {
-                        const u32 byte = (wd[j >> 2] >> (8 * (j & 3))) & 0xffu;
-                        const u64 *eq = s_peq + byte * TS;
+                    for (int h = 0; h < 2; ++h) { // two 8-column groups per 16-byte load
+                        u64 Pv0[AP][NW], Mv0[AP][NW]; // state at the group start (only read on the rare path)
 #pragma unroll
-                        for (int x = 0; x < AP; ++x) myers_step_state<NW>(Pv[x], Mv[x], eq + x * NW);
-                    }
-                    if (tracked) {
+                        for (int x = 0; x < AP; ++x)
+#pragma unroll
+                            for (int w = 0; w < NW; ++w) { Pv0[x][w] = Pv[x][w]; Mv0[x][w] = Mv[x][w]; }
+#pragma unroll
+                        for (int j = 8 * h; j < 8 * h + 8; ++j) {
+                            const char *row = (const char *)s_peq + mid_row_off(wd, j, M.byte_mul);
+                            u64 eq[TS]; // 16-byte loads when rows are 16-byte multiples (the offset hides that)
+                            if constexpr (TS % 2 == 0) {
+#pragma unroll
+                                for (int i = 0; i < TS; i += 2) {
+                                    const ulonglong2 v = *(const ulonglong2 *)(row + 8 * i);
+                                    eq[i] = v.x;
+                                    eq[i + 1] = v.y;
+                                }
+                            } else {
+#pragma unroll
+                                for (int i = 0; i < TS; ++i) eq[i] = *(const u64 *)(row + 8 * i);
+                            }
+#pragma unroll
+                            for (int x = 0; x < AP; ++x) myers_step_state<NW>(Pv[x], Mv[x], eq + x * NW);
+                        }
 #pragma unroll
                         for (int x = 0; x < AP; ++x) {
                             const int s_end = myers_score<NW>(Pv[x], Mv[x]);
-                            // adjacent columns differ by at most 1: group minimum >= (s_0 + s_8 - 8) / 2
-                            if (((score[x] + s_end - 8 + 1) >> 1) <= min(A[x].k_mid, best[x] - 1))
-                                best[x] = mid_replay_group<NW>(Pv0[x], Mv0[x], wd[2 * h], wd[2 * h + 1],
-                                                               s_peq + x * NW, TS, best[x]);
+                            if (score[x] + s_end <= thr[x])
+                                thr[x] = mid_replay_group<NW>(Pv0[x], Mv0[x], wd[2 * h], wd[2 * h + 1],
+                                                              s_peq + x * NW, TS, thr[x]);
                             score[x] = s_end;
                         }
                     }
                 }
-                if (!tracked && p + 16 >= ob) { // last halo group: the first tracked group needs s_0
+                p = oe & ~15ull;
+                // tail (the window's last chunk only)
+                for (; p < oe; ++p) {
+                    const u64 *eq = s_peq + (u32)B.bases[p] * TS;
 #pragma unroll
-                    for (int x = 0; x < AP; ++x) score[x] = myers_score<NW>(Pv[x], Mv[x]);
+                    for (int x = 0; x < AP; ++x) {
+                        myers_step_state<NW>(Pv[x], Mv[x], eq + x * NW);
+                        score[x] = myers_score<NW>(Pv[x], Mv[x]);
+                        thr[x] = min(thr[x], 2 * score[x] + 6);
+                    }
                 }
             }
-            // tail
-            for (; p < oe; ++p) {
-                const u64 *eq = s_peq + (u32)B.bases[p] * TS;
+            // close chunk ci
 #pragma unroll
-                for (int x = 0; x < AP; ++x) {
-                    myers_step_state<NW>(Pv[x], Mv[x], eq + x * NW);
-                    score[x] = myers_score<NW>(Pv[x], Mv[x]);
-                    if (p >= ob) best[x] = min(best[x], score[x]);
+            for (int x = 0; x < AP; ++x) {
+                uint8_t result = 255;
+                const u64 slot = (u64)M.a[x] * M.chunk_stride + ci;
+                if (on[x] && thr[x] < thr0[x]) {
+                    const int best = (thr[x] - 6) >> 1; // <= k
+                    result = (uint8_t)min(best, 254);
+                    atomicMin(best_mid + (u64)re.read * M.n_adapters + M.a[x], (u32)best);
+                    // rare: this chunk holds a candidate; record how many columns reach the chunk
+                    // minimum and the first of them so that k_mid_count never has to rescan.
+                    const u64 cob = max(cb, mb);
+                    u64 csb = cob > (u64)halo ? cob - (u64)halo : 0;
+                    if (csb < mb) csb = mb;
+                    u32 cnt;
+                    u64 first;
+                    mid_chunk_record<NW>(s_peq + x * NW, TS, A[x].qlen, B.bases, csb, cob, oe, best, cnt, first);
+                    chunk_cnt[slot] = cnt;
+                    chunk_first[slot] = first | ((u64)best << 48);
                 }
+                chunk_min[slot] = result;
+                thr[x] = thr0[x];
             }
-        }
-#pragma unroll
-        for (int x = 0; x < AP; ++x) {
-            uint8_t result = 255;
-            const u64 slot = (u64)M.a[x] * M.chunk_stride + ci;
-            if (on[x] && best[x] <= A[x].k_mid) {
-                result = (uint8_t)min(best[x], 254);
-                atomicMin(best_mid + (u64)ce.read * M.n_adapters + M.a[x], (u32)best[x]);
-                // rare: this chunk holds a candidate; record how many columns reach the chunk
-                // minimum and the first of them so that k_mid_count never has to rescan.
-                u32 cnt;
-                u64 first;
-                mid_chunk_record<NW>(s_peq + x * NW, TS, A[x].qlen, B.bases, sb, ob, oe, best[x], cnt, first);
-                chunk_cnt[slot] = cnt;
-                chunk_first[slot] = first | ((u64)best[x] << 48);
-            }
-            chunk_min[slot] = result;
+            if (c == c_last) break;
+            ++c;
+            ++ci;
         }
     }
 }

@@ -18,10 +18,12 @@ typedef unsigned int u32;
 #define SCAN_TILE_BINS 32
 #define SCAN_TILE (SCAN_BIN * SCAN_TILE_BINS) /* 3200 bases */
 // K3: the middle window is cut into 16-byte-aligned absolute chunks of 2^chunk_shift columns
-// (1024..4096, chosen per batch); each chunk is re-started a halo of q+k-1 columns early (exact
-// for scores <= k, see DESIGN.md).
+// (1024..4096, chosen per batch), the unit of the per-chunk minima.  k_mid_scan works through runs of consecutive
+// chunks, absolute blocks of 2^MID_RUN_BLOCK_SHIFT columns, and re-starts a halo of q+k-1 columns before each run
+// (exact for scores <= k, see DESIGN.md).
 #define MID_CHUNK_SHIFT_MIN 10
 #define MID_CHUNK_SHIFT_MAX 12
+#define MID_RUN_BLOCK_SHIFT 12
 
 // Per-adapter constants precomputed on the host (tgsf_create), replacing the float expressions of
 // GetEditDistance (T.cpp:1233, 1250, 1267, 1271, 1287).

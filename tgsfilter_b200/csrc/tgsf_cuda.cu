@@ -220,13 +220,14 @@ struct Slot {
     bool has_qual = false;
     // work arrays
     DBuf seg_start, seg_len, seg_sum, seg_flag, tile_cnt, tile_off, tiles;
-    DBuf read_active, piece_cnt, piece_begin, chunk_cnt, chunk_off, chunks, chunk_min, chunk_hits, chunk_first, chunk_perm, chunk_hist;
-    int chunk_shift = MID_CHUNK_SHIFT_MIN;
+    DBuf read_active, piece_cnt, piece_begin, chunk_cnt, chunk_off, chunks, chunk_min, chunk_hits, chunk_first;
+    DBuf run_cnt, run_off, runs, run_perm, run_hist; // middle-scan work items: runs of consecutive chunks
+    int chunk_shift = MID_CHUNK_SHIFT_MIN, run_shift = 0;
     DBuf best_mid, mid_n, mid_off, end_n, end_pos, pool, sortbuf, tmp, pieces, res, header;
     DBuf scan_tmp, kmer_long_list, mid_work, gz_blob, gz_spans;
     DBuf contam_cnt, contam_off, contam_chunks; // contaminant screen (only with a set installed)
     Scratch scratch, scratch2; // traceback stores: main stream (k_mid_count) / side stream (k_ends)
-    u32 pool_cap = 0, pieces_cap = 0, chunks_cap = 0, tiles_cap = 0;
+    u32 pool_cap = 0, pieces_cap = 0, chunks_cap = 0, runs_cap = 0, tiles_cap = 0;
     // host results
     HBuf h_res, h_pieces, h_header;
     u32 h_pieces_copied = 0;
@@ -264,6 +265,7 @@ struct tgsf_ctx {
     float last_kernel_ms = 0, last_total_ms = 0;
     float last_stage_ms[TGSF_N_STAGES] = {};
     int last_chunk_shift = 0; // middle-scan chunk shift of the last collected batch (tgsf_launch_shape)
+    int last_run_shift = 0;   // and its run shift (tgsf_mid_run_shift)
     cudaEvent_t ev_epoch = nullptr; // recorded at creation: origin of tgsf_last_span
     float last_span_start = 0, last_span_end = 0;
 };
@@ -311,7 +313,8 @@ int slot_init(Slot &s) {
 void slot_release(Slot &s) {
     DBuf *bufs[] = {&s.in_bases, &s.in_quals, &s.in_offsets, &s.in_packed, &s.in_exc_pos, &s.in_exc_val, &s.seg_start, &s.seg_len, &s.seg_sum,
                     &s.seg_flag, &s.tile_cnt, &s.tile_off, &s.tiles, &s.read_active, &s.piece_cnt,
-                    &s.piece_begin, &s.chunk_cnt, &s.chunk_off, &s.chunks, &s.chunk_min, &s.chunk_hits, &s.chunk_first, &s.chunk_perm, &s.chunk_hist,
+                    &s.piece_begin, &s.chunk_cnt, &s.chunk_off, &s.chunks, &s.chunk_min, &s.chunk_hits, &s.chunk_first,
+                    &s.run_cnt, &s.run_off, &s.runs, &s.run_perm, &s.run_hist,
                     &s.best_mid, &s.mid_n, &s.mid_off, &s.end_n, &s.end_pos, &s.pool, &s.sortbuf,
                     &s.tmp, &s.pieces, &s.res, &s.header, &s.scan_tmp, &s.kmer_long_list, &s.mid_work, &s.gz_blob, &s.gz_spans, &s.scratch.buf, &s.scratch2.buf,
                     &s.contam_cnt, &s.contam_off, &s.contam_chunks};
@@ -342,6 +345,11 @@ int slot_reserve(tgsf_ctx *c, Slot &s, u32 n, u64 n_bases) {
            (n_bases >> (s.chunk_shift + 1)) >= (u64)c->sm_count * 2048ull * 4ull)
         s.chunk_shift++;
     s.chunks_cap = (u32)((n_bases >> s.chunk_shift) + 2ull * n + 16);
+    // the middle scan restarts a halo per run of 2^run_shift chunks, not per chunk: runs of 4 096 columns (B200,
+    // DESIGN.md §4: with 1 024-column chunks runs of 4 beat 1, 2 and 8; with 4 096-column chunks every longer run
+    // was slower than none)
+    s.run_shift = MID_RUN_BLOCK_SHIFT - s.chunk_shift;
+    s.runs_cap = (u32)((n_bases >> (s.chunk_shift + s.run_shift)) + 2ull * n + 16);
     s.tiles_cap = (u32)(n_bases / SCAN_TILE + (u64)s.pieces_cap + 16);
     const size_t nseg = std::max<size_t>(n, s.pieces_cap) + 1;
     TRY(s.seg_start.ensure(nseg * sizeof(u64)));
@@ -360,8 +368,11 @@ int slot_reserve(tgsf_ctx *c, Slot &s, u32 n, u64 n_bases) {
     TRY(s.chunk_min.ensure((size_t)s.chunks_cap * (size_t)A));
     TRY(s.chunk_hits.ensure((size_t)s.chunks_cap * (size_t)A * sizeof(u32)));
     TRY(s.chunk_first.ensure((size_t)s.chunks_cap * (size_t)A * sizeof(u64)));
-    TRY(s.chunk_perm.ensure((size_t)s.chunks_cap * sizeof(u32)));
-    TRY(s.chunk_hist.ensure(CHUNK_BUCKETS * sizeof(u32)));
+    TRY(s.run_cnt.ensure(((size_t)n + 1) * sizeof(u32)));
+    TRY(s.run_off.ensure(((size_t)n + 2) * sizeof(u32)));
+    TRY(s.runs.ensure((size_t)s.runs_cap * sizeof(ChunkEntry)));
+    TRY(s.run_perm.ensure((size_t)s.runs_cap * sizeof(u32)));
+    TRY(s.run_hist.ensure(CHUNK_BUCKETS * sizeof(u32)));
     TRY(s.best_mid.ensure(((size_t)n * A + 1) * sizeof(u32)));
     TRY(s.mid_n.ensure(((size_t)n * A + 1) * sizeof(u32)));
     TRY(s.mid_off.ensure(((size_t)n * A + 2) * sizeof(u32)));
@@ -546,24 +557,28 @@ int launch_head(tgsf_ctx *c, Slot &s) {
             TRY(launch_ends(s.stream2, s.scratch2));
             CU(cudaEventRecord(s.ev_join, s.stream2));
         }
-        k_count_chunks<<<cdiv(n, 256), 256, 0, st>>>(s.B, s.read_active.as<int>(), P.end_len, s.chunk_shift, c->ads.min_q,
-                                                     s.chunk_cnt.as<u32>(), s.best_mid.as<u32>(),
-                                                     s.mid_n.as<u32>(), A);
+        k_count_chunks<<<cdiv(n, 256), 256, 0, st>>>(s.B, s.read_active.as<int>(), P.end_len, s.chunk_shift, s.run_shift,
+                                                     c->ads.min_q, s.chunk_cnt.as<u32>(), s.run_cnt.as<u32>(),
+                                                     s.best_mid.as<u32>(), s.mid_n.as<u32>(), A);
         c->launches++;
         TRY(exclusive_scan(c, st, s.chunk_cnt.as<u32>(), s.chunk_off.as<u32>(), n, s.scan_tmp.as<u32>(),
                            s.scan_tmp.cap / sizeof(u32)));
+        TRY(exclusive_scan(c, st, s.run_cnt.as<u32>(), s.run_off.as<u32>(), n, s.scan_tmp.as<u32>(),
+                           s.scan_tmp.cap / sizeof(u32)));
+        const int run_block = s.chunk_shift + s.run_shift;
         k_fill_chunks<<<cdiv(n, 256), 256, 0, st>>>(s.B, s.chunk_off.as<u32>(), P.end_len, s.chunk_shift, s.chunks.as<ChunkEntry>());
-        c->launches++;
-        CU(cudaMemsetAsync(s.chunk_hist.p, 0, CHUNK_BUCKETS * sizeof(u32), st));
-        k_chunk_hist<<<cdiv(n, UTIL_THREADS), UTIL_THREADS, 0, st>>>(s.B, s.chunk_off.as<u32>(), s.chunks.as<ChunkEntry>(),
-                                                                   P.end_len, s.chunk_shift, s.chunk_hist.as<u32>());
-        k_chunk_base<<<1, 32, 0, st>>>(s.chunk_hist.as<u32>());
-        k_chunk_scatter<<<cdiv(n, UTIL_THREADS), UTIL_THREADS, 0, st>>>(s.B, s.chunk_off.as<u32>(), s.chunks.as<ChunkEntry>(),
-                                                                      P.end_len, s.chunk_shift, s.chunk_hist.as<u32>(),
-                                                                      s.chunk_perm.as<u32>());
+        k_fill_chunks<<<cdiv(n, 256), 256, 0, st>>>(s.B, s.run_off.as<u32>(), P.end_len, run_block, s.runs.as<ChunkEntry>());
+        c->launches += 2;
+        CU(cudaMemsetAsync(s.run_hist.p, 0, CHUNK_BUCKETS * sizeof(u32), st));
+        k_chunk_hist<<<cdiv(n, UTIL_THREADS), UTIL_THREADS, 0, st>>>(s.B, s.run_off.as<u32>(), s.runs.as<ChunkEntry>(),
+                                                                   P.end_len, run_block, s.run_hist.as<u32>());
+        k_chunk_base<<<1, 32, 0, st>>>(s.run_hist.as<u32>());
+        k_chunk_scatter<<<cdiv(n, UTIL_THREADS), UTIL_THREADS, 0, st>>>(s.B, s.run_off.as<u32>(), s.runs.as<ChunkEntry>(),
+                                                                      P.end_len, run_block, s.run_hist.as<u32>(),
+                                                                      s.run_perm.as<u32>());
         c->launches += 3;
         const AdapterCtx AC = c->ads.ctx();
-        const u32 *n_chunks_ptr = s.chunk_off.as<u32>() + n;
+        const u32 *n_runs_ptr = s.run_off.as<u32>() + n;
         const int res_grid = c->sm_count * c->res_ctas_per_sm;
         int mid_launch = 0;
         CU(cudaMemsetAsync(s.mid_work.p, 0, (size_t)A * sizeof(u32), st));
@@ -580,24 +595,31 @@ int launch_head(tgsf_ctx *c, Slot &s) {
                 M.a[1] = pair ? grp[i + 1] : grp[i];
                 M.end_len = P.end_len;
                 M.chunk_shift = s.chunk_shift;
+                M.run_shift = s.run_shift;
                 M.chunk_stride = s.chunks_cap;
                 M.n_adapters = A;
+                M.byte_mul[0] = 1u << 24;
+                M.byte_mul[1] = 1u << 16;
+                M.byte_mul[2] = 1u << 8;
                 TRY(for_nw(nw, [&](auto nwc) {
                     constexpr int NW = decltype(nwc)::value;
-                    auto launch = [&](auto kern, size_t smem) {
+                    // AP adapters per thread: the table row of a byte value is AP * NW words, and so is the row
+                    // stride mid_row_off scales by
+                    auto launch = [&](auto kern, size_t smem, int ap) {
+                        M.byte_mul[3] = (u32)(8 * ap * NW);
                         int occ = 0; // persistent grid: exactly the resident CTA count
                         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, MID_THREADS, smem) != cudaSuccess || occ < 1) occ = 4;
                         if (c->mid_ctas_per_sm > 0) occ = std::min(occ, c->mid_ctas_per_sm);
                         kern<<<c->sm_count * occ, MID_THREADS, smem, st>>>(
-                            s.B, AC, M, s.chunks.as<ChunkEntry>(), s.chunk_perm.as<u32>(), n_chunks_ptr,
+                            s.B, AC, M, s.chunk_off.as<u32>(), s.runs.as<ChunkEntry>(), s.run_perm.as<u32>(), n_runs_ptr,
                             s.chunk_min.as<uint8_t>(), s.chunk_hits.as<u32>(), s.chunk_first.as<u64>(),
                             s.best_mid.as<u32>(), s.mid_work.as<u32>() + mid_launch);
                     };
                     if constexpr (NW <= 4) {
-                        if (pair) launch(k_mid_scan_dyn<NW, 2>, 256 * 2 * NW * sizeof(u64));
-                        else launch(k_mid_scan_dyn<NW, 1>, 256 * NW * sizeof(u64));
+                        if (pair) launch(k_mid_scan_dyn<NW, 2>, 256 * 2 * NW * sizeof(u64), 2);
+                        else launch(k_mid_scan_dyn<NW, 1>, 256 * NW * sizeof(u64), 1);
                     } else {
-                        launch(k_mid_scan_dyn<NW, 1>, 0); // table read from global memory
+                        launch(k_mid_scan_dyn<NW, 1>, 0, 1); // table read from global memory
                     }
                     c->launches++;
                     ++mid_launch;
@@ -1305,6 +1327,7 @@ int tgsf_collect(tgsf_ctx *c, tgsf_read_result *reads, uint32_t n_reads, tgsf_pi
         c->last_stage_ms[i] = ms;
     }
     c->last_chunk_shift = s.chunk_shift;
+    c->last_run_shift = s.run_shift;
 
     auto retire = [&]() {
         s.busy = false;
@@ -1395,6 +1418,12 @@ int tgsf_launch_shape(const tgsf_ctx *c, int32_t *sm_count, int32_t *last_chunk_
     if (!c) { set_err("ctx is NULL"); return TGSF_ERR_INVALID; }
     if (sm_count) *sm_count = c->sm_count;
     if (last_chunk_shift) *last_chunk_shift = c->last_chunk_shift;
+    return TGSF_OK;
+}
+
+int tgsf_mid_run_shift(const tgsf_ctx *c, int32_t *last_run_shift) {
+    if (!c) { set_err("ctx is NULL"); return TGSF_ERR_INVALID; }
+    if (last_run_shift) *last_run_shift = c->last_run_shift;
     return TGSF_OK;
 }
 

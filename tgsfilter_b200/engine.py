@@ -240,6 +240,12 @@ class FilterEngine:
         _capi.check(self._lib.tgsf_launch_shape(self._ctx, C.byref(sm), C.byref(shift)), "tgsf_launch_shape")
         return sm.value, shift.value
 
+    def mid_run_shift(self) -> int:
+        """log2 of the chunks per middle-scan run of the last collected batch."""
+        rs = C.c_int32(0)
+        _capi.check(self._lib.tgsf_mid_run_shift(self._ctx, C.byref(rs)), "tgsf_mid_run_shift")
+        return rs.value
+
 
 def align_hw(pairs, device: int = 0) -> np.ndarray:
     """tgsf_align_hw on [(query, target, k)]: edlib HW+PATH semantics, one result per pair."""
