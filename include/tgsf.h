@@ -263,6 +263,16 @@ int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint3
                  int32_t n_lib, float min_sim, int32_t *bases_num5p, int32_t *bases_num3p,
                  int64_t *map5p, int64_t *map3p);
 
+/* Extension (no counterpart in v1.11): k-mer counts of sampled read ends for the de novo adapter assembly
+ * (--adapter-denovo).  rows: n rows of row_len bytes (ends5p or ends3p of tgsf_prepass).  Window j of a row is
+ * row[j, j+k), never wrapped, and counts only when its k bytes are all upper-case A/C/G/T; its code is 2 bits per
+ * base, A0 C1 G2 T3, first base most significant.  outer[x] / inner[x] ([4^k] u32 each) count the valid windows of
+ * k-mer x with j < split / j >= split.  k in [1, 13]; NULL rows, outer or inner with n > 0, or n x max(0,
+ * row_len - k + 1) >= 2^32, give TGSF_ERR_INVALID before the device is touched.  n = 0 (or no window) zeroes the
+ * tables without touching the device. */
+int tgsf_end_kmer_counts(int device, const uint8_t *rows, uint32_t n, uint32_t row_len, int32_t k, uint32_t split,
+                         uint32_t *outer, uint32_t *inner);
+
 /* Stand-alone adapter alignment with edlib semantics (EDLIB_MODE_HW + EDLIB_TASK_PATH,
  * include/edlib.cpp:141-296) for n independent (query, target) pairs: the unit the parity tests
  * pin against edlib's known answers.  Pair i: query = queries + q_off[i] .. q_off[i+1], likewise

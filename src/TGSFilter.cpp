@@ -74,6 +74,7 @@ struct Params {
     string ContamFile;            // --contam (extension): drop pieces that share k-mers with this FASTA
     int ContamK = 17;             // --contam-k
     float ContamFrac = 0.05f;     // --contam-frac
+    bool Denovo = false;          // --adapter-denovo (extension): assemble an end's adapter when the library has none
     uint64_t batch_bases = 64ull << 20; // bases per batch (TGSF_BATCH_MB)
 };
 
@@ -104,6 +105,7 @@ int usage() {
                  "   -s  <float>  min similarity for end adapter\n"
                  "   -S  <float>  min similarity for middle adapter\n"
                  "   -D           discard reads with middle adapter instead of split\n"
+                 "   --adapter-denovo  assemble an end's adapter from its sampled reads when no library adapter is found\n"
                  " Downsampling options:\n"
                  "   -g   <str>   genome size (k/m/g)\n"
                  "   -d   <int>   downsample to the desired coverage (requires -g) \n"
@@ -193,6 +195,7 @@ int parse_cmd(int argc, char **argv, Params *P) {
         else if (flag == "contam") { if (!need()) return 1; P->ContamFile = argv[i]; }
         else if (flag == "contamk") { if (!need()) return 1; P->ContamK = atoi(argv[i]); }
         else if (flag == "contamfrac") { if (!need()) return 1; P->ContamFrac = (float)atof(argv[i]); }
+        else if (flag == "adapterdenovo") { P->Denovo = true; }
         else if (flag == "help" || flag == "h") { usage(); return 1; }
         else { cerr << "Error: UnKnow argument -" << flag << endl; return 1; }
     }
@@ -210,6 +213,11 @@ int parse_cmd(int argc, char **argv, Params *P) {
             exit(-1);
         }
         if (access(P->ContamFile.c_str(), R_OK) != 0) { cerr << "Error: Can't find this file for --contam " << P->ContamFile << endl; exit(-1); }
+    }
+    if (P->Denovo && (!P->AdapterFile.empty() || P->OnlyQC || !P->Filter)) {
+        cerr << "Error: --adapter-denovo searches the sampled reads for adapters and cannot be combined with -a, --qc or -F"
+             << endl;
+        exit(-1);
     }
     if (P->OnlyQC) P->Filter = false;
     if (P->Filter) {
@@ -790,6 +798,118 @@ int resolve_quality(Params &P, bool has_qual, Sample &S) {
     return qType;
 }
 
+// ---- de novo adapter assembly (--adapter-denovo, an extension; tgsfilter_b200/prepass.py mirrors it) ----------------
+// The constants are chosen for synthetic reads with one planted adapter per end; they have not been checked on real kits.
+constexpr int kDenovoK = 12;          // k-mer size of the counts
+constexpr int kDenovoSupport = 100;   // a seed occurs in at least 1/100 of the rows ...
+constexpr uint32_t kDenovoMinSeed = 20; // ... and at least 20 times
+constexpr uint64_t kDenovoEnrich = 4; // outer-half count >= 4 x (inner-half count + 1): adapters sit at the outer end
+constexpr int kDenovoMaxRun = 4;      // longest run of one base in a seed
+constexpr size_t kDenovoMinLen = 20, kDenovoMaxLen = 100; // candidate length bounds
+
+// Seed and extension over the outer / inner k-mer counts O, I of n rows (tgsf_end_kmer_counts with the split at
+// (row_len - k + 1) / 2).  The seed is the k-mer with the largest O that has >= 3 distinct bases, no run longer than
+// kDenovoMaxRun, O >= max(20, ceil(n/100)) and O >= 4 (I + 1); ties go to the smallest code.  The path grows to the
+// right, then to the left, by the neighbour with the largest O + I (A, C, G, T order breaks ties) until that total is
+// below half the seed's, the k-mer is already in the path, or the path has kDenovoMaxLen bases.  Returns "" when no
+// seed qualifies or the path is shorter than kDenovoMinLen.
+string assemble_adapter(const std::vector<uint32_t> &O, const std::vector<uint32_t> &I, uint32_t n) {
+    const int k = kDenovoK;
+    const uint32_t mask = (1u << (2 * k)) - 1;
+    const uint32_t support = std::max(kDenovoMinSeed, (n + kDenovoSupport - 1) / kDenovoSupport);
+    auto base = [&](uint32_t code, int i) { return (int)((code >> (2 * (k - 1 - i))) & 3); };
+    auto complex_enough = [&](uint32_t code) {
+        int seen = 0, run = 1, longest = 1;
+        for (int i = 0; i < k; i++) {
+            seen |= 1 << base(code, i);
+            if (i) { run = base(code, i) == base(code, i - 1) ? run + 1 : 1; longest = std::max(longest, run); }
+        }
+        return __builtin_popcount(seen) >= 3 && longest <= kDenovoMaxRun;
+    };
+    int64_t seed = -1;
+    for (uint32_t x = 0; x <= mask; x++)
+        if (O[x] >= support && O[x] >= kDenovoEnrich * ((uint64_t)I[x] + 1) && (seed < 0 || O[x] > O[(size_t)seed]) &&
+            complex_enough(x))
+            seed = x;
+    if (seed < 0) return "";
+    auto total = [&](uint32_t x) { return (uint64_t)O[x] + I[x]; };
+    const uint64_t cut = total((uint32_t)seed);
+    std::deque<int> path;
+    for (int i = 0; i < k; i++) path.push_back(base((uint32_t)seed, i));
+    std::unordered_set<uint32_t> in_path{(uint32_t)seed};
+    for (int right = 1; right >= 0; right--) {
+        while (path.size() < kDenovoMaxLen) {
+            uint32_t end = 0; // the last (right) or first (left) k - 1 bases
+            for (int i = 0; i < k - 1; i++) end = (end << 2) | (uint32_t)path[right ? path.size() - (k - 1) + i : i];
+            int best = 0;
+            uint32_t y = 0;
+            for (int b = 0; b < 4; b++) {
+                const uint32_t z = right ? ((end << 2) | b) & mask : ((uint32_t)b << (2 * (k - 1))) | end;
+                if (b == 0 || total(z) > total(y)) { best = b; y = z; }
+            }
+            if (2 * total(y) < cut || !in_path.insert(y).second) break;
+            if (right) path.push_back(best);
+            else path.push_front(best);
+        }
+    }
+    if (path.size() < kDenovoMinLen) return "";
+    string s;
+    for (int v : path) s += "ACGT"[v];
+    return s;
+}
+
+// --adapter-denovo for each end without a library pick (empty a5 / a3): assembles a candidate from that end's sampled
+// rows and scores the candidates with the library search.  A candidate is accepted as the end's adapter when its mean
+// depth (as `pick` computes it) reaches 2 x minSim and n / 100: the first rule alone accepts about two matching rows.
+void denovo_adapters(const Sample &S, float minSim, string &a5, float &d5, string &a3, float &d3) {
+    const uint32_t n = (uint32_t)S.seqNum, len = (uint32_t)S.checkLen;
+    const bool run[2] = {a5.empty(), a3.empty()};
+    const std::vector<uint8_t> *rows[2] = {&S.e5, &S.e3};
+    string cand[2];
+    if (n && (run[0] || run[1])) {
+        std::vector<uint32_t> O((size_t)1 << (2 * kDenovoK)), I(O.size());
+        const uint32_t split = (len - kDenovoK + 1) / 2; // checkLen >= 100 > k
+        for (int e = 0; e < 2; e++) {
+            if (!run[e]) continue;
+            if (tgsf_end_kmer_counts(0, rows[e]->data(), n, len, kDenovoK, split, O.data(), I.data()) != TGSF_OK)
+                die_tgsf("tgsf_end_kmer_counts");
+            cand[e] = assemble_adapter(O, I, n);
+        }
+    }
+    std::vector<const uint8_t *> lib_seq;
+    std::vector<int32_t> lib_len;
+    int slot[2] = {-1, -1};
+    for (int e = 0; e < 2; e++)
+        if (!cand[e].empty()) {
+            slot[e] = (int)lib_seq.size();
+            lib_seq.push_back((const uint8_t *)cand[e].data());
+            lib_len.push_back((int32_t)cand[e].size());
+        }
+    float dep[2] = {0, 0};
+    if (!lib_seq.empty()) {
+        std::vector<int32_t> bn((size_t)len * 4 * 2);
+        std::vector<int64_t> m5(lib_seq.size()), m3(lib_seq.size());
+        if (tgsf_prepass(0, S.e5.data(), S.e3.data(), n, len, lib_seq.data(), lib_len.data(), (int32_t)lib_seq.size(),
+                         minSim, bn.data(), bn.data() + (size_t)len * 4, m5.data(), m3.data()) != TGSF_OK)
+            die_tgsf("tgsf_prepass");
+        const std::vector<int64_t> *maps[2] = {&m5, &m3};
+        for (int e = 0; e < 2; e++) {
+            if (slot[e] < 0) continue;
+            const float meanDep = static_cast<float>((int)(*maps[e])[(size_t)slot[e]]) / cand[e].size();
+            if (meanDep >= 2 * minSim && meanDep >= n / 100.0f) dep[e] = meanDep;
+            else cand[e].clear();
+        }
+    }
+    const char *name[2] = {"5'", "3'"};
+    for (int e = 0; e < 2; e++)
+        if (run[e]) {
+            cerr << "INFO: de novo " << name[e] << " adapter: " << cand[e] << endl;
+            cerr << "INFO: mean depth of de novo " << name[e] << " adapter: " << dep[e] << endl;
+        }
+    if (run[0]) { a5 = cand[0]; d5 = dep[0]; }
+    if (run[1]) { a3 = cand[1]; d3 = dep[1]; }
+}
+
 // End trims from the base content of the sample and the adapter set (the global `adapters`, T.cpp:1324): from -a, or
 // searched for in the sample.  -A ends the run here.
 std::vector<string> resolve_adapters(Params &P, bool has_qual, const Sample &S) {
@@ -849,6 +969,7 @@ std::vector<string> resolve_adapters(Params &P, bool has_qual, const Sample &S) 
     float d5, d3;
     pick(m5, a5, d5);
     pick(m3, a3, d3);
+    if (P.Denovo) denovo_adapters(S, minSim, a5, d5, a3, d3);
     if (d5 > 5 * d3) { a3 = ""; d3 = 0; }
     else if (d3 > 5 * d5) { a5 = ""; d5 = 0; }
     cerr << "INFO: 5' adapter: " << a5 << endl;

@@ -116,6 +116,7 @@ EXPORTED_SYMBOLS = (
     "tgsf_host_free", "tgsf_submit", "tgsf_submit_packed", "tgsf_pack_bases", "tgsf_submit_device", "tgsf_collect", "tgsf_collect_gz", "tgsf_last_timing", "tgsf_last_span", "tgsf_last_stage_ms",
     "tgsf_counter_layout_get", "tgsf_counters", "tgsf_counters_reset", "tgsf_counters_device",
     "tgsf_launch_count", "tgsf_launch_shape", "tgsf_mid_run_shift", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw", "tgsf_set_contaminants",
+    "tgsf_end_kmer_counts",
 )
 
 _lib = None
@@ -163,6 +164,7 @@ def load() -> C.CDLL:
                                  C.POINTER(C.c_char_p), C.POINTER(C.c_int32), C.c_int32, C.c_float,
                                  vp, vp, vp, vp]
     lib.tgsf_align_hw.argtypes = [C.c_int, u8p, vp, u8p, vp, vp, C.c_uint32, vp]
+    lib.tgsf_end_kmer_counts.argtypes = [C.c_int, u8p, C.c_uint32, C.c_uint32, C.c_int32, C.c_uint32, vp, vp]
     lib.tgsf_set_contaminants.argtypes = [vp, u8p, u64p, C.c_uint32, C.c_int32, C.c_float, C.POINTER(C.c_uint64)]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)

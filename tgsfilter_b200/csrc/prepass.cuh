@@ -2,6 +2,7 @@
 //
 // k_base_content : counting loop of CheckBaseContent (T.cpp:1080-1095)
 // k_lib_search   : edlib loop of adapterSearch (T.cpp:1156-1176): maps[i] += mlen
+// k_end_kmers    : k-mer counts of the sampled ends for the de novo adapter assembly (extension, tgsf_end_kmer_counts)
 // k_align_pairs  : edlibAlign(HW, PATH) for independent (query, target) pairs (tgsf_align_hw)
 #pragma once
 #include "adapters.cuh"
@@ -64,6 +65,34 @@ k_lib_search(const uint8_t *__restrict__ rows, u32 n, u32 row_len, AdapterCtx C,
     }
     acc = warp_sum_i64(acc);
     if ((threadIdx.x & 31) == 0 && acc) atomicAdd((u64 *)maps, (u64)acc);
+}
+
+// k-mer counts of the sampled ends for the de novo adapter assembly (tgsf_end_kmer_counts).  One warp per row, grid
+// stride; the windows [w_lo, w_hi) of a row (window j = row[j, j+k)) are cut into 32 contiguous runs, one per lane,
+// and each lane rolls a 2-bit code (A0 C1 G2 T3, first base most significant) over its run.  A window counts only
+// when its k bytes are all upper-case A/C/G/T.  table: [4^k] u32, one band (outer or inner) per launch.
+__global__ void __launch_bounds__(PRE_THREADS)
+k_end_kmers(const uint8_t *__restrict__ rows, u32 n, u32 row_len, int k, u32 w_lo, u32 w_hi,
+            u32 *__restrict__ table) {
+    const int lane = threadIdx.x & 31;
+    const u32 wpb = PRE_THREADS / 32;
+    const u32 per_lane = (w_hi - w_lo + 31) / 32;
+    const u32 j0 = min(w_lo + lane * per_lane, w_hi), j1 = min(j0 + per_lane, w_hi);
+    if (j0 == j1) return; // no barrier below: idle lanes may leave
+    const u32 mask = (1u << (2 * k)) - 1u; // k <= 13
+    for (u32 r = blockIdx.x * wpb + (threadIdx.x >> 5); r < n; r += gridDim.x * wpb) {
+        const uint8_t *row = rows + (u64)r * row_len;
+        u32 code = 0;
+        int run = 0; // valid bases ending at column c, counted from j0
+        for (u32 c = j0; c < j1 + k - 1; ++c) {
+            const uint8_t b = __ldg(row + c);
+            const int v = b == 'A' ? 0 : b == 'C' ? 1 : b == 'G' ? 2 : b == 'T' ? 3 : -1;
+            if (v < 0) { run = 0; continue; }
+            code = ((code << 2) | (u32)v) & mask;
+            run = min(run + 1, k);
+            if (run == k) atomicAdd(table + code, 1u);
+        }
+    }
 }
 
 static __device__ __forceinline__ void fnv_mix(u32 &h, u32 v) {

@@ -1561,6 +1561,51 @@ int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint3
     return TGSF_OK;
 }
 
+int tgsf_end_kmer_counts(int device, const uint8_t *rows, uint32_t n, uint32_t row_len, int32_t k, uint32_t split,
+                         uint32_t *outer, uint32_t *inner) {
+    if (k < 1 || k > 13) { set_err("end_kmer_counts: k must be in [1,13], got %d", k); return TGSF_ERR_INVALID; }
+    if (n > 0 && (!rows || !outer || !inner)) { set_err("end_kmer_counts: NULL argument"); return TGSF_ERR_INVALID; }
+    const u64 windows = row_len >= (u32)k ? (u64)row_len - k + 1 : 0;
+    if ((u64)n * windows >= (1ull << 32)) { set_err("end_kmer_counts: 2^32 windows or more"); return TGSF_ERR_INVALID; }
+    const size_t table_bytes = ((size_t)1 << (2 * k)) * sizeof(u32);
+    if (n == 0 || windows == 0) {
+        if (outer) memset(outer, 0, table_bytes);
+        if (inner) memset(inner, 0, table_bytes);
+        return TGSF_OK;
+    }
+    CU(cudaSetDevice(device));
+    cudaDeviceProp prop;
+    CU(cudaGetDeviceProperties(&prop, device));
+    DBuf d_rows, d_table;
+    auto cleanup = [&]() { d_rows.release(); d_table.release(); };
+    const size_t row_bytes = (size_t)n * row_len;
+    int rc = d_rows.ensure(row_bytes);
+    if (rc == TGSF_OK) rc = d_table.ensure(table_bytes);
+    if (rc != TGSF_OK) { cleanup(); return rc; }
+    cudaError_t e = cudaMemcpy(d_rows.p, rows, row_bytes, cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { set_err("end_kmer_counts upload: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+    // one band per launch into one table: at k = 12 a band's table (64 MB) stays resident in the 126 MB L2, where the
+    // two bands' tables together would not
+    const u32 grid = std::max<u32>(1, std::min<u32>(cdiv(n, PRE_THREADS / 32), (u32)prop.multiProcessorCount * 8));
+    const u32 cut = (u32)std::min<u64>(split, windows);
+    const u32 bands[2][2] = {{0, cut}, {cut, (u32)windows}};
+    uint32_t *out[2] = {outer, inner};
+    for (int b = 0; b < 2; ++b) {
+        e = cudaMemset(d_table.p, 0, table_bytes);
+        if (e != cudaSuccess) { set_err("end_kmer_counts: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+        if (bands[b][1] > bands[b][0]) {
+            k_end_kmers<<<grid, PRE_THREADS>>>(d_rows.as<uint8_t>(), n, row_len, k, bands[b][0], bands[b][1],
+                                               d_table.as<u32>());
+            rc = check_launch("k_end_kmers");
+            if (rc != TGSF_OK) { cleanup(); return rc; }
+        }
+        e = cudaMemcpy(out[b], d_table.p, table_bytes, cudaMemcpyDeviceToHost);
+        if (e != cudaSuccess) { set_err("end_kmer_counts download: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+    }
+    cleanup();
+    return TGSF_OK;
+}
+
 int tgsf_align_hw(int device, const uint8_t *queries, const uint32_t *q_off, const uint8_t *targets,
                   const uint32_t *t_off, const int32_t *k, uint32_t n, tgsf_align_result *out) {
     if (!q_off || !t_off || !k || !out) { set_err("align: NULL argument"); return TGSF_ERR_INVALID; }
