@@ -106,6 +106,7 @@ typedef struct tgsf_piece {
 #define TGSF_PIECE_LOWQ 2         /* DropInfo[13]/[14] (T.cpp:1995-2000) */
 #define TGSF_PIECE_QC_ONLY 3      /* --qc: region kept but nothing emitted (T.cpp:1976) */
 #define TGSF_PIECE_CONTAM 4       /* contaminant screen: hit share >= min_frac (tgsf_set_contaminants) */
+#define TGSF_PIECE_FOLDBACK 5     /* fold-back screen: the kept arm is shorter than min_len (tgsf_set_foldback) */
 
 /* Layout (in uint64 words) of the cumulative counter block.  Every member is a sum, so blocks of
  * different GPUs combine with one allreduce(sum, u64).  [x][5] = {A,T,G,C,all} as in T.cpp:1462-1476. */
@@ -205,6 +206,37 @@ int tgsf_collect(tgsf_ctx *ctx, tgsf_read_result *reads, uint32_t n_reads, tgsf_
 int tgsf_set_contaminants(tgsf_ctx *ctx, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs, int32_t k,
                           float min_frac, uint64_t *n_kmers);
 
+/* Fold-back screen (an extension; the reference has none).  A piece that reads through a junction without adapter
+ * is one strand followed by its own reverse complement, X·rc(X').  Rules, on piece-relative positions of s[0, L):
+ * window i = s[i, i+15), valid when its 15 bytes are A/C/G/T in either case; codes A0 C1 G2 T3, first base most
+ * significant; key = min(f, r) of the forward and reverse-complement codes, o = (f < r) ? 0 : 1.  A window is
+ * sampled iff (fmix32(key) & 7) == 0 (murmur3's finaliser).  An anchor is a key that occurs among the sampled windows
+ * exactly once with o = 0 (at p0) and exactly once with o = 1 (at p1); d = p0 + p1 + 15, g = |p1 - p0| - 15.  The
+ * peak is the bin b (of d >> 7) maximising n[b] + n[b+1], smallest b on ties; V = the anchors of bins b and b+1,
+ * c = floor(sum d / 2V).  The piece is cut iff V >= 8, min g <= 500 (over those anchors), 400 V >= min(c, L - c) and
+ * 0 < c < L: it keeps its longer arm, [0, c) if c >= L - c, else [c, L), and becomes TGSF_PIECE_FOLDBACK when that
+ * arm is shorter than min_len (sum_q = 0, repeat_len = -1, no counter).  One fold per piece.
+ * With enable = 1, every piece the length filter kept (not with TGSF_FLAG_ONLY_QC) is screened, before the repeat
+ * check, so the repeat check, the contaminant screen, the clean step and the deflate blocks all see the kept arm; the
+ * kernels are timed in TGSF_STAGE_KMER.  enable 0 or 1, otherwise TGSF_ERR_INVALID; TGSF_ERR_STATE while a batch is
+ * outstanding. */
+int tgsf_set_foldback(tgsf_ctx *ctx, int32_t enable);
+/* Cumulative since create or tgsf_counters_reset (all batches must have been collected): out[0] pieces cut, out[1]
+ * bases removed by the cuts, out[2] of those pieces the ones dropped as TGSF_PIECE_FOLDBACK, out[3] the kept-arm
+ * bases of the dropped ones.  Zero while the screen was never enabled. */
+int tgsf_foldback_stats(tgsf_ctx *ctx, uint64_t out[4]);
+/* The screen's kernels on n stand-alone pieces seq[offsets[i], offsets[i+1]) (host buffers, offsets[0] == 0, each
+ * piece < 2^31 bases): fold = c when the piece would be cut, else -1; anchors = V; centre = c (-1 without anchors);
+ * min_gap = min g over the peak anchors (-1 without anchors).  Bad arguments give TGSF_ERR_INVALID before the device
+ * is touched; n = 0 touches nothing. */
+typedef struct tgsf_fold_result {
+    int32_t fold;
+    int32_t anchors;
+    int32_t centre;
+    int32_t min_gap;
+} tgsf_fold_result;
+int tgsf_fold_detect(int device, const uint8_t *seq, const uint64_t *offsets, uint32_t n, tgsf_fold_result *out);
+
 /* Device time (ms, CUDA events on the slot's stream) of the batch retired by the last collect:
  * kernels only, and H2D+kernels+D2H. */
 int tgsf_last_timing(tgsf_ctx *ctx, float *kernel_ms, float *total_ms);
@@ -217,7 +249,7 @@ int tgsf_last_timing(tgsf_ctx *ctx, float *kernel_ms, float *total_ms);
 #define TGSF_STAGE_MID_SCAN 2    /* K3 k_mid_scan, all adapters (chunk table included) */
 #define TGSF_STAGE_RESOLVE 3     /* K3 k_mid_count + k_ends (start search, traceback, thresholds) */
 #define TGSF_STAGE_REGIONS 4     /* K3 k_mid_emit + K5 regions / piece compaction */
-#define TGSF_STAGE_KMER 5        /* K4 + the contaminant screen */
+#define TGSF_STAGE_KMER 5        /* the fold-back screen + K4 + the contaminant screen */
 #define TGSF_STAGE_CLEAN 6       /* K1 over the kept pieces + clean decisions + clean 5'/3' */
 int tgsf_last_stage_ms(tgsf_ctx *ctx, float *out, int n);
 

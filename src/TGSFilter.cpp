@@ -74,6 +74,7 @@ struct Params {
     string ContamFile;            // --contam (extension): drop pieces that share k-mers with this FASTA
     int ContamK = 17;             // --contam-k
     float ContamFrac = 0.05f;     // --contam-frac
+    bool Foldback = false;        // --foldback (extension): cut pieces at a fold-back junction, keep the longer arm
     bool Denovo = false;          // --adapter-denovo (extension): assemble an end's adapter when the library has none
     uint64_t batch_bases = 64ull << 20; // bases per batch (TGSF_BATCH_MB)
 };
@@ -124,6 +125,8 @@ int usage() {
                  "   --contam <str>        FASTA[.gz] of contaminant sequences; pieces sharing enough k-mers are discarded\n"
                  "   --contam-k <int>      k-mer size of the contaminant screen, 11-31 [17]\n"
                  "   --contam-frac <float> min fraction of a piece's k-mers found in the set to discard it [0.05]\n"
+                 " Fold-back screen:\n"
+                 "   --foldback            cut reads that fold back onto their own reverse complement, keep the longer arm\n"
                  "   -h           show help [b200 host of v1.11]\n\n";
     return 1;
 }
@@ -196,6 +199,7 @@ int parse_cmd(int argc, char **argv, Params *P) {
         else if (flag == "contamk") { if (!need()) return 1; P->ContamK = atoi(argv[i]); }
         else if (flag == "contamfrac") { if (!need()) return 1; P->ContamFrac = (float)atof(argv[i]); }
         else if (flag == "adapterdenovo") { P->Denovo = true; }
+        else if (flag == "foldback") { P->Foldback = true; }
         else if (flag == "help" || flag == "h") { usage(); return 1; }
         else { cerr << "Error: UnKnow argument -" << flag << endl; return 1; }
     }
@@ -213,6 +217,10 @@ int parse_cmd(int argc, char **argv, Params *P) {
             exit(-1);
         }
         if (access(P->ContamFile.c_str(), R_OK) != 0) { cerr << "Error: Can't find this file for --contam " << P->ContamFile << endl; exit(-1); }
+    }
+    if (P->Foldback && (P->OnlyQC || P->ONLYAD || !P->Filter)) {
+        cerr << "Error: --foldback screens filtered reads and cannot be combined with --qc, -A or -F" << endl;
+        exit(-1);
     }
     if (P->Denovo && (!P->AdapterFile.empty() || P->OnlyQC || !P->Filter)) {
         cerr << "Error: --adapter-denovo searches the sampled reads for adapters and cannot be combined with -a, --qc or -F"
@@ -991,7 +999,7 @@ std::vector<string> resolve_adapters(Params &P, bool has_qual, const Sample &S) 
     return adapters;
 }
 
-// ---- contexts: one per GPU, with the contaminant set (--contam) installed on each ------------------------
+// ---- contexts: one per GPU, with the contaminant set (--contam) and the fold-back screen (--foldback) on each ------------------------
 std::vector<tgsf_ctx *> create_contexts(const Params &P, int qType, const std::vector<string> &adapters, bool gz_gpu,
                                         std::vector<uint8_t> &contam_seq, const std::vector<uint64_t> &contam_offs) {
     tgsf_params tp;
@@ -1031,6 +1039,9 @@ std::vector<tgsf_ctx *> create_contexts(const Params &P, int qType, const std::v
         cerr << "INFO: " << n_kmers << " distinct " << P.ContamK << "-mers loaded from " << P.ContamFile << "." << endl;
         std::vector<uint8_t>().swap(contam_seq);
     }
+    if (P.Foldback)
+        for (int g = 0; g < P.gpus; g++)
+            if (tgsf_set_foldback(ctx[(size_t)g], 1) != TGSF_OK) die_tgsf("tgsf_set_foldback");
     return ctx;
 }
 
@@ -1556,6 +1567,17 @@ void report_filter(const Params &P, std::vector<tgsf_ctx *> &ctx, const MainPass
             cerr << "INFO: " << D[15] << " reads were discarded with " << D[16] << " bases due to short repeat length." << endl;
         if (!P.ContamFile.empty())
             cerr << "INFO: " << w.contamNum << " reads were discarded with " << w.contamBases << " bases as contaminant." << endl;
+        if (P.Foldback) {
+            uint64_t F[4] = {0, 0, 0, 0};
+            for (tgsf_ctx *c : ctx) {
+                uint64_t f[4];
+                if (tgsf_foldback_stats(c, f) != TGSF_OK) die_tgsf("tgsf_foldback_stats");
+                for (int i = 0; i < 4; i++) F[i] += f[i];
+            }
+            cerr << "INFO: " << F[0] << " reads were cut at a fold-back junction, removing " << F[1] << " bases." << endl;
+            cerr << "INFO: " << F[2] << " reads were discarded with " << F[3] << " bases as too short after a fold-back cut."
+                 << endl;
+        }
         cerr << "INFO: " << w.cleanNum << " reads with a total of " << w.cleanBases << " bases after filtering." << endl;
         if (!P.Downsample && !P.OutFile.empty()) cerr << "INFO: Filtered reads were written to: " << P.OutFile << "." << endl;
     }

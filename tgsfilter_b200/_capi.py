@@ -26,7 +26,7 @@ FLAG_GZ_BLOCKS = 8
 FLAG_GZ_FASTA = 16
 
 READ_EVALUATED, READ_LOWQ, READ_EMPTY = 0, 1, 2
-PIECE_EMIT, PIECE_SHORT_REPEAT, PIECE_LOWQ, PIECE_QC_ONLY, PIECE_CONTAM = 0, 1, 2, 3, 4
+PIECE_EMIT, PIECE_SHORT_REPEAT, PIECE_LOWQ, PIECE_QC_ONLY, PIECE_CONTAM, PIECE_FOLDBACK = 0, 1, 2, 3, 4, 5
 
 N_STAGES = 7
 STAGE_NAMES = ("raw_scan", "raw_final", "mid_scan", "resolve", "regions", "kmer", "clean")
@@ -109,6 +109,7 @@ PIECE_DTYPE = [("sum_q", "<u8"), ("read", "<i4"), ("start", "<i4"), ("len", "<i4
 ALIGN_RESULT_DTYPE = [("edit_distance", "<i4"), ("n_locations", "<i4"), ("align_len", "<i4"),
                       ("first_start", "<i4"), ("first_end", "<i4"), ("last_start", "<i4"),
                       ("last_end", "<i4"), ("loc_hash", "<u4")]
+FOLD_RESULT_DTYPE = [("fold", "<i4"), ("anchors", "<i4"), ("centre", "<i4"), ("min_gap", "<i4")]
 
 # every symbol include/tgsf.h declares; tests check the built library exports all of them
 EXPORTED_SYMBOLS = (
@@ -116,7 +117,7 @@ EXPORTED_SYMBOLS = (
     "tgsf_host_free", "tgsf_submit", "tgsf_submit_packed", "tgsf_pack_bases", "tgsf_submit_device", "tgsf_collect", "tgsf_collect_gz", "tgsf_last_timing", "tgsf_last_span", "tgsf_last_stage_ms",
     "tgsf_counter_layout_get", "tgsf_counters", "tgsf_counters_reset", "tgsf_counters_device",
     "tgsf_launch_count", "tgsf_launch_shape", "tgsf_mid_run_shift", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw", "tgsf_set_contaminants",
-    "tgsf_end_kmer_counts",
+    "tgsf_end_kmer_counts", "tgsf_set_foldback", "tgsf_foldback_stats", "tgsf_fold_detect",
 )
 
 _lib = None
@@ -166,6 +167,9 @@ def load() -> C.CDLL:
     lib.tgsf_align_hw.argtypes = [C.c_int, u8p, vp, u8p, vp, vp, C.c_uint32, vp]
     lib.tgsf_end_kmer_counts.argtypes = [C.c_int, u8p, C.c_uint32, C.c_uint32, C.c_int32, C.c_uint32, vp, vp]
     lib.tgsf_set_contaminants.argtypes = [vp, u8p, u64p, C.c_uint32, C.c_int32, C.c_float, C.POINTER(C.c_uint64)]
+    lib.tgsf_set_foldback.argtypes = [vp, C.c_int32]
+    lib.tgsf_foldback_stats.argtypes = [vp, u64p]
+    lib.tgsf_fold_detect.argtypes = [C.c_int, u8p, u64p, C.c_uint32, vp]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)
         if fn.restype is C.c_int and name not in ("tgsf_version", "tgsf_last_error",

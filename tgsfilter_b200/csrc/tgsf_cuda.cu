@@ -15,6 +15,7 @@
 #include "adapters.cuh"
 #include "common.cuh"
 #include "contam.cuh"
+#include "foldback.cuh"
 #include "kmer.cuh"
 #include "kmer16.cuh"
 #include "gzenc.cuh"
@@ -204,6 +205,7 @@ struct DevHeader { // small block mirrored to the host with every batch
     unsigned long long gz_cursor; // bytes of deflate blocks produced
     u32 kmer_work;   // k_kmer_tag16: next piece to take
     u32 kmer_long;   // pieces it left for k_kmer_smem (too long for 16-bit positions)
+    u32 fold_work, fold_long, fold_long_work; // fold-back screen: next piece, long-list size, next long piece
 };
 
 struct Slot {
@@ -226,6 +228,7 @@ struct Slot {
     DBuf best_mid, mid_n, mid_off, end_n, end_pos, pool, sortbuf, tmp, pieces, res, header;
     DBuf scan_tmp, kmer_long_list, mid_work, gz_blob, gz_spans;
     DBuf contam_cnt, contam_off, contam_chunks; // contaminant screen (only with a set installed)
+    DBuf fold_long_list, fold_ws;                // fold-back screen (only while enabled)
     Scratch scratch, scratch2; // traceback stores: main stream (k_mid_count) / side stream (k_ends)
     u32 pool_cap = 0, pieces_cap = 0, chunks_cap = 0, runs_cap = 0, tiles_cap = 0;
     // host results
@@ -253,6 +256,8 @@ struct tgsf_ctx {
     DevParams P{};
     AdapterSet ads;
     ContamSet contam;
+    bool foldback = false;
+    DBuf fold_stats; // u64[4] (tgsf_foldback_stats), allocated when the screen is first enabled
     DBuf counters;
     std::vector<Slot> slots;
     u32 head = 0, tail = 0, outstanding = 0; // ring: submit at head, collect at tail
@@ -317,7 +322,7 @@ void slot_release(Slot &s) {
                     &s.run_cnt, &s.run_off, &s.runs, &s.run_perm, &s.run_hist,
                     &s.best_mid, &s.mid_n, &s.mid_off, &s.end_n, &s.end_pos, &s.pool, &s.sortbuf,
                     &s.tmp, &s.pieces, &s.res, &s.header, &s.scan_tmp, &s.kmer_long_list, &s.mid_work, &s.gz_blob, &s.gz_spans, &s.scratch.buf, &s.scratch2.buf,
-                    &s.contam_cnt, &s.contam_off, &s.contam_chunks};
+                    &s.contam_cnt, &s.contam_off, &s.contam_chunks, &s.fold_long_list, &s.fold_ws};
     for (DBuf *b : bufs) b->release();
     s.h_res.release();
     s.h_pieces.release();
@@ -717,6 +722,26 @@ int launch_contam(tgsf_ctx *c, Slot &s) {
     return check_launch("contam");
 }
 
+// Fold-back screen over the pieces K5 emitted, before K4: the shared-memory path for every piece, then the global
+// path for the pieces it handed over.  Writes piece fields and the context's fold statistics only.
+int launch_fold(tgsf_ctx *c, Slot &s, tgsf_piece *pieces, const u32 *n_pieces, DevHeader *H, tgsf_fold_result *out,
+                u32 max_len) {
+    cudaStream_t st = s.stream;
+    const u32 bins_cap = fold_bins(std::max<u32>(max_len, FOLD_K));
+    const u32 grid = (u32)c->sm_count;
+    TRY(s.fold_long_list.ensure((size_t)std::max<u32>(s.pieces_cap, 1) * sizeof(u32)));
+    TRY(s.fold_ws.ensure((size_t)grid * fold_ws_bytes(bins_cap)));
+    unsigned long long *stats = out ? nullptr : c->fold_stats.as<unsigned long long>();
+    k_fold_smem<<<grid, FOLD_THREADS, FOLD_SMEM_BYTES, st>>>(s.B, pieces, n_pieces, &H->fold_work,
+                                                             s.fold_long_list.as<u32>(), &H->fold_long, c->P.min_len,
+                                                             stats, out, &H->status);
+    k_fold_global<<<grid, FOLD_THREADS, 0, st>>>(s.B, pieces, s.fold_long_list.as<u32>(), &H->fold_long,
+                                                 &H->fold_long_work, s.fold_ws.as<uint8_t>(), bins_cap, c->P.min_len,
+                                                 stats, out, &H->status);
+    c->launches += 2;
+    return check_launch("fold");
+}
+
 // From the region pool onwards; re-runnable after a pool overflow (touches no counter before the
 // overflow check has passed).
 int launch_tail(tgsf_ctx *c, Slot &s) {
@@ -771,6 +796,8 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
     c->launches++;
     CU(cudaEventRecord(s.ev_stage[5], st));
     if (!(P.flags & TGSF_FLAG_ONLY_QC)) {
+        if (c->foldback)
+            TRY(launch_fold(c, s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, nullptr, P.L.max_bins * SCAN_BIN));
         if (P.min_repeat > 0) TRY(launch_kmer(c, s, P));
         if (c->contam.installed()) TRY(launch_contam(c, s));
         CU(cudaEventRecord(s.ev_stage[6], st));
@@ -947,6 +974,7 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
         if (e4 == cudaSuccess) e4 = cudaFuncSetAttribute(k_kmer_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SB_SMEM_BYTES);
         if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_kmer_tag16, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER16_SMEM_BYTES);
         if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_contam_screen<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, CONTAM_PF_SMEM_BYTES);
+        if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_fold_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, FOLD_SMEM_BYTES);
         if (e3 == cudaSuccess) {
             int occ = 0;
             if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_kmer_tag16, KMER16_THREADS, KMER16_SMEM_BYTES) == cudaSuccess && occ >= 1)
@@ -973,6 +1001,7 @@ int tgsf_destroy(tgsf_ctx *c) {
     if (c->ev_epoch) cudaEventDestroy(c->ev_epoch);
     c->ads.release();
     c->contam.release();
+    c->fold_stats.release();
     c->counters.release();
     delete c;
     return TGSF_OK;
@@ -1046,6 +1075,94 @@ int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offse
     next.table.p = next.pf_bits.p = nullptr;
     *n_kmers = c->contam.n_keys;
     return TGSF_OK;
+}
+
+int tgsf_set_foldback(tgsf_ctx *c, int32_t enable) {
+    if (!c) { set_err("tgsf_set_foldback: ctx is NULL"); return TGSF_ERR_INVALID; }
+    if (enable != 0 && enable != 1) { set_err("tgsf_set_foldback: enable must be 0 or 1, got %d", enable); return TGSF_ERR_INVALID; }
+    if (c->outstanding) { set_err("tgsf_set_foldback with %u batch(es) outstanding", c->outstanding); return TGSF_ERR_STATE; }
+    if (enable && !c->fold_stats.p) {
+        CU(cudaSetDevice(c->device));
+        TRY(c->fold_stats.ensure(4 * sizeof(u64)));
+        CU(cudaMemset(c->fold_stats.p, 0, 4 * sizeof(u64)));
+    }
+    c->foldback = enable != 0;
+    return TGSF_OK;
+}
+
+int tgsf_foldback_stats(tgsf_ctx *c, uint64_t out[4]) {
+    if (!c || !out) { set_err("tgsf_foldback_stats: NULL argument"); return TGSF_ERR_INVALID; }
+    if (c->outstanding) { set_err("collect all batches first"); return TGSF_ERR_STATE; }
+    if (!c->fold_stats.p) {
+        memset(out, 0, 4 * sizeof(uint64_t));
+        return TGSF_OK;
+    }
+    CU(cudaSetDevice(c->device));
+    CU(cudaMemcpy(out, c->fold_stats.p, 4 * sizeof(u64), cudaMemcpyDeviceToHost));
+    return TGSF_OK;
+}
+
+int tgsf_fold_detect(int device, const uint8_t *seq, const uint64_t *offsets, uint32_t n, tgsf_fold_result *out) {
+    if (n == 0) return TGSF_OK;
+    if (!offsets || !out) { set_err("tgsf_fold_detect: NULL argument"); return TGSF_ERR_INVALID; }
+    if (offsets[0] != 0) { set_err("tgsf_fold_detect: offsets[0] must be 0"); return TGSF_ERR_INVALID; }
+    u64 longest = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        if (offsets[i + 1] < offsets[i]) { set_err("tgsf_fold_detect: offsets not ascending at %u", i); return TGSF_ERR_INVALID; }
+        longest = std::max<u64>(longest, offsets[i + 1] - offsets[i]);
+    }
+    if (longest >= (1ull << 31)) { set_err("tgsf_fold_detect: a piece of %llu bases", (unsigned long long)longest); return TGSF_ERR_INVALID; }
+    const u64 n_bytes = offsets[n];
+    if (n_bytes && !seq) { set_err("tgsf_fold_detect: seq is NULL"); return TGSF_ERR_INVALID; }
+    CU(cudaSetDevice(device));
+    // a context without adapters owns the stream, the header and the workspaces; the pieces are whole records
+    tgsf_params p;
+    memset(&p, 0, sizeof(p));
+    p.n_slots = 1;
+    tgsf_ctx *c = nullptr;
+    TRY(tgsf_create(device, &p, &c));
+    Slot &s = c->slots[0];
+    DBuf d_off, d_out;
+    auto run = [&]() -> int {
+        cudaStream_t st = s.stream;
+        s.pieces_cap = n;
+        TRY(s.in_bases.ensure(std::max<u64>(n_bytes, 1)));
+        TRY(d_off.ensure(((size_t)n + 1) * sizeof(u64)));
+        TRY(s.pieces.ensure((size_t)n * sizeof(tgsf_piece)));
+        TRY(s.header.ensure(sizeof(DevHeader)));
+        TRY(d_out.ensure((size_t)n * sizeof(tgsf_fold_result)));
+        std::vector<tgsf_piece> pc((size_t)n);
+        for (uint32_t i = 0; i < n; ++i) {
+            memset(&pc[i], 0, sizeof(tgsf_piece));
+            pc[i].read = (int32_t)i;
+            pc[i].len = (int32_t)(offsets[i + 1] - offsets[i]);
+            pc[i].repeat_len = -1;
+            pc[i].status = TGSF_PIECE_EMIT;
+        }
+        DevHeader h;
+        memset(&h, 0, sizeof(h));
+        h.tmp_cursor = n;
+        if (n_bytes) CU(cudaMemcpyAsync(s.in_bases.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(s.pieces.p, pc.data(), (size_t)n * sizeof(tgsf_piece), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(s.header.p, &h, sizeof(h), cudaMemcpyHostToDevice, st));
+        s.B.bases = s.in_bases.as<uint8_t>();
+        s.B.quals = nullptr;
+        s.B.offsets = d_off.as<u64>();
+        s.B.n_reads = n;
+        DevHeader *H = s.header.as<DevHeader>();
+        TRY(launch_fold(c, s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, d_out.as<tgsf_fold_result>(), (u32)longest));
+        CU(cudaMemcpyAsync(out, d_out.p, (size_t)n * sizeof(tgsf_fold_result), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&h, s.header.p, sizeof(h), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (h.status != DEV_STATUS_OK) { set_err("tgsf_fold_detect: device status %u", h.status); return TGSF_ERR_CUDA; }
+        return TGSF_OK;
+    };
+    const int rc = run();
+    d_off.release();
+    d_out.release();
+    tgsf_destroy(c);
+    return rc;
 }
 
 int tgsf_device_count(int *count) {
@@ -1402,6 +1519,7 @@ int tgsf_counters_reset(tgsf_ctx *c) {
     if (c->outstanding) { set_err("collect all batches first"); return TGSF_ERR_STATE; }
     CU(cudaSetDevice(c->device));
     CU(cudaMemset(c->counters.p, 0, (size_t)c->P.L.n_u64 * sizeof(u64)));
+    if (c->fold_stats.p) CU(cudaMemset(c->fold_stats.p, 0, 4 * sizeof(u64)));
     return TGSF_OK;
 }
 

@@ -86,6 +86,17 @@ class FilterEngine:
                                                      min_frac, C.byref(n)), "tgsf_set_contaminants")
         return int(n.value)
 
+    # -- fold-back screen ------------------------------------------------------------------------
+    def set_foldback(self, enable: bool = True) -> None:
+        """tgsf_set_foldback: cut every later batch's pieces at a fold-back junction (keep the longer arm)."""
+        _capi.check(self._lib.tgsf_set_foldback(self._ctx, 1 if enable else 0), "tgsf_set_foldback")
+
+    def foldback_stats(self) -> Tuple[int, int, int, int]:
+        """(pieces cut, bases removed, pieces dropped as too short, their kept-arm bases), cumulative."""
+        out = np.zeros(4, dtype=np.uint64)
+        _capi.check(self._lib.tgsf_foldback_stats(self._ctx, out.ctypes.data), "tgsf_foldback_stats")
+        return tuple(int(x) for x in out)
+
     # -- batches --------------------------------------------------------------------------------
     def submit(self, batch) -> None:
         bases = np.ascontiguousarray(batch.bases, dtype=np.uint8)
@@ -245,6 +256,19 @@ class FilterEngine:
         rs = C.c_int32(0)
         _capi.check(self._lib.tgsf_mid_run_shift(self._ctx, C.byref(rs)), "tgsf_mid_run_shift")
         return rs.value
+
+
+def fold_detect(seqs, device: int = 0) -> np.ndarray:
+    """tgsf_fold_detect on stand-alone pieces (bytes / str): one (fold, anchors, centre, min_gap) row per piece."""
+    lib = _capi.load()
+    recs = [s.encode() if isinstance(s, str) else bytes(s) for s in seqs]
+    offs = np.zeros(len(recs) + 1, dtype=np.uint64)
+    np.cumsum([len(r) for r in recs], out=offs[1:])
+    buf = np.frombuffer(b"".join(recs) + b"\0", dtype=np.uint8)
+    out = np.zeros(len(recs), dtype=_capi.FOLD_RESULT_DTYPE)
+    _capi.check(lib.tgsf_fold_detect(device, buf.ctypes.data, offs.ctypes.data, len(recs), out.ctypes.data),
+                "tgsf_fold_detect")
+    return out
 
 
 def align_hw(pairs, device: int = 0) -> np.ndarray:
