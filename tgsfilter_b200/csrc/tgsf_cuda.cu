@@ -8,8 +8,11 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 #include "adapters.cuh"
@@ -50,55 +53,65 @@ void set_err(const char *fmt, ...) {
         if (rc_ != TGSF_OK) return rc_; \
     } while (0)
 
-// A growable device buffer.
-struct DBuf {
+// A growable buffer that owns its memory: device memory (DBuf) or pinned host memory (HBuf).  Move-only; the
+// destructor frees.  Destructors of owned CUDA resources (this, Stream, Event) never call cudaSetDevice: the entry
+// point that owns a resource has made its device current, and tgsf_destroy makes the context's device current
+// before it deletes the context.
+template <bool Pinned>
+struct Buf {
     void *p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(Buf &&o) noexcept : p(std::exchange(o.p, nullptr)), cap(std::exchange(o.cap, 0)) {}
+    Buf &operator=(Buf &&o) noexcept {
+        if (this != &o) {
+            reset();
+            p = std::exchange(o.p, nullptr);
+            cap = std::exchange(o.cap, 0);
+        }
+        return *this;
+    }
+    ~Buf() { reset(); }
     int ensure(size_t bytes) {
         if (bytes <= cap) return TGSF_OK;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
+        reset();
         size_t want = bytes + bytes / 8 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
+        cudaError_t e = Pinned ? cudaHostAlloc(&p, want, cudaHostAllocDefault) : cudaMalloc(&p, want);
         if (e != cudaSuccess) {
-            set_err("cudaMalloc(%zu): %s", want, cudaGetErrorString(e));
+            set_err("%s(%zu): %s", Pinned ? "cudaHostAlloc" : "cudaMalloc", want, cudaGetErrorString(e));
             return TGSF_ERR_NOMEM;
         }
         cap = want;
         return TGSF_OK;
     }
-    void release() {
-        if (p) cudaFree(p);
+    void reset() {
+        if (p) Pinned ? cudaFreeHost(p) : cudaFree(p);
         p = nullptr;
         cap = 0;
     }
     template <typename T> T *as() const { return (T *)p; }
 };
+using DBuf = Buf<false>;
+using HBuf = Buf<true>;
 
-struct HBuf { // pinned host
-    void *p = nullptr;
-    size_t cap = 0;
-    int ensure(size_t bytes) {
-        if (bytes <= cap) return TGSF_OK;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        size_t want = bytes + bytes / 8 + 256;
-        cudaError_t e = cudaHostAlloc(&p, want, cudaHostAllocDefault);
-        if (e != cudaSuccess) {
-            set_err("cudaHostAlloc(%zu): %s", want, cudaGetErrorString(e));
-            return TGSF_ERR_NOMEM;
-        }
-        cap = want;
-        return TGSF_OK;
-    }
-    void release() {
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-    }
-};
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+using Stream = std::unique_ptr<std::remove_pointer_t<cudaStream_t>, StreamDestroy>;
+using Event = std::unique_ptr<std::remove_pointer_t<cudaEvent_t>, EventDestroy>;
+
+int create(Stream &s) {
+    cudaStream_t h;
+    CU(cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking));
+    s.reset(h);
+    return TGSF_OK;
+}
+
+int create(Event &e, unsigned flags = cudaEventDefault) {
+    cudaEvent_t h;
+    CU(cudaEventCreateWithFlags(&h, flags));
+    e.reset(h);
+    return TGSF_OK;
+}
 
 inline int round_nw(int nw);
 
@@ -170,7 +183,6 @@ struct AdapterSet {
         c.peq_pool = d_peq.as<u64>();
         return c;
     }
-    void release() { d_ad.release(); d_peq.release(); }
 };
 
 // Per-thread traceback scratch (nw_traceback_len: one (2*nw+1)-word record per target column and thread).  The
@@ -209,11 +221,11 @@ struct DevHeader { // small block mirrored to the host with every batch
 };
 
 struct Slot {
-    cudaStream_t stream = nullptr;
-    cudaStream_t stream2 = nullptr;              // side stream: the end-window search runs next to the middle scan
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-    cudaEvent_t ev_start = nullptr, ev_k0 = nullptr, ev_k1 = nullptr, ev_end = nullptr;
-    cudaEvent_t ev_stage[TGSF_N_STAGES + 1] = {};
+    Stream stream;
+    Stream stream2; // side stream: the end-window search runs next to the middle scan
+    Event ev_fork, ev_join;
+    Event ev_start, ev_k0, ev_k1, ev_end;
+    Event ev_stage[TGSF_N_STAGES + 1];
     bool busy = false;
     // input
     DBuf in_bases, in_quals, in_offsets, in_packed, in_exc_pos, in_exc_val;
@@ -245,7 +257,6 @@ struct ContamSet {
     u64 ppm = 0;
     int k = 0;
     bool installed() const { return table.p != nullptr; }
-    void release() { table.release(); pf_bits.release(); n_keys = 0; }
 };
 
 }  // namespace
@@ -271,11 +282,15 @@ struct tgsf_ctx {
     float last_stage_ms[TGSF_N_STAGES] = {};
     int last_chunk_shift = 0; // middle-scan chunk shift of the last collected batch (tgsf_launch_shape)
     int last_run_shift = 0;   // and its run shift (tgsf_mid_run_shift)
-    cudaEvent_t ev_epoch = nullptr; // recorded at creation: origin of tgsf_last_span
+    Event ev_epoch; // recorded at creation: origin of tgsf_last_span
     float last_span_start = 0, last_span_end = 0;
 };
 
 namespace {
+
+// A context owned by the entry point that creates it, until it is handed out.
+struct CtxDestroy { void operator()(tgsf_ctx *c) const { tgsf_destroy(c); } };
+using CtxPtr = std::unique_ptr<tgsf_ctx, CtxDestroy>;
 
 inline u32 cdiv(u64 a, u64 b) { return (u32)((a + b - 1) / b); }
 
@@ -303,40 +318,13 @@ int exclusive_scan(tgsf_ctx *c, cudaStream_t st, const u32 *in, u32 *out, u32 n,
 }
 
 int slot_init(Slot &s) {
-    CU(cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&s.stream2, cudaStreamNonBlocking));
-    CU(cudaEventCreateWithFlags(&s.ev_fork, cudaEventDisableTiming));
-    CU(cudaEventCreateWithFlags(&s.ev_join, cudaEventDisableTiming));
-    CU(cudaEventCreate(&s.ev_start));
-    CU(cudaEventCreate(&s.ev_k0));
-    CU(cudaEventCreate(&s.ev_k1));
-    CU(cudaEventCreate(&s.ev_end));
-    for (auto &e : s.ev_stage) CU(cudaEventCreate(&e));
+    TRY(create(s.stream));
+    TRY(create(s.stream2));
+    TRY(create(s.ev_fork, cudaEventDisableTiming));
+    TRY(create(s.ev_join, cudaEventDisableTiming));
+    for (Event *e : {&s.ev_start, &s.ev_k0, &s.ev_k1, &s.ev_end}) TRY(create(*e));
+    for (auto &e : s.ev_stage) TRY(create(e));
     return TGSF_OK;
-}
-
-void slot_release(Slot &s) {
-    DBuf *bufs[] = {&s.in_bases, &s.in_quals, &s.in_offsets, &s.in_packed, &s.in_exc_pos, &s.in_exc_val, &s.seg_start, &s.seg_len, &s.seg_sum,
-                    &s.seg_flag, &s.tile_cnt, &s.tile_off, &s.tiles, &s.read_active, &s.piece_cnt,
-                    &s.piece_begin, &s.chunk_cnt, &s.chunk_off, &s.chunks, &s.chunk_min, &s.chunk_hits, &s.chunk_first,
-                    &s.run_cnt, &s.run_off, &s.runs, &s.run_perm, &s.run_hist,
-                    &s.best_mid, &s.mid_n, &s.mid_off, &s.end_n, &s.end_pos, &s.pool, &s.sortbuf,
-                    &s.tmp, &s.pieces, &s.res, &s.header, &s.scan_tmp, &s.kmer_long_list, &s.mid_work, &s.gz_blob, &s.gz_spans, &s.scratch.buf, &s.scratch2.buf,
-                    &s.contam_cnt, &s.contam_off, &s.contam_chunks, &s.fold_long_list, &s.fold_ws};
-    for (DBuf *b : bufs) b->release();
-    s.h_res.release();
-    s.h_pieces.release();
-    s.h_header.release();
-    if (s.ev_start) cudaEventDestroy(s.ev_start);
-    if (s.ev_k0) cudaEventDestroy(s.ev_k0);
-    if (s.ev_k1) cudaEventDestroy(s.ev_k1);
-    if (s.ev_end) cudaEventDestroy(s.ev_end);
-    for (auto &e : s.ev_stage)
-        if (e) cudaEventDestroy(e);
-    if (s.ev_fork) cudaEventDestroy(s.ev_fork);
-    if (s.ev_join) cudaEventDestroy(s.ev_join);
-    if (s.stream2) cudaStreamDestroy(s.stream2);
-    if (s.stream) cudaStreamDestroy(s.stream);
 }
 
 // Size every work array for a batch of n reads / n_bases bases.
@@ -435,7 +423,7 @@ int check_launch(const char *what) {
 
 // K1 over a segment list (raw reads or kept pieces) + tile table construction.
 int launch_scan_pass(tgsf_ctx *c, Slot &s, u32 n_seg, u64 *bin_cnt, u64 *bin_qual) {
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     const size_t scan_words = s.scan_tmp.cap / sizeof(u32);
     TRY(exclusive_scan(c, st, s.tile_cnt.as<u32>(), s.tile_off.as<u32>(), n_seg, s.scan_tmp.as<u32>(), scan_words));
     if (n_seg) {
@@ -467,20 +455,20 @@ int launch_ends_qc(tgsf_ctx *c, Slot &s, u32 n_seg, const int *flag, bool clean)
     const int grid = std::min<u32>((u32)c->sm_count * 4, cdiv(n_seg, ENDS_THREADS / 32));
     const size_t sm = c->P.bc_len <= ENDS_SMEM_ROWS ? (size_t)2 * c->P.bc_len * 10 * sizeof(u32) : 0;
     if (s.has_qual)
-        k_ends_qc<true><<<grid, ENDS_THREADS, sm, s.stream>>>(s.B.bases, s.B.quals, n_seg, s.seg_start.as<u64>(),
-                                                              s.seg_len.as<int>(), flag, c->P.bc_len, c->P.qtype,
-                                                              cnt5, q5, cnt3, q3);
+        k_ends_qc<true><<<grid, ENDS_THREADS, sm, s.stream.get()>>>(s.B.bases, s.B.quals, n_seg, s.seg_start.as<u64>(),
+                                                                    s.seg_len.as<int>(), flag, c->P.bc_len, c->P.qtype,
+                                                                    cnt5, q5, cnt3, q3);
     else
-        k_ends_qc<false><<<grid, ENDS_THREADS, sm, s.stream>>>(s.B.bases, s.B.quals, n_seg, s.seg_start.as<u64>(),
-                                                               s.seg_len.as<int>(), flag, c->P.bc_len, c->P.qtype,
-                                                               cnt5, q5, cnt3, q3);
+        k_ends_qc<false><<<grid, ENDS_THREADS, sm, s.stream.get()>>>(s.B.bases, s.B.quals, n_seg, s.seg_start.as<u64>(),
+                                                                     s.seg_len.as<int>(), flag, c->P.bc_len, c->P.qtype,
+                                                                     cnt5, q5, cnt3, q3);
     c->launches++;
     return check_launch("k_ends_qc");
 }
 
 // Everything up to (and including) the pool-size check: raw QC, quality band, K3 scans + counts.
 int launch_head(tgsf_ctx *c, Slot &s) {
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     const u32 n = s.B.n_reads;
     const int A = c->P.n_adapters;
     u64 *C = c->counters.as<u64>();
@@ -490,16 +478,16 @@ int launch_head(tgsf_ctx *c, Slot &s) {
     CU(cudaMemsetAsync(s.header.p, 0, sizeof(DevHeader), st));
     u32 *status = &s.header.as<DevHeader>()->status;
     if (n == 0) {
-        for (int i = 0; i <= 4; ++i) CU(cudaEventRecord(s.ev_stage[i], st));
+        for (int i = 0; i <= 4; ++i) CU(cudaEventRecord(s.ev_stage[i].get(), st));
         return TGSF_OK;
     }
 
-    CU(cudaEventRecord(s.ev_stage[0], st));
+    CU(cudaEventRecord(s.ev_stage[0].get(), st));
     k_read_segments<<<cdiv(n, 256), 256, 0, st>>>(s.B, s.seg_start.as<u64>(), s.seg_len.as<int>(),
                                                   s.seg_sum.as<u64>(), s.tile_cnt.as<u32>(), L.max_bins, status);
     c->launches++;
     TRY(launch_scan_pass(c, s, n, C + L.raw_bin_cnt, C + L.raw_bin_qual));
-    CU(cudaEventRecord(s.ev_stage[1], st));
+    CU(cudaEventRecord(s.ev_stage[1].get(), st));
     if (s.has_qual)
         k_finalize_raw<true><<<cdiv(n, REG_THREADS), REG_THREADS, 0, st>>>(
             s.B, P, s.seg_sum.as<u64>(), s.res.as<tgsf_read_result>(), s.read_active.as<int>(),
@@ -510,7 +498,7 @@ int launch_head(tgsf_ctx *c, Slot &s) {
             s.piece_cnt.as<u32>(), C);
     c->launches++;
     TRY(launch_ends_qc(c, s, n, nullptr, false));
-    CU(cudaEventRecord(s.ev_stage[2], st));
+    CU(cudaEventRecord(s.ev_stage[2].get(), st));
 
     const bool filter = (P.flags & TGSF_FLAG_FILTER) != 0;
     if (filter && A > 0) {
@@ -557,10 +545,10 @@ int launch_head(tgsf_ctx *c, Slot &s) {
             return TGSF_OK;
         };
         if (c->fork_ends) {
-            CU(cudaEventRecord(s.ev_fork, st));
-            CU(cudaStreamWaitEvent(s.stream2, s.ev_fork, 0));
-            TRY(launch_ends(s.stream2, s.scratch2));
-            CU(cudaEventRecord(s.ev_join, s.stream2));
+            CU(cudaEventRecord(s.ev_fork.get(), st));
+            CU(cudaStreamWaitEvent(s.stream2.get(), s.ev_fork.get(), 0));
+            TRY(launch_ends(s.stream2.get(), s.scratch2));
+            CU(cudaEventRecord(s.ev_join.get(), s.stream2.get()));
         }
         k_count_chunks<<<cdiv(n, 256), 256, 0, st>>>(s.B, s.read_active.as<int>(), P.end_len, s.chunk_shift, s.run_shift,
                                                      c->ads.min_q, s.chunk_cnt.as<u32>(), s.run_cnt.as<u32>(),
@@ -632,7 +620,7 @@ int launch_head(tgsf_ctx *c, Slot &s) {
                 }));
             }
         }
-        CU(cudaEventRecord(s.ev_stage[3], st));
+        CU(cudaEventRecord(s.ev_stage[3].get(), st));
         for (int a = 0; a < A; ++a) {
             const DevAdapter &Ah = c->ads.host[(size_t)a];
             if (Ah.k_mid <= 0) continue;
@@ -647,16 +635,16 @@ int launch_head(tgsf_ctx *c, Slot &s) {
                 return check_launch("k_mid_count");
             }));
         }
-        if (c->fork_ends) CU(cudaStreamWaitEvent(st, s.ev_join, 0)); // the end-window results (side stream)
+        if (c->fork_ends) CU(cudaStreamWaitEvent(st, s.ev_join.get(), 0)); // the end-window results (side stream)
         else TRY(launch_ends(st, s.scratch));
         TRY(exclusive_scan(c, st, s.mid_n.as<u32>(), s.mid_off.as<u32>(), n * (u32)A, s.scan_tmp.as<u32>(),
                            s.scan_tmp.cap / sizeof(u32)));
         k_check_pool<<<1, 1, 0, st>>>(s.mid_off.as<u32>() + (size_t)n * A, s.pool_cap, status);
         c->launches++;
     } else {
-        CU(cudaEventRecord(s.ev_stage[3], st));
+        CU(cudaEventRecord(s.ev_stage[3].get(), st));
     }
-    CU(cudaEventRecord(s.ev_stage[4], st));
+    CU(cudaEventRecord(s.ev_stage[4].get(), st));
     return check_launch("head");
 }
 
@@ -664,7 +652,7 @@ int launch_head(tgsf_ctx *c, Slot &s) {
 // long for its 16-bit positions to a long list, which k_kmer_smem (k <= 12) or the hash kernel k_kmer (k = 13 .. 16)
 // works through next.  k > 16: k_kmer over all pieces.
 int launch_kmer(tgsf_ctx *c, Slot &s, const DevParams &P) {
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     DevHeader *H = s.header.as<DevHeader>();
     u64 *C = c->counters.as<u64>();
     tgsf_piece *pieces = s.pieces.as<tgsf_piece>();
@@ -690,7 +678,7 @@ int launch_kmer(tgsf_ctx *c, Slot &s, const DevParams &P) {
 
 // Contaminant screen over the pieces still emitted after K4; writes piece fields only.
 int launch_contam(tgsf_ctx *c, Slot &s) {
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     const ContamSet &cs = c->contam;
     DevHeader *H = s.header.as<DevHeader>();
     const u32 cap = s.pieces_cap;
@@ -726,7 +714,7 @@ int launch_contam(tgsf_ctx *c, Slot &s) {
 // path for the pieces it handed over.  Writes piece fields and the context's fold statistics only.
 int launch_fold(tgsf_ctx *c, Slot &s, tgsf_piece *pieces, const u32 *n_pieces, DevHeader *H, tgsf_fold_result *out,
                 u32 max_len) {
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     const u32 bins_cap = fold_bins(std::max<u32>(max_len, FOLD_K));
     const u32 grid = (u32)c->sm_count;
     TRY(s.fold_long_list.ensure((size_t)std::max<u32>(s.pieces_cap, 1) * sizeof(u32)));
@@ -745,7 +733,7 @@ int launch_fold(tgsf_ctx *c, Slot &s, tgsf_piece *pieces, const u32 *n_pieces, D
 // From the region pool onwards; re-runnable after a pool overflow (touches no counter before the
 // overflow check has passed).
 int launch_tail(tgsf_ctx *c, Slot &s) {
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     const u32 n = s.B.n_reads;
     const int A = c->P.n_adapters;
     u64 *C = c->counters.as<u64>();
@@ -754,7 +742,7 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
     P.has_qual = s.has_qual;
     DevHeader *H = s.header.as<DevHeader>();
     if (n == 0) {
-        for (int i = 5; i <= TGSF_N_STAGES; ++i) CU(cudaEventRecord(s.ev_stage[i], st));
+        for (int i = 5; i <= TGSF_N_STAGES; ++i) CU(cudaEventRecord(s.ev_stage[i].get(), st));
         return TGSF_OK;
     }
     const bool filter = (P.flags & TGSF_FLAG_FILTER) != 0;
@@ -794,13 +782,13 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
                                                        s.pieces.as<tgsf_piece>(), n,
                                                        (P.flags & TGSF_FLAG_ONLY_QC) ? 1 : 0, &H->status);
     c->launches++;
-    CU(cudaEventRecord(s.ev_stage[5], st));
+    CU(cudaEventRecord(s.ev_stage[5].get(), st));
     if (!(P.flags & TGSF_FLAG_ONLY_QC)) {
         if (c->foldback)
             TRY(launch_fold(c, s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, nullptr, P.L.max_bins * SCAN_BIN));
         if (P.min_repeat > 0) TRY(launch_kmer(c, s, P));
         if (c->contam.installed()) TRY(launch_contam(c, s));
-        CU(cudaEventRecord(s.ev_stage[6], st));
+        CU(cudaEventRecord(s.ev_stage[6].get(), st));
         // clean pass over the kept pieces (T.cpp:1991-2009); piece count is device-side, the
         // kernels are launched over the capacity and bound themselves by the header.
         k_piece_segments_dyn<<<cdiv(s.pieces_cap, 256), 256, 0, st>>>(
@@ -819,7 +807,7 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
         c->launches++;
         TRY(launch_ends_qc(c, s, s.pieces_cap, s.seg_flag.as<int>(), true));
     } else {
-        CU(cudaEventRecord(s.ev_stage[6], st));
+        CU(cudaEventRecord(s.ev_stage[6].get(), st));
     }
     if ((P.flags & TGSF_FLAG_GZ_BLOCKS) && !(P.flags & TGSF_FLAG_ONLY_QC)) {
         // deflate blocks of the emitted pieces (timed with the clean stage)
@@ -832,13 +820,13 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
                                                           s.gz_spans.as<GzSpan>(), &H->gz_overflow, &H->status);
         c->launches++;
     }
-    CU(cudaEventRecord(s.ev_stage[7], st));
+    CU(cudaEventRecord(s.ev_stage[7].get(), st));
     return check_launch("tail");
 }
 
 int enqueue_d2h(tgsf_ctx *c, Slot &s) {
     (void)c;
-    cudaStream_t st = s.stream;
+    cudaStream_t st = s.stream.get();
     const u32 n = s.B.n_reads;
     CU(cudaMemcpyAsync(s.h_header.p, s.header.p, sizeof(DevHeader), cudaMemcpyDeviceToHost, st));
     if (n) CU(cudaMemcpyAsync(s.h_res.p, s.res.p, (size_t)n * sizeof(tgsf_read_result), cudaMemcpyDeviceToHost, st));
@@ -854,9 +842,9 @@ int enqueue_d2h(tgsf_ctx *c, Slot &s) {
 int run_pipeline(tgsf_ctx *c, Slot &s) {
     TRY(launch_head(c, s));
     TRY(launch_tail(c, s));
-    CU(cudaEventRecord(s.ev_k1, s.stream));
+    CU(cudaEventRecord(s.ev_k1.get(), s.stream.get()));
     TRY(enqueue_d2h(c, s));
-    CU(cudaEventRecord(s.ev_end, s.stream));
+    CU(cudaEventRecord(s.ev_end.get(), s.stream.get()));
     return TGSF_OK;
 }
 
@@ -917,7 +905,7 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
     *out = nullptr;
     TRY(validate_params(params));
     CU(cudaSetDevice(device));
-    tgsf_ctx *c = new (std::nothrow) tgsf_ctx();
+    CtxPtr c(new (std::nothrow) tgsf_ctx());
     if (!c) return TGSF_ERR_NOMEM;
     c->device = device;
     cudaDeviceProp prop;
@@ -941,55 +929,38 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
     P.has_qual = 1;
     tgsf_make_layout(params->bc_len, params->max_read_len, &P.L);
 
-    int rc = c->ads.build((const uint8_t *const *)params->adapter_seq, params->adapter_len, params->n_adapters);
-    if (rc == TGSF_OK) {
-        for (auto &A : c->ads.host) fill_thresholds(A, params);
-        rc = c->ads.upload();
-    }
-    if (rc == TGSF_OK) rc = c->counters.ensure((size_t)P.L.n_u64 * sizeof(u64));
-    if (rc == TGSF_OK && cudaMemset(c->counters.p, 0, (size_t)P.L.n_u64 * sizeof(u64)) != cudaSuccess) rc = TGSF_ERR_CUDA;
-    const int ns = params->n_slots > 0 ? params->n_slots : 2;
-    c->slots.resize((size_t)ns);
-    for (int i = 0; i < ns && rc == TGSF_OK; ++i) rc = slot_init(c->slots[(size_t)i]);
-    if (rc == TGSF_OK && (cudaEventCreate(&c->ev_epoch) != cudaSuccess ||
-                          cudaEventRecord(c->ev_epoch, c->slots[0].stream) != cudaSuccess ||
-                          cudaEventSynchronize(c->ev_epoch) != cudaSuccess)) {
-        set_err("epoch event: %s", cudaGetErrorString(cudaGetLastError()));
-        rc = TGSF_ERR_CUDA;
-    }
-    if (rc == TGSF_OK) {
-        // dynamic shared-memory limits only: no kernel asks for a carve-out (measured, DESIGN §8)
-        cudaError_t e1 = cudaFuncSetAttribute(k_scan_tiles_dyn<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
-        cudaError_t e2 = cudaFuncSetAttribute(k_scan_tiles_dyn<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES);
-        if (e1 == cudaSuccess) e1 = cudaFuncSetAttribute(k_scan_tiles_dyn<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SCAN_SMEM_BYTES_WIDE);
-        if (const char *e = getenv("TGSF_MID_CTAS")) c->mid_ctas_per_sm = atoi(e);
-        if (const char *e = getenv("TGSF_FORK_ENDS")) c->fork_ends = atoi(e) != 0;
-        if (const char *e = getenv("TGSF_RES_CTAS")) c->res_ctas_per_sm = std::max(1, std::min(16, atoi(e)));
-        // TGSF_SM_COUNT=n: size every grid and the chunk-shift rule as if the device had n SMs (clamped to
-        // [1, real count]), so that tests reach the launch shapes of multi-Gbase batches with small batches
-        if (const char *e = getenv("TGSF_SM_COUNT")) c->sm_count = std::max(1, std::min(c->sm_count, atoi(e)));
-        if (const char *e = getenv("TGSF_KMER16_LIST_CAP")) c->kmer16_list_cap = (u32)std::min<long>(std::max<long>(atol(e), 32), (long)KMER16_LIST_CAP);
-        cudaError_t e3 = cudaFuncSetAttribute(k_kmer<u32>, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SMEM_BYTES);
-        cudaError_t e4 = cudaFuncSetAttribute(k_kmer<u64>, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SMEM_BYTES);
-        if (e4 == cudaSuccess) e4 = cudaFuncSetAttribute(k_kmer_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER_SB_SMEM_BYTES);
-        if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_kmer_tag16, cudaFuncAttributeMaxDynamicSharedMemorySize, KMER16_SMEM_BYTES);
-        if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_contam_screen<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, CONTAM_PF_SMEM_BYTES);
-        if (e3 == cudaSuccess) e3 = cudaFuncSetAttribute(k_fold_smem, cudaFuncAttributeMaxDynamicSharedMemorySize, FOLD_SMEM_BYTES);
-        if (e3 == cudaSuccess) {
-            int occ = 0;
-            if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_kmer_tag16, KMER16_THREADS, KMER16_SMEM_BYTES) == cudaSuccess && occ >= 1)
-                c->kmer16_ctas_per_sm = occ;
-        }
-        if (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess || e4 != cudaSuccess) {
-            set_err("cudaFuncSetAttribute(smem): %s", cudaGetErrorString(e1 != cudaSuccess ? e1 : e2 != cudaSuccess ? e2 : e3 != cudaSuccess ? e3 : e4));
-            rc = TGSF_ERR_CUDA;
-        }
-    }
-    if (rc != TGSF_OK) {
-        tgsf_destroy(c);
-        return rc;
-    }
-    *out = c;
+    TRY(c->ads.build((const uint8_t *const *)params->adapter_seq, params->adapter_len, params->n_adapters));
+    for (auto &A : c->ads.host) fill_thresholds(A, params);
+    TRY(c->ads.upload());
+    TRY(c->counters.ensure((size_t)P.L.n_u64 * sizeof(u64)));
+    CU(cudaMemset(c->counters.p, 0, (size_t)P.L.n_u64 * sizeof(u64)));
+    c->slots.resize((size_t)(params->n_slots > 0 ? params->n_slots : 2));
+    for (auto &s : c->slots) TRY(slot_init(s));
+    TRY(create(c->ev_epoch));
+    CU(cudaEventRecord(c->ev_epoch.get(), c->slots[0].stream.get()));
+    CU(cudaEventSynchronize(c->ev_epoch.get()));
+    // dynamic shared-memory limits only: no kernel asks for a carve-out (measured, DESIGN §8)
+    auto smem = [](auto kern, int bytes) { return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); };
+    CU(smem(k_scan_tiles_dyn<true, false>, SCAN_SMEM_BYTES));
+    CU(smem(k_scan_tiles_dyn<false, false>, SCAN_SMEM_BYTES));
+    CU(smem(k_scan_tiles_dyn<true, true>, SCAN_SMEM_BYTES_WIDE));
+    CU(smem(k_kmer<u32>, KMER_SMEM_BYTES));
+    CU(smem(k_kmer<u64>, KMER_SMEM_BYTES));
+    CU(smem(k_kmer_smem, KMER_SB_SMEM_BYTES));
+    CU(smem(k_kmer_tag16, KMER16_SMEM_BYTES));
+    CU(smem(k_contam_screen<true>, CONTAM_PF_SMEM_BYTES));
+    CU(smem(k_fold_smem, FOLD_SMEM_BYTES));
+    int occ = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_kmer_tag16, KMER16_THREADS, KMER16_SMEM_BYTES) == cudaSuccess && occ >= 1)
+        c->kmer16_ctas_per_sm = occ;
+    if (const char *e = getenv("TGSF_MID_CTAS")) c->mid_ctas_per_sm = atoi(e);
+    if (const char *e = getenv("TGSF_FORK_ENDS")) c->fork_ends = atoi(e) != 0;
+    if (const char *e = getenv("TGSF_RES_CTAS")) c->res_ctas_per_sm = std::max(1, std::min(16, atoi(e)));
+    // TGSF_SM_COUNT=n: size every grid and the chunk-shift rule as if the device had n SMs (clamped to
+    // [1, real count]), so that tests reach the launch shapes of multi-Gbase batches with small batches
+    if (const char *e = getenv("TGSF_SM_COUNT")) c->sm_count = std::max(1, std::min(c->sm_count, atoi(e)));
+    if (const char *e = getenv("TGSF_KMER16_LIST_CAP")) c->kmer16_list_cap = (u32)std::min<long>(std::max<long>(atol(e), 32), (long)KMER16_LIST_CAP);
+    *out = c.release();
     return TGSF_OK;
 }
 
@@ -997,12 +968,6 @@ int tgsf_destroy(tgsf_ctx *c) {
     if (!c) return TGSF_OK;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    for (auto &s : c->slots) slot_release(s);
-    if (c->ev_epoch) cudaEventDestroy(c->ev_epoch);
-    c->ads.release();
-    c->contam.release();
-    c->fold_stats.release();
-    c->counters.release();
     delete c;
     return TGSF_OK;
 }
@@ -1025,54 +990,41 @@ int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offse
     // distinct keys <= windows < n_bytes, so a capacity >= 2 x n_bytes keeps the load <= 0.5
     u64 cap = 1024;
     while (cap < 2 * n_bytes) cap <<= 1;
-    cudaStream_t st = c->slots[0].stream;
+    cudaStream_t st = c->slots[0].stream.get();
     ContamSet next;
     DBuf d_seq, d_off, d_cnt;
-    auto build = [&]() -> int {
-        TRY(next.table.ensure(cap * sizeof(u64)));
-        TRY(d_seq.ensure(n_bytes));
-        TRY(d_off.ensure(((size_t)n_seqs + 1) * sizeof(u64)));
-        TRY(d_cnt.ensure(sizeof(unsigned long long)));
-        CU(cudaMemsetAsync(next.table.p, 0xFF, cap * sizeof(u64), st));
-        CU(cudaMemsetAsync(d_cnt.p, 0, sizeof(unsigned long long), st));
-        CU(cudaMemcpyAsync(d_seq.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n_seqs + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
-        const u64 threads = (n_bytes + CONTAM_BUILD_SEG - 1) / CONTAM_BUILD_SEG;
-        const u32 grid = (u32)std::min<u64>((threads + 255) / 256, (u64)c->sm_count * 16);
-        k_contam_build<<<grid, 256, 0, st>>>(d_seq.as<uint8_t>(), d_off.as<u64>(), n_seqs, k, next.table.as<u64>(),
-                                             cap - 1, d_cnt.as<unsigned long long>());
+    TRY(next.table.ensure(cap * sizeof(u64)));
+    TRY(d_seq.ensure(n_bytes));
+    TRY(d_off.ensure(((size_t)n_seqs + 1) * sizeof(u64)));
+    TRY(d_cnt.ensure(sizeof(unsigned long long)));
+    CU(cudaMemsetAsync(next.table.p, 0xFF, cap * sizeof(u64), st));
+    CU(cudaMemsetAsync(d_cnt.p, 0, sizeof(unsigned long long), st));
+    CU(cudaMemcpyAsync(d_seq.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n_seqs + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
+    const u64 threads = (n_bytes + CONTAM_BUILD_SEG - 1) / CONTAM_BUILD_SEG;
+    const u32 grid = (u32)std::min<u64>((threads + 255) / 256, (u64)c->sm_count * 16);
+    k_contam_build<<<grid, 256, 0, st>>>(d_seq.as<uint8_t>(), d_off.as<u64>(), n_seqs, k, next.table.as<u64>(),
+                                         cap - 1, d_cnt.as<unsigned long long>());
+    c->launches++;
+    TRY(check_launch("k_contam_build"));
+    unsigned long long n = 0;
+    CU(cudaMemcpyAsync(&n, d_cnt.p, sizeof(n), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    next.n_keys = n;
+    if (n == 0) { set_err("contaminant set has no valid %d-mer", k); return TGSF_ERR_INVALID; }
+    if (n <= CONTAM_PF_MAX_KEYS) {
+        TRY(next.pf_bits.ensure(CONTAM_PF_SMEM_BYTES));
+        CU(cudaMemsetAsync(next.pf_bits.p, 0, CONTAM_PF_SMEM_BYTES, st));
+        k_contam_bitmap<<<(u32)std::min<u64>(cap / 256 + 1, (u64)c->sm_count * 8), 256, 0, st>>>(
+            next.table.as<u64>(), cap, next.pf_bits.as<u32>());
         c->launches++;
-        TRY(check_launch("k_contam_build"));
-        unsigned long long n = 0;
-        CU(cudaMemcpyAsync(&n, d_cnt.p, sizeof(n), cudaMemcpyDeviceToHost, st));
+        TRY(check_launch("k_contam_bitmap"));
         CU(cudaStreamSynchronize(st));
-        next.n_keys = n;
-        if (n == 0) { set_err("contaminant set has no valid %d-mer", k); return TGSF_ERR_INVALID; }
-        if (n <= CONTAM_PF_MAX_KEYS) {
-            TRY(next.pf_bits.ensure(CONTAM_PF_SMEM_BYTES));
-            CU(cudaMemsetAsync(next.pf_bits.p, 0, CONTAM_PF_SMEM_BYTES, st));
-            k_contam_bitmap<<<(u32)std::min<u64>(cap / 256 + 1, (u64)c->sm_count * 8), 256, 0, st>>>(
-                next.table.as<u64>(), cap, next.pf_bits.as<u32>());
-            c->launches++;
-            TRY(check_launch("k_contam_bitmap"));
-            CU(cudaStreamSynchronize(st));
-        }
-        return TGSF_OK;
-    };
-    const int rc = build();
-    d_seq.release();
-    d_off.release();
-    d_cnt.release();
-    if (rc != TGSF_OK) {
-        next.release();
-        return rc;
     }
     next.mask = cap - 1;
     next.ppm = (u64)ppm;
     next.k = k;
-    c->contam.release();
-    c->contam = next; // takes over the buffers
-    next.table.p = next.pf_bits.p = nullptr;
+    c->contam = std::move(next); // frees the set it replaces
     *n_kmers = c->contam.n_keys;
     return TGSF_OK;
 }
@@ -1119,50 +1071,44 @@ int tgsf_fold_detect(int device, const uint8_t *seq, const uint64_t *offsets, ui
     tgsf_params p;
     memset(&p, 0, sizeof(p));
     p.n_slots = 1;
-    tgsf_ctx *c = nullptr;
-    TRY(tgsf_create(device, &p, &c));
+    tgsf_ctx *raw = nullptr;
+    TRY(tgsf_create(device, &p, &raw));
+    CtxPtr c(raw);
     Slot &s = c->slots[0];
+    cudaStream_t st = s.stream.get();
     DBuf d_off, d_out;
-    auto run = [&]() -> int {
-        cudaStream_t st = s.stream;
-        s.pieces_cap = n;
-        TRY(s.in_bases.ensure(std::max<u64>(n_bytes, 1)));
-        TRY(d_off.ensure(((size_t)n + 1) * sizeof(u64)));
-        TRY(s.pieces.ensure((size_t)n * sizeof(tgsf_piece)));
-        TRY(s.header.ensure(sizeof(DevHeader)));
-        TRY(d_out.ensure((size_t)n * sizeof(tgsf_fold_result)));
-        std::vector<tgsf_piece> pc((size_t)n);
-        for (uint32_t i = 0; i < n; ++i) {
-            memset(&pc[i], 0, sizeof(tgsf_piece));
-            pc[i].read = (int32_t)i;
-            pc[i].len = (int32_t)(offsets[i + 1] - offsets[i]);
-            pc[i].repeat_len = -1;
-            pc[i].status = TGSF_PIECE_EMIT;
-        }
-        DevHeader h;
-        memset(&h, 0, sizeof(h));
-        h.tmp_cursor = n;
-        if (n_bytes) CU(cudaMemcpyAsync(s.in_bases.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(s.pieces.p, pc.data(), (size_t)n * sizeof(tgsf_piece), cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(s.header.p, &h, sizeof(h), cudaMemcpyHostToDevice, st));
-        s.B.bases = s.in_bases.as<uint8_t>();
-        s.B.quals = nullptr;
-        s.B.offsets = d_off.as<u64>();
-        s.B.n_reads = n;
-        DevHeader *H = s.header.as<DevHeader>();
-        TRY(launch_fold(c, s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, d_out.as<tgsf_fold_result>(), (u32)longest));
-        CU(cudaMemcpyAsync(out, d_out.p, (size_t)n * sizeof(tgsf_fold_result), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(&h, s.header.p, sizeof(h), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        if (h.status != DEV_STATUS_OK) { set_err("tgsf_fold_detect: device status %u", h.status); return TGSF_ERR_CUDA; }
-        return TGSF_OK;
-    };
-    const int rc = run();
-    d_off.release();
-    d_out.release();
-    tgsf_destroy(c);
-    return rc;
+    s.pieces_cap = n;
+    TRY(s.in_bases.ensure(std::max<u64>(n_bytes, 1)));
+    TRY(d_off.ensure(((size_t)n + 1) * sizeof(u64)));
+    TRY(s.pieces.ensure((size_t)n * sizeof(tgsf_piece)));
+    TRY(s.header.ensure(sizeof(DevHeader)));
+    TRY(d_out.ensure((size_t)n * sizeof(tgsf_fold_result)));
+    std::vector<tgsf_piece> pc((size_t)n);
+    for (uint32_t i = 0; i < n; ++i) {
+        memset(&pc[i], 0, sizeof(tgsf_piece));
+        pc[i].read = (int32_t)i;
+        pc[i].len = (int32_t)(offsets[i + 1] - offsets[i]);
+        pc[i].repeat_len = -1;
+        pc[i].status = TGSF_PIECE_EMIT;
+    }
+    DevHeader h;
+    memset(&h, 0, sizeof(h));
+    h.tmp_cursor = n;
+    if (n_bytes) CU(cudaMemcpyAsync(s.in_bases.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(s.pieces.p, pc.data(), (size_t)n * sizeof(tgsf_piece), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(s.header.p, &h, sizeof(h), cudaMemcpyHostToDevice, st));
+    s.B.bases = s.in_bases.as<uint8_t>();
+    s.B.quals = nullptr;
+    s.B.offsets = d_off.as<u64>();
+    s.B.n_reads = n;
+    DevHeader *H = s.header.as<DevHeader>();
+    TRY(launch_fold(c.get(), s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, d_out.as<tgsf_fold_result>(), (u32)longest));
+    CU(cudaMemcpyAsync(out, d_out.p, (size_t)n * sizeof(tgsf_fold_result), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&h, s.header.p, sizeof(h), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (h.status != DEV_STATUS_OK) { set_err("tgsf_fold_detect: device status %u", h.status); return TGSF_ERR_CUDA; }
+    return TGSF_OK;
 }
 
 int tgsf_device_count(int *count) {
@@ -1188,7 +1134,7 @@ int tgsf_host_free(void *ptr) {
 static int grow_counters_to(tgsf_ctx *c, u32 new_bins) { // exactly new_bins bins per table
     if (new_bins <= c->P.L.max_bins) return TGSF_OK;
     for (auto &s : c->slots) // batches in flight were launched on the old block
-        if (s.busy) CU(cudaStreamSynchronize(s.stream));
+        if (s.busy) CU(cudaStreamSynchronize(s.stream.get()));
     const tgsf_counter_layout OL = c->P.L;
     tgsf_counter_layout NL;
     tgsf_make_layout(OL.bc_len, (int32_t)((u64)(new_bins - 1) * SCAN_BIN), &NL);
@@ -1202,8 +1148,7 @@ static int grow_counters_to(tgsf_ctx *c, u32 new_bins) { // exactly new_bins bin
     const u32 nsec[4] = {NL.raw_bin_cnt, NL.raw_bin_qual, NL.clean_bin_cnt, NL.clean_bin_qual};
     for (int i = 0; i < 4; ++i)
         CU(cudaMemcpy(n + nsec[i], o + osec[i], (size_t)OL.max_bins * 5 * sizeof(u64), cudaMemcpyDeviceToDevice));
-    c->counters.release();
-    c->counters = nb;
+    c->counters = std::move(nb);
     c->P.L = NL;
     return TGSF_OK;
 }
@@ -1236,7 +1181,7 @@ static int submit_common(tgsf_ctx *c, const uint8_t *bases, const uint8_t *quals
     s.has_qual = quals != nullptr;
     s.n_bases = n_bases;
     TRY(slot_reserve(c, s, n_reads, n_bases));
-    CU(cudaEventRecord(s.ev_start, s.stream));
+    CU(cudaEventRecord(s.ev_start.get(), s.stream.get()));
     if (on_device) {
         if (((uintptr_t)bases & 15) || ((uintptr_t)quals & 15)) { set_err("device streams must be 16-byte aligned"); return TGSF_ERR_INVALID; }
         s.B.bases = bases;
@@ -1252,34 +1197,34 @@ static int submit_common(tgsf_ctx *c, const uint8_t *bases, const uint8_t *quals
             TRY(s.in_packed.ensure((size_t)n_words * 4 + pad));
             if (n_bases) {
                 // the unpack kernel reads whole 32-bit words: define the bytes of the last word beyond the copy
-                CU(cudaMemsetAsync((uint8_t *)s.in_packed.p + (n_words - 1) * 4, 0, 4, s.stream));
-                CU(cudaMemcpyAsync(s.in_packed.p, pk->packed, (size_t)((n_bases + 3) / 4), cudaMemcpyHostToDevice, s.stream));
-                k_unpack_bases<<<c->sm_count * 8, 256, 0, s.stream>>>(s.in_packed.as<u32>(), n_words, s.in_bases.as<uint4>());
+                CU(cudaMemsetAsync((uint8_t *)s.in_packed.p + (n_words - 1) * 4, 0, 4, s.stream.get()));
+                CU(cudaMemcpyAsync(s.in_packed.p, pk->packed, (size_t)((n_bases + 3) / 4), cudaMemcpyHostToDevice, s.stream.get()));
+                k_unpack_bases<<<c->sm_count * 8, 256, 0, s.stream.get()>>>(s.in_packed.as<u32>(), n_words, s.in_bases.as<uint4>());
                 c->launches++;
             }
             if (pk->n_exc) {
                 TRY(s.in_exc_pos.ensure((size_t)pk->n_exc * sizeof(u64)));
                 TRY(s.in_exc_val.ensure((size_t)pk->n_exc));
-                CU(cudaMemcpyAsync(s.in_exc_pos.p, pk->exc_pos, (size_t)pk->n_exc * sizeof(u64), cudaMemcpyHostToDevice, s.stream));
-                CU(cudaMemcpyAsync(s.in_exc_val.p, pk->exc_val, (size_t)pk->n_exc, cudaMemcpyHostToDevice, s.stream));
-                k_apply_exceptions<<<c->sm_count, 256, 0, s.stream>>>(s.in_bases.as<uint8_t>(), s.in_exc_pos.as<u64>(),
-                                                                     s.in_exc_val.as<uint8_t>(), pk->n_exc);
+                CU(cudaMemcpyAsync(s.in_exc_pos.p, pk->exc_pos, (size_t)pk->n_exc * sizeof(u64), cudaMemcpyHostToDevice, s.stream.get()));
+                CU(cudaMemcpyAsync(s.in_exc_val.p, pk->exc_val, (size_t)pk->n_exc, cudaMemcpyHostToDevice, s.stream.get()));
+                k_apply_exceptions<<<c->sm_count, 256, 0, s.stream.get()>>>(s.in_bases.as<uint8_t>(), s.in_exc_pos.as<u64>(),
+                                                                           s.in_exc_val.as<uint8_t>(), pk->n_exc);
                 c->launches++;
             }
         } else if (n_bases) {
-            CU(cudaMemcpyAsync(s.in_bases.p, bases, (size_t)n_bases, cudaMemcpyHostToDevice, s.stream));
+            CU(cudaMemcpyAsync(s.in_bases.p, bases, (size_t)n_bases, cudaMemcpyHostToDevice, s.stream.get()));
         }
         if (quals) {
             TRY(s.in_quals.ensure((size_t)n_bases + pad));
-            if (n_bases) CU(cudaMemcpyAsync(s.in_quals.p, quals, (size_t)n_bases, cudaMemcpyHostToDevice, s.stream));
+            if (n_bases) CU(cudaMemcpyAsync(s.in_quals.p, quals, (size_t)n_bases, cudaMemcpyHostToDevice, s.stream.get()));
         }
-        if (n_reads) CU(cudaMemcpyAsync(s.in_offsets.p, offsets, ((size_t)n_reads + 1) * sizeof(u64), cudaMemcpyHostToDevice, s.stream));
+        if (n_reads) CU(cudaMemcpyAsync(s.in_offsets.p, offsets, ((size_t)n_reads + 1) * sizeof(u64), cudaMemcpyHostToDevice, s.stream.get()));
         s.B.bases = s.in_bases.as<uint8_t>();
         s.B.quals = quals ? s.in_quals.as<uint8_t>() : nullptr;
         s.B.offsets = s.in_offsets.as<u64>();
     }
     s.B.n_reads = n_reads;
-    CU(cudaEventRecord(s.ev_k0, s.stream));
+    CU(cudaEventRecord(s.ev_k0.get(), s.stream.get()));
     TRY(run_pipeline(c, s));
     s.busy = true;
     c->head = (c->head + 1) % (u32)c->slots.size();
@@ -1381,7 +1326,7 @@ int tgsf_collect_gz(tgsf_ctx *c, uint8_t *blob, uint64_t blob_cap, uint64_t *blo
     if (c->outstanding == 0) { set_err("nothing outstanding"); return TGSF_ERR_STATE; }
     CU(cudaSetDevice(c->device));
     Slot &s = c->slots[c->tail];
-    CU(cudaEventSynchronize(s.ev_end));
+    CU(cudaEventSynchronize(s.ev_end.get()));
     const DevHeader *H = (const DevHeader *)s.h_header.p;
     if (H->status == DEV_STATUS_POOL_OVERFLOW) { // the tail has to be re-run first: tgsf_collect does that
         set_err("collect_gz: this batch overflowed the region pool; tgsf_collect re-runs it, compress its records on the host");
@@ -1392,9 +1337,9 @@ int tgsf_collect_gz(tgsf_ctx *c, uint8_t *blob, uint64_t blob_cap, uint64_t *blo
     *blob_bytes = (uint64_t)H->gz_cursor;
     *n_spans = np;
     if (H->gz_cursor > blob_cap || np > spans_cap) { set_err("collect_gz: buffers too small"); return TGSF_ERR_CAPACITY; }
-    if (H->gz_cursor) CU(cudaMemcpyAsync(blob, s.gz_blob.p, (size_t)H->gz_cursor, cudaMemcpyDeviceToHost, s.stream));
-    if (np) CU(cudaMemcpyAsync(spans, s.gz_spans.p, (size_t)np * sizeof(tgsf_gz_span), cudaMemcpyDeviceToHost, s.stream));
-    CU(cudaStreamSynchronize(s.stream));
+    if (H->gz_cursor) CU(cudaMemcpyAsync(blob, s.gz_blob.p, (size_t)H->gz_cursor, cudaMemcpyDeviceToHost, s.stream.get()));
+    if (np) CU(cudaMemcpyAsync(spans, s.gz_spans.p, (size_t)np * sizeof(tgsf_gz_span), cudaMemcpyDeviceToHost, s.stream.get()));
+    CU(cudaStreamSynchronize(s.stream.get()));
     return TGSF_OK;
 }
 
@@ -1404,7 +1349,7 @@ int tgsf_collect(tgsf_ctx *c, tgsf_read_result *reads, uint32_t n_reads, tgsf_pi
     if (c->outstanding == 0) { set_err("nothing outstanding"); return TGSF_ERR_STATE; }
     CU(cudaSetDevice(c->device));
     Slot &s = c->slots[c->tail];
-    CU(cudaEventSynchronize(s.ev_end));
+    CU(cudaEventSynchronize(s.ev_end.get()));
     DevHeader *H = (DevHeader *)s.h_header.p;
     float extra_ms = 0;
     int guard = 0;
@@ -1415,32 +1360,30 @@ int tgsf_collect(tgsf_ctx *c, tgsf_read_result *reads, uint32_t n_reads, tgsf_pi
                       cudaMemcpyDeviceToHost));
         s.pool_cap = std::max(need + need / 4 + 1024, s.pool_cap * 2);
         TRY(slot_reserve(c, s, s.B.n_reads, s.n_bases));
-        CU(cudaMemsetAsync(s.header.p, 0, sizeof(DevHeader), s.stream));
-        cudaEvent_t e0, e1;
-        CU(cudaEventCreate(&e0));
-        CU(cudaEventCreate(&e1));
-        CU(cudaEventRecord(e0, s.stream));
+        CU(cudaMemsetAsync(s.header.p, 0, sizeof(DevHeader), s.stream.get()));
+        Event e0, e1;
+        TRY(create(e0));
+        TRY(create(e1));
+        CU(cudaEventRecord(e0.get(), s.stream.get()));
         TRY(launch_tail(c, s));
-        CU(cudaEventRecord(e1, s.stream));
+        CU(cudaEventRecord(e1.get(), s.stream.get()));
         TRY(enqueue_d2h(c, s));
-        CU(cudaStreamSynchronize(s.stream));
+        CU(cudaStreamSynchronize(s.stream.get()));
         float ms = 0;
-        cudaEventElapsedTime(&ms, e0, e1);
+        cudaEventElapsedTime(&ms, e0.get(), e1.get());
         extra_ms += ms;
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
     }
     float k_ms = 0, t_ms = 0;
-    cudaEventElapsedTime(&k_ms, s.ev_k0, s.ev_k1);
-    cudaEventElapsedTime(&t_ms, s.ev_start, s.ev_end);
+    cudaEventElapsedTime(&k_ms, s.ev_k0.get(), s.ev_k1.get());
+    cudaEventElapsedTime(&t_ms, s.ev_start.get(), s.ev_end.get());
     c->last_kernel_ms = k_ms + extra_ms;
     c->last_total_ms = t_ms + extra_ms;
-    cudaEventElapsedTime(&c->last_span_start, c->ev_epoch, s.ev_k0);
-    cudaEventElapsedTime(&c->last_span_end, c->ev_epoch, s.ev_k1);
+    cudaEventElapsedTime(&c->last_span_start, c->ev_epoch.get(), s.ev_k0.get());
+    cudaEventElapsedTime(&c->last_span_end, c->ev_epoch.get(), s.ev_k1.get());
     c->last_span_end += extra_ms;
     for (int i = 0; i < TGSF_N_STAGES; ++i) {
         float ms = 0;
-        cudaEventElapsedTime(&ms, s.ev_stage[i], s.ev_stage[i + 1]);
+        cudaEventElapsedTime(&ms, s.ev_stage[i].get(), s.ev_stage[i + 1].get());
         c->last_stage_ms[i] = ms;
     }
     c->last_chunk_shift = s.chunk_shift;
@@ -1575,24 +1518,15 @@ int tgsf_allreduce(tgsf_ctx **ctxs, int n) {
     }
     DBuf scratch;
     TRY(scratch.ensure(bytes));
-    int rc = TGSF_OK;
-    for (int i = 1; i < n && rc == TGSF_OK; ++i) {
-        if (cudaMemcpyPeer(scratch.p, root->device, ctxs[i]->counters.p, ctxs[i]->device, bytes) != cudaSuccess) {
-            set_err("allreduce: peer copy failed: %s", cudaGetErrorString(cudaGetLastError()));
-            rc = TGSF_ERR_CUDA;
-            break;
-        }
+    for (int i = 1; i < n; ++i) {
+        CU(cudaMemcpyPeer(scratch.p, root->device, ctxs[i]->counters.p, ctxs[i]->device, bytes));
         k_add_u64<<<root->sm_count, 256>>>(root->counters.as<u64>(), scratch.as<u64>(), words);
         root->launches++;
-        if (cudaDeviceSynchronize() != cudaSuccess) { set_err("allreduce: add kernel failed"); rc = TGSF_ERR_CUDA; }
+        CU(cudaDeviceSynchronize());
     }
-    for (int i = 1; i < n && rc == TGSF_OK; ++i)
-        if (cudaMemcpyPeer(ctxs[i]->counters.p, ctxs[i]->device, root->counters.p, root->device, bytes) != cudaSuccess) {
-            set_err("allreduce: broadcast failed: %s", cudaGetErrorString(cudaGetLastError()));
-            rc = TGSF_ERR_CUDA;
-        }
-    scratch.release();
-    return rc;
+    for (int i = 1; i < n; ++i)
+        CU(cudaMemcpyPeer(ctxs[i]->counters.p, ctxs[i]->device, root->counters.p, root->device, bytes));
+    return TGSF_OK;
 }
 
 int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint32_t n, uint32_t row_len,
@@ -1612,22 +1546,16 @@ int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint3
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
     const int sms = prop.multiProcessorCount;
-    DBuf d_rows, d_cnt, d_maps;
-    AdapterSet ads;
-    Scratch scratch;
-    auto cleanup = [&]() { d_rows.release(); d_cnt.release(); d_maps.release(); ads.release(); scratch.buf.release(); };
+    DBuf d_rows, d_cnt;
     const size_t row_bytes = (size_t)n * row_len;
-    int rc = d_rows.ensure(2 * row_bytes + 64);
-    if (rc == TGSF_OK) rc = d_cnt.ensure((size_t)2 * row_len * 4 * sizeof(int));
-    if (rc != TGSF_OK) { cleanup(); return rc; }
+    TRY(d_rows.ensure(2 * row_bytes + 64));
+    TRY(d_cnt.ensure((size_t)2 * row_len * 4 * sizeof(int)));
     uint8_t *r5 = d_rows.as<uint8_t>(), *r3 = r5 + row_bytes;
-    cudaError_t e = cudaSuccess;
     if (row_bytes) {
-        e = cudaMemcpy(r5, ends5p, row_bytes, cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMemcpy(r3, ends3p, row_bytes, cudaMemcpyHostToDevice);
+        CU(cudaMemcpy(r5, ends5p, row_bytes, cudaMemcpyHostToDevice));
+        CU(cudaMemcpy(r3, ends3p, row_bytes, cudaMemcpyHostToDevice));
     }
-    if (e == cudaSuccess) e = cudaMemset(d_cnt.p, 0, (size_t)2 * row_len * 4 * sizeof(int));
-    if (e != cudaSuccess) { set_err("prepass upload: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+    CU(cudaMemset(d_cnt.p, 0, (size_t)2 * row_len * 4 * sizeof(int)));
     int *c5 = d_cnt.as<int>(), *c3 = c5 + (size_t)row_len * 4;
     if (n) {
         // column tiles on y; about 4 CTAs per SM in all, so the flush of the per-CTA tables does not grow with row_len
@@ -1636,46 +1564,40 @@ int tgsf_prepass(int device, const uint8_t *ends5p, const uint8_t *ends3p, uint3
         const size_t smem = (size_t)std::min<u32>(row_len, PRE_TILE_COLS) * 4 * sizeof(u32);
         k_base_content<<<grid, PRE_THREADS, smem>>>(r5, n, row_len, c5);
         k_base_content<<<grid, PRE_THREADS, smem>>>(r3, n, row_len, c3);
-        rc = check_launch("k_base_content");
-        if (rc != TGSF_OK) { cleanup(); return rc; }
+        TRY(check_launch("k_base_content"));
     }
     if (lib_seq) {
-        rc = ads.build(lib_seq, lib_len, n_lib);
-        if (rc == TGSF_OK) {
-            if (min_sim < 0.9) min_sim = 0.9; // T.cpp:1151-1154 (float compared against a double literal)
-            for (auto &A : ads.host) {
-                int minK = static_cast<int>((1 - min_sim) * A.qlen) + 1; // T.cpp:1161
-                A.k_end = std::min(minK, A.qlen - 1);
-            }
+        AdapterSet ads;
+        DBuf d_maps;
+        Scratch scratch;
+        TRY(ads.build(lib_seq, lib_len, n_lib));
+        if (min_sim < 0.9) min_sim = 0.9; // T.cpp:1151-1154 (float compared against a double literal)
+        for (auto &A : ads.host) {
+            int minK = static_cast<int>((1 - min_sim) * A.qlen) + 1; // T.cpp:1161
+            A.k_end = std::min(minK, A.qlen - 1);
         }
-        if (rc == TGSF_OK) rc = ads.upload();
-        if (rc == TGSF_OK) rc = d_maps.ensure((size_t)2 * n_lib * sizeof(long long));
-        if (rc == TGSF_OK) rc = scratch.ensure(ads.host, sms * 4, RES_THREADS);
-        if (rc != TGSF_OK) { cleanup(); return rc; }
-        e = cudaMemset(d_maps.p, 0, (size_t)2 * n_lib * sizeof(long long));
-        if (e != cudaSuccess) { set_err("prepass maps: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+        TRY(ads.upload());
+        TRY(d_maps.ensure((size_t)2 * n_lib * sizeof(long long)));
+        TRY(scratch.ensure(ads.host, sms * 4, RES_THREADS));
+        CU(cudaMemset(d_maps.p, 0, (size_t)2 * n_lib * sizeof(long long)));
         long long *m5 = d_maps.as<long long>(), *m3 = m5 + n_lib;
         const AdapterCtx AC = ads.ctx();
         for (int a = 0; a < n_lib && n; ++a) {
             const DevAdapter &Ah = ads.host[(size_t)a];
             const int grid_a = Scratch::grid_for(sms * 4, RES_THREADS, 2 * Ah.qlen + 2, Ah.nw);
             const u64 stride_a = (u64)grid_a * RES_THREADS;
-            rc = for_nw(Ah.nw, [&](auto nwc) {
+            TRY(for_nw(Ah.nw, [&](auto nwc) {
                 constexpr int NW = decltype(nwc)::value;
                 k_lib_search<NW><<<grid_a, RES_THREADS>>>(r5, n, row_len, AC, a, m5 + a, scratch.buf.as<u64>(), stride_a);
                 k_lib_search<NW><<<grid_a, RES_THREADS>>>(r3, n, row_len, AC, a, m3 + a, scratch.buf.as<u64>(), stride_a);
                 return check_launch("k_lib_search");
-            });
-            if (rc != TGSF_OK) { cleanup(); return rc; }
+            }));
         }
-        e = cudaMemcpy(map5p, m5, (size_t)n_lib * sizeof(long long), cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(map3p, m3, (size_t)n_lib * sizeof(long long), cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) { set_err("prepass maps: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+        CU(cudaMemcpy(map5p, m5, (size_t)n_lib * sizeof(long long), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(map3p, m3, (size_t)n_lib * sizeof(long long), cudaMemcpyDeviceToHost));
     }
-    e = cudaMemcpy(bases_num5p, c5, (size_t)row_len * 4 * sizeof(int), cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemcpy(bases_num3p, c3, (size_t)row_len * 4 * sizeof(int), cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) { set_err("prepass download: %s", cudaGetErrorString(e)); return TGSF_ERR_CUDA; }
+    CU(cudaMemcpy(bases_num5p, c5, (size_t)row_len * 4 * sizeof(int), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(bases_num3p, c3, (size_t)row_len * 4 * sizeof(int), cudaMemcpyDeviceToHost));
     return TGSF_OK;
 }
 
@@ -1695,13 +1617,10 @@ int tgsf_end_kmer_counts(int device, const uint8_t *rows, uint32_t n, uint32_t r
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
     DBuf d_rows, d_table;
-    auto cleanup = [&]() { d_rows.release(); d_table.release(); };
     const size_t row_bytes = (size_t)n * row_len;
-    int rc = d_rows.ensure(row_bytes);
-    if (rc == TGSF_OK) rc = d_table.ensure(table_bytes);
-    if (rc != TGSF_OK) { cleanup(); return rc; }
-    cudaError_t e = cudaMemcpy(d_rows.p, rows, row_bytes, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { set_err("end_kmer_counts upload: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+    TRY(d_rows.ensure(row_bytes));
+    TRY(d_table.ensure(table_bytes));
+    CU(cudaMemcpy(d_rows.p, rows, row_bytes, cudaMemcpyHostToDevice));
     // one band per launch into one table: at k = 12 a band's table (64 MB) stays resident in the 126 MB L2, where the
     // two bands' tables together would not
     const u32 grid = std::max<u32>(1, std::min<u32>(cdiv(n, PRE_THREADS / 32), (u32)prop.multiProcessorCount * 8));
@@ -1709,18 +1628,14 @@ int tgsf_end_kmer_counts(int device, const uint8_t *rows, uint32_t n, uint32_t r
     const u32 bands[2][2] = {{0, cut}, {cut, (u32)windows}};
     uint32_t *out[2] = {outer, inner};
     for (int b = 0; b < 2; ++b) {
-        e = cudaMemset(d_table.p, 0, table_bytes);
-        if (e != cudaSuccess) { set_err("end_kmer_counts: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+        CU(cudaMemset(d_table.p, 0, table_bytes));
         if (bands[b][1] > bands[b][0]) {
             k_end_kmers<<<grid, PRE_THREADS>>>(d_rows.as<uint8_t>(), n, row_len, k, bands[b][0], bands[b][1],
                                                d_table.as<u32>());
-            rc = check_launch("k_end_kmers");
-            if (rc != TGSF_OK) { cleanup(); return rc; }
+            TRY(check_launch("k_end_kmers"));
         }
-        e = cudaMemcpy(out[b], d_table.p, table_bytes, cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) { set_err("end_kmer_counts download: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+        CU(cudaMemcpy(out[b], d_table.p, table_bytes, cudaMemcpyDeviceToHost));
     }
-    cleanup();
     return TGSF_OK;
 }
 
@@ -1743,26 +1658,20 @@ int tgsf_align_hw(int device, const uint8_t *queries, const uint32_t *q_off, con
     AdapterSet ads;
     DBuf d_t, d_toff, d_k, d_out;
     Scratch scratch;
-    auto cleanup = [&]() { ads.release(); d_t.release(); d_toff.release(); d_k.release(); d_out.release(); scratch.buf.release(); };
-    int rc = ads.build(seqs.data(), lens.data(), (int)n);
-    if (rc == TGSF_OK) {
-        for (u32 i = 0; i < n; ++i)
-            if (lens[i] == 0 || t_off[i + 1] == t_off[i]) ads.host[i].nw = 0; // handled on the host below
-        rc = ads.upload();
-    }
+    TRY(ads.build(seqs.data(), lens.data(), (int)n));
+    for (u32 i = 0; i < n; ++i)
+        if (lens[i] == 0 || t_off[i + 1] == t_off[i]) ads.host[i].nw = 0; // handled on the host below
+    TRY(ads.upload());
     const size_t tbytes = t_off[n];
-    if (rc == TGSF_OK) rc = d_t.ensure(tbytes + 64);
-    if (rc == TGSF_OK) rc = d_toff.ensure(((size_t)n + 1) * sizeof(u32));
-    if (rc == TGSF_OK) rc = d_k.ensure((size_t)n * sizeof(int));
-    if (rc == TGSF_OK) rc = d_out.ensure((size_t)n * sizeof(tgsf_align_result));
-    if (rc == TGSF_OK) rc = scratch.ensure(ads.host, sms * 2, RES_THREADS);
-    if (rc != TGSF_OK) { cleanup(); return rc; }
-    cudaError_t e = cudaSuccess;
-    if (tbytes) e = cudaMemcpy(d_t.p, targets, tbytes, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(d_toff.p, t_off, ((size_t)n + 1) * sizeof(u32), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemcpy(d_k.p, k, (size_t)n * sizeof(int), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemset(d_out.p, 0, (size_t)n * sizeof(tgsf_align_result));
-    if (e != cudaSuccess) { set_err("align upload: %s", cudaGetErrorString(e)); cleanup(); return TGSF_ERR_CUDA; }
+    TRY(d_t.ensure(tbytes + 64));
+    TRY(d_toff.ensure(((size_t)n + 1) * sizeof(u32)));
+    TRY(d_k.ensure((size_t)n * sizeof(int)));
+    TRY(d_out.ensure((size_t)n * sizeof(tgsf_align_result)));
+    TRY(scratch.ensure(ads.host, sms * 2, RES_THREADS));
+    if (tbytes) CU(cudaMemcpy(d_t.p, targets, tbytes, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_toff.p, t_off, ((size_t)n + 1) * sizeof(u32), cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(d_k.p, k, (size_t)n * sizeof(int), cudaMemcpyHostToDevice));
+    CU(cudaMemset(d_out.p, 0, (size_t)n * sizeof(tgsf_align_result)));
     const AdapterCtx AC = ads.ctx();
     for (int nw : {1, 2, 3, 4, 8, 16, 32}) {
         int max_q = 0;
@@ -1770,18 +1679,15 @@ int tgsf_align_hw(int device, const uint8_t *queries, const uint32_t *q_off, con
             if (ads.host[i].nw == nw) max_q = std::max(max_q, ads.host[i].qlen);
         if (max_q == 0) continue;
         const int grid_nw = Scratch::grid_for(sms * 2, RES_THREADS, 2 * max_q + 2, nw);
-        rc = for_nw(nw, [&](auto nwc) {
+        TRY(for_nw(nw, [&](auto nwc) {
             constexpr int NW = decltype(nwc)::value;
             k_align_pairs<NW><<<grid_nw, RES_THREADS>>>(d_t.as<uint8_t>(), d_toff.as<u32>(), d_k.as<int>(), AC, n, NW,
                                                         d_out.as<tgsf_align_result>(), scratch.buf.as<u64>(),
                                                         (u64)grid_nw * RES_THREADS);
             return check_launch("k_align_pairs");
-        });
-        if (rc != TGSF_OK) { cleanup(); return rc; }
+        }));
     }
-    e = cudaMemcpy(out, d_out.p, (size_t)n * sizeof(tgsf_align_result), cudaMemcpyDeviceToHost);
-    cleanup();
-    if (e != cudaSuccess) { set_err("align download: %s", cudaGetErrorString(e)); return TGSF_ERR_CUDA; }
+    CU(cudaMemcpy(out, d_out.p, (size_t)n * sizeof(tgsf_align_result), cudaMemcpyDeviceToHost));
     for (u32 i = 0; i < n; ++i) {
         if (lens[i] == 0 || t_off[i + 1] == t_off[i]) { // E.cpp:161-179
             tgsf_align_result R;
