@@ -107,6 +107,7 @@ typedef struct tgsf_piece {
 #define TGSF_PIECE_QC_ONLY 3      /* --qc: region kept but nothing emitted (T.cpp:1976) */
 #define TGSF_PIECE_CONTAM 4       /* contaminant screen: hit share >= min_frac (tgsf_set_contaminants) */
 #define TGSF_PIECE_FOLDBACK 5     /* fold-back screen: the kept arm is shorter than min_len (tgsf_set_foldback) */
+#define TGSF_PIECE_LOWCOMPLEX 6   /* DUST screen: masked share >= min_frac (tgsf_set_dust) */
 
 /* Layout (in uint64 words) of the cumulative counter block.  Every member is a sum, so blocks of
  * different GPUs combine with one allreduce(sum, u64).  [x][5] = {A,T,G,C,all} as in T.cpp:1462-1476. */
@@ -237,6 +238,25 @@ typedef struct tgsf_fold_result {
 } tgsf_fold_result;
 int tgsf_fold_detect(int device, const uint8_t *seq, const uint64_t *offsets, uint32_t n, tgsf_fold_result *out);
 
+/* Low-complexity screen (an extension; the reference has none): the original windowed DUST score, not dustmasker's
+ * symmetric DUST.  Rules, on piece-relative positions of s[0, L): codes A0 C1 G2 T3, case-insensitive; triplet i =
+ * s[i, i+3), code 16a + 4b + c.  Window j = s[j, j+64), 0 <= j <= L - 64, is valid iff all 64 bytes are ACGT/acgt;
+ * for a valid window c_t counts its 62 triplets j .. j+61 by code and S_j = sum_t c_t (c_t - 1) / 2 (0 .. 1891).
+ * Window j is masked iff it is valid and S_j > 61 level.  M = the size of the union of [j, j+64) over the masked
+ * windows.  A piece becomes TGSF_PIECE_LOWCOMPLEX iff L >= 64 and M * 1000000 >= ppm * L (u64),
+ * ppm = llround((double)min_frac * 1e6).  With level in [1, 30], every piece that is still TGSF_PIECE_EMIT after the
+ * repeat check and the contaminant screen (not with TGSF_FLAG_ONLY_QC) is screened, after a fold-back cut; a dropped
+ * piece keeps sum_q = 0, its repeat_len and contam_hits, touches no counter and gets no deflate bytes.  Callers count
+ * the dropped pieces from the piece array.  level 0 turns the screen off (min_frac is then ignored); another level
+ * outside [1, 30] or a ppm outside [1, 1000000] gives TGSF_ERR_INVALID; TGSF_ERR_STATE while a batch is outstanding.
+ * The screen's kernels are timed in TGSF_STAGE_KMER. */
+int tgsf_set_dust(tgsf_ctx *ctx, int32_t level, float min_frac);
+/* The screen's kernels on n stand-alone pieces seq[offsets[i], offsets[i+1]) (host buffers, offsets[0] == 0, each
+ * piece < 2^31 bases): masked[i] = M of piece i at this level (in [1, 30]).  Bad arguments give TGSF_ERR_INVALID
+ * before the device is touched; n = 0 touches nothing. */
+int tgsf_dust_detect(int device, const uint8_t *seq, const uint64_t *offsets, uint32_t n, int32_t level,
+                     uint32_t *masked);
+
 /* Device time (ms, CUDA events on the slot's stream) of the batch retired by the last collect:
  * kernels only, and H2D+kernels+D2H. */
 int tgsf_last_timing(tgsf_ctx *ctx, float *kernel_ms, float *total_ms);
@@ -249,7 +269,7 @@ int tgsf_last_timing(tgsf_ctx *ctx, float *kernel_ms, float *total_ms);
 #define TGSF_STAGE_MID_SCAN 2    /* K3 k_mid_scan, all adapters (chunk table included) */
 #define TGSF_STAGE_RESOLVE 3     /* K3 k_mid_count + k_ends (start search, traceback, thresholds) */
 #define TGSF_STAGE_REGIONS 4     /* K3 k_mid_emit + K5 regions / piece compaction */
-#define TGSF_STAGE_KMER 5        /* the fold-back screen + K4 + the contaminant screen */
+#define TGSF_STAGE_KMER 5        /* the fold-back screen + K4 + the contaminant screen + the DUST screen */
 #define TGSF_STAGE_CLEAN 6       /* K1 over the kept pieces + clean decisions + clean 5'/3' */
 int tgsf_last_stage_ms(tgsf_ctx *ctx, float *out, int n);
 

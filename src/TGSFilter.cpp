@@ -75,6 +75,9 @@ struct Params {
     int ContamK = 17;             // --contam-k
     float ContamFrac = 0.05f;     // --contam-frac
     bool Foldback = false;        // --foldback (extension): cut pieces at a fold-back junction, keep the longer arm
+    bool Dust = false;            // --dust (extension): drop pieces dominated by low-complexity sequence
+    int DustLevel = 7;            // --dust-level
+    float DustFrac = 0.5f;        // --dust-frac
     bool Denovo = false;          // --adapter-denovo (extension): assemble an end's adapter when the library has none
     uint64_t batch_bases = 64ull << 20; // bases per batch (TGSF_BATCH_MB)
 };
@@ -127,6 +130,10 @@ int usage() {
                  "   --contam-frac <float> min fraction of a piece's k-mers found in the set to discard it [0.05]\n"
                  " Fold-back screen:\n"
                  "   --foldback            cut reads that fold back onto their own reverse complement, keep the longer arm\n"
+                 " Low-complexity screen:\n"
+                 "   --dust                discard reads dominated by homopolymer or short tandem repeat (windowed DUST)\n"
+                 "   --dust-level <int>    DUST score above which a 64-base window is masked, 1-30 [7]\n"
+                 "   --dust-frac <float>   min fraction of a read's bases in masked windows to discard it [0.5]\n"
                  "   -h           show help [b200 host of v1.11]\n\n";
     return 1;
 }
@@ -200,6 +207,9 @@ int parse_cmd(int argc, char **argv, Params *P) {
         else if (flag == "contamfrac") { if (!need()) return 1; P->ContamFrac = (float)atof(argv[i]); }
         else if (flag == "adapterdenovo") { P->Denovo = true; }
         else if (flag == "foldback") { P->Foldback = true; }
+        else if (flag == "dust") { P->Dust = true; }
+        else if (flag == "dustlevel") { if (!need()) return 1; P->DustLevel = atoi(argv[i]); }
+        else if (flag == "dustfrac") { if (!need()) return 1; P->DustFrac = (float)atof(argv[i]); }
         else if (flag == "help" || flag == "h") { usage(); return 1; }
         else { cerr << "Error: UnKnow argument -" << flag << endl; return 1; }
     }
@@ -220,6 +230,16 @@ int parse_cmd(int argc, char **argv, Params *P) {
     }
     if (P->Foldback && (P->OnlyQC || P->ONLYAD || !P->Filter)) {
         cerr << "Error: --foldback screens filtered reads and cannot be combined with --qc, -A or -F" << endl;
+        exit(-1);
+    }
+    if (P->DustLevel < 1 || P->DustLevel > 30) { cerr << "Error: --dust-level must be in [1,30]" << endl; exit(-1); }
+    const long long dust_ppm = llround((double)P->DustFrac * 1e6); // as tgsf_set_dust computes it
+    if (!(P->DustFrac == P->DustFrac) || dust_ppm < 1 || dust_ppm > 1000000) {
+        cerr << "Error: --dust-frac must be in (0,1]" << endl;
+        exit(-1);
+    }
+    if (P->Dust && (P->OnlyQC || P->ONLYAD || !P->Filter)) {
+        cerr << "Error: --dust screens filtered reads and cannot be combined with --qc, -A or -F" << endl;
         exit(-1);
     }
     if (P->Denovo && (!P->AdapterFile.empty() || P->OnlyQC || !P->Filter)) {
@@ -999,7 +1019,7 @@ std::vector<string> resolve_adapters(Params &P, bool has_qual, const Sample &S) 
     return adapters;
 }
 
-// ---- contexts: one per GPU, with the contaminant set (--contam) and the fold-back screen (--foldback) on each ------------------------
+// ---- contexts: one per GPU, with the contaminant set (--contam), the fold-back screen (--foldback) and the DUST screen (--dust) on each
 std::vector<tgsf_ctx *> create_contexts(const Params &P, int qType, const std::vector<string> &adapters, bool gz_gpu,
                                         std::vector<uint8_t> &contam_seq, const std::vector<uint64_t> &contam_offs) {
     tgsf_params tp;
@@ -1042,6 +1062,9 @@ std::vector<tgsf_ctx *> create_contexts(const Params &P, int qType, const std::v
     if (P.Foldback)
         for (int g = 0; g < P.gpus; g++)
             if (tgsf_set_foldback(ctx[(size_t)g], 1) != TGSF_OK) die_tgsf("tgsf_set_foldback");
+    if (P.Dust)
+        for (int g = 0; g < P.gpus; g++)
+            if (tgsf_set_dust(ctx[(size_t)g], P.DustLevel, P.DustFrac) != TGSF_OK) die_tgsf("tgsf_set_dust");
     return ctx;
 }
 
@@ -1099,6 +1122,7 @@ public:
     PinnedPool gz_pool;
     uint64_t cleanNum = 0, cleanBases = 0;
     uint64_t contamNum = 0, contamBases = 0; // pieces discarded by the contaminant screen (--contam)
+    uint64_t dustNum = 0, dustBases = 0;     // pieces discarded by the DUST screen (--dust)
     std::vector<int> cleanLens;              // T.cpp:1794
     Filtered kept;
     // Opens the output (stdout, -o, or with downsampling the buffer / tmp file) and starts the thread.
@@ -1153,6 +1177,7 @@ private:
             const tgsf_piece &p = job.pieces[pi];
             if ((uint32_t)p.read != last) { last = (uint32_t)p.read; pass = 1; }
             if (p.status == TGSF_PIECE_CONTAM) { contamNum++; contamBases += (uint64_t)p.len; }
+            if (p.status == TGSF_PIECE_LOWCOMPLEX) { dustNum++; dustBases += (uint64_t)p.len; }
             if (p.status != TGSF_PIECE_EMIT) continue;
             emits_.push_back(Emit{last, (uint32_t)p.start, (uint32_t)p.len, pass, (uint32_t)pi});
             pass++;
@@ -1567,6 +1592,8 @@ void report_filter(const Params &P, std::vector<tgsf_ctx *> &ctx, const MainPass
             cerr << "INFO: " << D[15] << " reads were discarded with " << D[16] << " bases due to short repeat length." << endl;
         if (!P.ContamFile.empty())
             cerr << "INFO: " << w.contamNum << " reads were discarded with " << w.contamBases << " bases as contaminant." << endl;
+        if (P.Dust)
+            cerr << "INFO: " << w.dustNum << " reads were discarded with " << w.dustBases << " bases as low complexity." << endl;
         if (P.Foldback) {
             uint64_t F[4] = {0, 0, 0, 0};
             for (tgsf_ctx *c : ctx) {

@@ -26,7 +26,8 @@ FLAG_GZ_BLOCKS = 8
 FLAG_GZ_FASTA = 16
 
 READ_EVALUATED, READ_LOWQ, READ_EMPTY = 0, 1, 2
-PIECE_EMIT, PIECE_SHORT_REPEAT, PIECE_LOWQ, PIECE_QC_ONLY, PIECE_CONTAM, PIECE_FOLDBACK = 0, 1, 2, 3, 4, 5
+PIECE_EMIT, PIECE_SHORT_REPEAT, PIECE_LOWQ, PIECE_QC_ONLY, PIECE_CONTAM, PIECE_FOLDBACK, PIECE_LOWCOMPLEX = \
+    0, 1, 2, 3, 4, 5, 6
 
 N_STAGES = 7
 STAGE_NAMES = ("raw_scan", "raw_final", "mid_scan", "resolve", "regions", "kmer", "clean")
@@ -117,7 +118,8 @@ EXPORTED_SYMBOLS = (
     "tgsf_host_free", "tgsf_submit", "tgsf_submit_packed", "tgsf_pack_bases", "tgsf_submit_device", "tgsf_collect", "tgsf_collect_gz", "tgsf_last_timing", "tgsf_last_span", "tgsf_last_stage_ms",
     "tgsf_counter_layout_get", "tgsf_counters", "tgsf_counters_reset", "tgsf_counters_device",
     "tgsf_launch_count", "tgsf_launch_shape", "tgsf_mid_run_shift", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw", "tgsf_set_contaminants",
-    "tgsf_end_kmer_counts", "tgsf_set_foldback", "tgsf_foldback_stats", "tgsf_fold_detect",
+    "tgsf_end_kmer_counts", "tgsf_set_foldback", "tgsf_foldback_stats", "tgsf_fold_detect", "tgsf_set_dust",
+    "tgsf_dust_detect",
 )
 
 _lib = None
@@ -170,6 +172,8 @@ def load() -> C.CDLL:
     lib.tgsf_set_foldback.argtypes = [vp, C.c_int32]
     lib.tgsf_foldback_stats.argtypes = [vp, u64p]
     lib.tgsf_fold_detect.argtypes = [C.c_int, u8p, u64p, C.c_uint32, vp]
+    lib.tgsf_set_dust.argtypes = [vp, C.c_int32, C.c_float]
+    lib.tgsf_dust_detect.argtypes = [C.c_int, u8p, u64p, C.c_uint32, C.c_int32, vp]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)
         if fn.restype is C.c_int and name not in ("tgsf_version", "tgsf_last_error",

@@ -28,7 +28,7 @@
 struct __align__(16) ContamChunk {
     u64 start; // absolute byte offset of the chunk's first window
     u32 piece;
-    u32 n_win; // windows in the chunk (1 .. CONTAM_CHUNK)
+    u32 n_win; // windows in the chunk (1 .. the chunk length)
 };
 
 static __device__ __forceinline__ u64 contam_mix(u64 x) { // splitmix64 finaliser
@@ -124,22 +124,23 @@ __global__ void k_contam_bitmap(const u64 *__restrict__ table, u64 cap, u32 *bit
     }
 }
 
-// Chunks per piece: only pieces still emitted and at least k long are screened.  Launched over the piece capacity; the
-// live count is device-side.
+// Chunks of `chunk` windows of length k per piece: only pieces still emitted and at least k long are screened.  Launched
+// over the piece capacity; the live count is device-side.  The DUST screen (dust.cuh) cuts its chunks with the same two
+// kernels.
 __global__ void k_contam_count(const tgsf_piece *__restrict__ pieces, const u32 *__restrict__ n_pieces_ptr, u32 cap,
-                               int k, u32 *__restrict__ n_chunks, const u32 *__restrict__ dev_status) {
+                               int k, u32 chunk, u32 *__restrict__ n_chunks, const u32 *__restrict__ dev_status) {
     const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= cap) return;
     u32 n = 0;
     if (*dev_status == DEV_STATUS_OK && i < *n_pieces_ptr) {
         const tgsf_piece p = pieces[i];
-        if (p.status == TGSF_PIECE_EMIT && p.len >= k) n = ((u32)(p.len - k) + CONTAM_CHUNK) / CONTAM_CHUNK;
+        if (p.status == TGSF_PIECE_EMIT && p.len >= k) n = ((u32)(p.len - k) + chunk) / chunk;
     }
     n_chunks[i] = n;
 }
 
 __global__ void k_contam_fill(DevBatch B, const tgsf_piece *__restrict__ pieces, const u32 *__restrict__ chunk_off,
-                              u32 cap, int k, ContamChunk *__restrict__ chunks) {
+                              u32 cap, int k, u32 chunk, ContamChunk *__restrict__ chunks) {
     const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= cap) return;
     const u32 b = chunk_off[i], e = chunk_off[i + 1];
@@ -148,11 +149,11 @@ __global__ void k_contam_fill(DevBatch B, const tgsf_piece *__restrict__ pieces,
     const u64 s0 = B.offsets[p.read] + (u64)p.start;
     const u32 windows = (u32)(p.len - k + 1);
     for (u32 c = b; c < e; ++c) {
-        const u32 w0 = (c - b) * CONTAM_CHUNK;
+        const u32 w0 = (c - b) * chunk;
         ContamChunk ch;
         ch.start = s0 + w0;
         ch.piece = i;
-        ch.n_win = min(CONTAM_CHUNK, windows - w0);
+        ch.n_win = min(chunk, windows - w0);
         chunks[c] = ch;
     }
 }

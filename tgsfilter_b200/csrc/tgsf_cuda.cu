@@ -18,6 +18,7 @@
 #include "adapters.cuh"
 #include "common.cuh"
 #include "contam.cuh"
+#include "dust.cuh"
 #include "foldback.cuh"
 #include "kmer.cuh"
 #include "kmer16.cuh"
@@ -239,7 +240,8 @@ struct Slot {
     int chunk_shift = MID_CHUNK_SHIFT_MIN, run_shift = 0;
     DBuf best_mid, mid_n, mid_off, end_n, end_pos, pool, sortbuf, tmp, pieces, res, header;
     DBuf scan_tmp, kmer_long_list, mid_work, gz_blob, gz_spans;
-    DBuf contam_cnt, contam_off, contam_chunks; // contaminant screen (only with a set installed)
+    DBuf contam_cnt, contam_off, contam_chunks; // chunk lists of the contaminant and the DUST screen (only while on)
+    DBuf dust_masked;                            // DUST screen: masked bases per piece (only while on)
     DBuf fold_long_list, fold_ws;                // fold-back screen (only while enabled)
     Scratch scratch, scratch2; // traceback stores: main stream (k_mid_count) / side stream (k_ends)
     u32 pool_cap = 0, pieces_cap = 0, chunks_cap = 0, runs_cap = 0, tiles_cap = 0;
@@ -268,6 +270,8 @@ struct tgsf_ctx {
     AdapterSet ads;
     ContamSet contam;
     bool foldback = false;
+    int dust_level = 0; // DUST screen (tgsf_set_dust): 0 = off
+    u64 dust_ppm = 0;
     DBuf fold_stats; // u64[4] (tgsf_foldback_stats), allocated when the screen is first enabled
     DBuf counters;
     std::vector<Slot> slots;
@@ -688,12 +692,12 @@ int launch_contam(tgsf_ctx *c, Slot &s) {
     TRY(s.contam_off.ensure(((size_t)cap + 1) * sizeof(u32)));
     TRY(s.contam_chunks.ensure(chunks_cap * sizeof(ContamChunk)));
     k_contam_count<<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap, cs.k,
-                                                   s.contam_cnt.as<u32>(), &H->status);
+                                                   CONTAM_CHUNK, s.contam_cnt.as<u32>(), &H->status);
     c->launches++;
     TRY(exclusive_scan(c, st, s.contam_cnt.as<u32>(), s.contam_off.as<u32>(), cap, s.scan_tmp.as<u32>(),
                        s.scan_tmp.cap / sizeof(u32)));
     k_contam_fill<<<cdiv(cap, 256), 256, 0, st>>>(s.B, s.pieces.as<tgsf_piece>(), s.contam_off.as<u32>(), cap, cs.k,
-                                                  s.contam_chunks.as<ContamChunk>());
+                                                  CONTAM_CHUNK, s.contam_chunks.as<ContamChunk>());
     c->launches++;
     if (cs.pf_bits.p)
         k_contam_screen<true><<<c->sm_count, CONTAM_THREADS, CONTAM_PF_SMEM_BYTES, st>>>(
@@ -708,6 +712,40 @@ int launch_contam(tgsf_ctx *c, Slot &s) {
                                                     &H->status);
     c->launches++;
     return check_launch("contam");
+}
+
+// DUST screen over the pieces still emitted after K4 and the contaminant screen: the contaminant screen's chunk
+// kernels with 64-base windows and DUST_CHUNK windows a chunk (the two screens run one after the other on the slot's
+// stream and share the chunk-list buffers), the masked bases of every piece into s.dust_masked, then the threshold.
+// ppm 0 skips the threshold (tgsf_dust_detect).  Writes piece status only.
+int launch_dust(tgsf_ctx *c, Slot &s, int level, u64 ppm) {
+    cudaStream_t st = s.stream.get();
+    DevHeader *H = s.header.as<DevHeader>();
+    const u32 cap = s.pieces_cap;
+    const size_t chunks_cap = (size_t)(s.n_bases / DUST_CHUNK) + cap + 16;
+    TRY(s.contam_cnt.ensure((size_t)cap * sizeof(u32)));
+    TRY(s.contam_off.ensure(((size_t)cap + 1) * sizeof(u32)));
+    TRY(s.contam_chunks.ensure(chunks_cap * sizeof(ContamChunk)));
+    TRY(s.dust_masked.ensure((size_t)std::max<u32>(cap, 1) * sizeof(u32)));
+    CU(cudaMemsetAsync(s.dust_masked.p, 0, (size_t)cap * sizeof(u32), st));
+    k_contam_count<<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap, DUST_WINDOW,
+                                                   DUST_CHUNK, s.contam_cnt.as<u32>(), &H->status);
+    c->launches++;
+    TRY(exclusive_scan(c, st, s.contam_cnt.as<u32>(), s.contam_off.as<u32>(), cap, s.scan_tmp.as<u32>(),
+                       s.scan_tmp.cap / sizeof(u32)));
+    k_contam_fill<<<cdiv(cap, 256), 256, 0, st>>>(s.B, s.pieces.as<tgsf_piece>(), s.contam_off.as<u32>(), cap,
+                                                  DUST_WINDOW, DUST_CHUNK, s.contam_chunks.as<ContamChunk>());
+    c->launches++;
+    k_dust_screen<<<c->sm_count * (2048 / DUST_THREADS), DUST_THREADS, 0, st>>>(
+        s.B.bases, s.contam_chunks.as<ContamChunk>(), s.contam_off.as<u32>() + cap, (u32)(61 * level),
+        s.dust_masked.as<u32>(), &H->status);
+    c->launches++;
+    if (ppm) {
+        k_dust_decide<<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap,
+                                                      s.dust_masked.as<u32>(), ppm, &H->status);
+        c->launches++;
+    }
+    return check_launch("dust");
 }
 
 // Fold-back screen over the pieces K5 emitted, before K4: the shared-memory path for every piece, then the global
@@ -788,6 +826,7 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
             TRY(launch_fold(c, s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, nullptr, P.L.max_bins * SCAN_BIN));
         if (P.min_repeat > 0) TRY(launch_kmer(c, s, P));
         if (c->contam.installed()) TRY(launch_contam(c, s));
+        if (c->dust_level) TRY(launch_dust(c, s, c->dust_level, c->dust_ppm));
         CU(cudaEventRecord(s.ev_stage[6].get(), st));
         // clean pass over the kept pieces (T.cpp:1991-2009); piece count is device-side, the
         // kernels are launched over the capacity and bound themselves by the header.
@@ -889,6 +928,75 @@ void fill_thresholds(DevAdapter &A, const tgsf_params *p) {
     A.end_extra = endSim > 0.0f ? int(qLen / endSim) : 0; // T.cpp:1267
     A.halo_mid = A.k_mid > 0 ? ((qLen + A.k_mid - 1 + 15) / 16) * 16 : 0;
 }
+
+// The set-up of the screens' stand-alone entry points (tgsf_fold_detect, tgsf_dust_detect): n > 0 host records
+// seq[offsets[i], offsets[i+1]) become whole TGSF_PIECE_EMIT pieces in the slot of a bare context (no adapters, one
+// slot), so that the pipeline's kernels run on them unchanged.  The arguments are checked (offsets[0] == 0, ascending,
+// each piece < 2^31 bases, seq present) before the device is touched; the copies are enqueued on the slot's stream.
+struct RecordPieces {
+    CtxPtr c;
+    DBuf d_off;
+    u64 longest = 0;
+
+    int setup(const char *fn, int device, const uint8_t *seq, const uint64_t *offsets, uint32_t n) {
+        if (offsets[0] != 0) { set_err("%s: offsets[0] must be 0", fn); return TGSF_ERR_INVALID; }
+        for (uint32_t i = 0; i < n; ++i) {
+            if (offsets[i + 1] < offsets[i]) { set_err("%s: offsets not ascending at %u", fn, i); return TGSF_ERR_INVALID; }
+            longest = std::max<u64>(longest, offsets[i + 1] - offsets[i]);
+        }
+        if (longest >= (1ull << 31)) { set_err("%s: a piece of %llu bases", fn, (unsigned long long)longest); return TGSF_ERR_INVALID; }
+        const u64 n_bytes = offsets[n];
+        if (n_bytes && !seq) { set_err("%s: seq is NULL", fn); return TGSF_ERR_INVALID; }
+        CU(cudaSetDevice(device));
+        tgsf_params p;
+        memset(&p, 0, sizeof(p));
+        p.n_slots = 1;
+        tgsf_ctx *raw = nullptr;
+        TRY(tgsf_create(device, &p, &raw));
+        c.reset(raw);
+        Slot &s = slot();
+        cudaStream_t st = s.stream.get();
+        s.pieces_cap = n;
+        s.n_bases = n_bytes;
+        TRY(s.in_bases.ensure(std::max<u64>(n_bytes, 1)));
+        TRY(d_off.ensure(((size_t)n + 1) * sizeof(u64)));
+        TRY(s.pieces.ensure((size_t)n * sizeof(tgsf_piece)));
+        TRY(s.header.ensure(sizeof(DevHeader)));
+        TRY(s.scan_tmp.ensure((4 * ((size_t)n / SCANB_TILE) + 4096) * sizeof(u32)));
+        pc.resize((size_t)n);
+        for (uint32_t i = 0; i < n; ++i) {
+            memset(&pc[i], 0, sizeof(tgsf_piece));
+            pc[i].read = (int32_t)i;
+            pc[i].len = (int32_t)(offsets[i + 1] - offsets[i]);
+            pc[i].repeat_len = -1;
+            pc[i].status = TGSF_PIECE_EMIT;
+        }
+        memset(&h, 0, sizeof(h));
+        h.tmp_cursor = n;
+        if (n_bytes) CU(cudaMemcpyAsync(s.in_bases.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(s.pieces.p, pc.data(), (size_t)n * sizeof(tgsf_piece), cudaMemcpyHostToDevice, st));
+        CU(cudaMemcpyAsync(s.header.p, &h, sizeof(h), cudaMemcpyHostToDevice, st));
+        s.B.bases = s.in_bases.as<uint8_t>();
+        s.B.quals = nullptr;
+        s.B.offsets = d_off.as<u64>();
+        s.B.n_reads = n;
+        return TGSF_OK;
+    }
+    Slot &slot() { return c->slots[0]; }
+    // Waits for the stream (the caller's result copies enqueued) and checks the device status.
+    int finish(const char *fn) {
+        Slot &s = slot();
+        CU(cudaMemcpyAsync(&h, s.header.p, sizeof(h), cudaMemcpyDeviceToHost, s.stream.get()));
+        CU(cudaStreamSynchronize(s.stream.get()));
+        if (h.status != DEV_STATUS_OK) { set_err("%s: device status %u", fn, h.status); return TGSF_ERR_CUDA; }
+        return TGSF_OK;
+    }
+
+private:
+    std::vector<tgsf_piece> pc; // host staging of the copies, alive until finish()
+    DevHeader h;
+};
 
 }  // namespace
 
@@ -1057,58 +1165,50 @@ int tgsf_foldback_stats(tgsf_ctx *c, uint64_t out[4]) {
 int tgsf_fold_detect(int device, const uint8_t *seq, const uint64_t *offsets, uint32_t n, tgsf_fold_result *out) {
     if (n == 0) return TGSF_OK;
     if (!offsets || !out) { set_err("tgsf_fold_detect: NULL argument"); return TGSF_ERR_INVALID; }
-    if (offsets[0] != 0) { set_err("tgsf_fold_detect: offsets[0] must be 0"); return TGSF_ERR_INVALID; }
-    u64 longest = 0;
-    for (uint32_t i = 0; i < n; ++i) {
-        if (offsets[i + 1] < offsets[i]) { set_err("tgsf_fold_detect: offsets not ascending at %u", i); return TGSF_ERR_INVALID; }
-        longest = std::max<u64>(longest, offsets[i + 1] - offsets[i]);
-    }
-    if (longest >= (1ull << 31)) { set_err("tgsf_fold_detect: a piece of %llu bases", (unsigned long long)longest); return TGSF_ERR_INVALID; }
-    const u64 n_bytes = offsets[n];
-    if (n_bytes && !seq) { set_err("tgsf_fold_detect: seq is NULL"); return TGSF_ERR_INVALID; }
-    CU(cudaSetDevice(device));
-    // a context without adapters owns the stream, the header and the workspaces; the pieces are whole records
-    tgsf_params p;
-    memset(&p, 0, sizeof(p));
-    p.n_slots = 1;
-    tgsf_ctx *raw = nullptr;
-    TRY(tgsf_create(device, &p, &raw));
-    CtxPtr c(raw);
-    Slot &s = c->slots[0];
-    cudaStream_t st = s.stream.get();
-    DBuf d_off, d_out;
-    s.pieces_cap = n;
-    TRY(s.in_bases.ensure(std::max<u64>(n_bytes, 1)));
-    TRY(d_off.ensure(((size_t)n + 1) * sizeof(u64)));
-    TRY(s.pieces.ensure((size_t)n * sizeof(tgsf_piece)));
-    TRY(s.header.ensure(sizeof(DevHeader)));
+    RecordPieces R;
+    TRY(R.setup("tgsf_fold_detect", device, seq, offsets, n));
+    Slot &s = R.slot();
+    DBuf d_out;
     TRY(d_out.ensure((size_t)n * sizeof(tgsf_fold_result)));
-    std::vector<tgsf_piece> pc((size_t)n);
-    for (uint32_t i = 0; i < n; ++i) {
-        memset(&pc[i], 0, sizeof(tgsf_piece));
-        pc[i].read = (int32_t)i;
-        pc[i].len = (int32_t)(offsets[i + 1] - offsets[i]);
-        pc[i].repeat_len = -1;
-        pc[i].status = TGSF_PIECE_EMIT;
-    }
-    DevHeader h;
-    memset(&h, 0, sizeof(h));
-    h.tmp_cursor = n;
-    if (n_bytes) CU(cudaMemcpyAsync(s.in_bases.p, seq, n_bytes, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(s.pieces.p, pc.data(), (size_t)n * sizeof(tgsf_piece), cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(s.header.p, &h, sizeof(h), cudaMemcpyHostToDevice, st));
-    s.B.bases = s.in_bases.as<uint8_t>();
-    s.B.quals = nullptr;
-    s.B.offsets = d_off.as<u64>();
-    s.B.n_reads = n;
     DevHeader *H = s.header.as<DevHeader>();
-    TRY(launch_fold(c.get(), s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, d_out.as<tgsf_fold_result>(), (u32)longest));
-    CU(cudaMemcpyAsync(out, d_out.p, (size_t)n * sizeof(tgsf_fold_result), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(&h, s.header.p, sizeof(h), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if (h.status != DEV_STATUS_OK) { set_err("tgsf_fold_detect: device status %u", h.status); return TGSF_ERR_CUDA; }
+    TRY(launch_fold(R.c.get(), s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, d_out.as<tgsf_fold_result>(),
+                    (u32)R.longest));
+    CU(cudaMemcpyAsync(out, d_out.p, (size_t)n * sizeof(tgsf_fold_result), cudaMemcpyDeviceToHost, s.stream.get()));
+    return R.finish("tgsf_fold_detect");
+}
+
+int tgsf_set_dust(tgsf_ctx *c, int32_t level, float min_frac) {
+    if (!c) { set_err("tgsf_set_dust: ctx is NULL"); return TGSF_ERR_INVALID; }
+    if (level != 0 && (level < DUST_LEVEL_MIN || level > DUST_LEVEL_MAX)) {
+        set_err("tgsf_set_dust: level must be 0 or in [%d,%d], got %d", DUST_LEVEL_MIN, DUST_LEVEL_MAX, level);
+        return TGSF_ERR_INVALID;
+    }
+    const double fd = (double)min_frac;
+    const long long ppm = fd == fd && fd >= 0.0 && fd <= 2.0 ? llround(fd * 1e6) : -1;
+    if (level != 0 && (ppm < 1 || ppm > 1000000)) {
+        set_err("tgsf_set_dust: min_frac must give ppm in [1,1000000], got %g", fd);
+        return TGSF_ERR_INVALID;
+    }
+    if (c->outstanding) { set_err("tgsf_set_dust with %u batch(es) outstanding", c->outstanding); return TGSF_ERR_STATE; }
+    c->dust_level = level;
+    c->dust_ppm = level ? (u64)ppm : 0;
     return TGSF_OK;
+}
+
+int tgsf_dust_detect(int device, const uint8_t *seq, const uint64_t *offsets, uint32_t n, int32_t level,
+                     uint32_t *masked) {
+    if (level < DUST_LEVEL_MIN || level > DUST_LEVEL_MAX) {
+        set_err("tgsf_dust_detect: level must be in [%d,%d], got %d", DUST_LEVEL_MIN, DUST_LEVEL_MAX, level);
+        return TGSF_ERR_INVALID;
+    }
+    if (n == 0) return TGSF_OK;
+    if (!offsets || !masked) { set_err("tgsf_dust_detect: NULL argument"); return TGSF_ERR_INVALID; }
+    RecordPieces R;
+    TRY(R.setup("tgsf_dust_detect", device, seq, offsets, n));
+    Slot &s = R.slot();
+    TRY(launch_dust(R.c.get(), s, level, 0));
+    CU(cudaMemcpyAsync(masked, s.dust_masked.p, (size_t)n * sizeof(u32), cudaMemcpyDeviceToHost, s.stream.get()));
+    return R.finish("tgsf_dust_detect");
 }
 
 int tgsf_device_count(int *count) {

@@ -97,6 +97,11 @@ class FilterEngine:
         _capi.check(self._lib.tgsf_foldback_stats(self._ctx, out.ctypes.data), "tgsf_foldback_stats")
         return tuple(int(x) for x in out)
 
+    # -- low-complexity (DUST) screen -----------------------------------------------------------
+    def set_dust(self, level: int = 7, min_frac: float = 0.5) -> None:
+        """tgsf_set_dust: drop every later batch's pieces whose DUST-masked share reaches ``min_frac`` (level 0: off)."""
+        _capi.check(self._lib.tgsf_set_dust(self._ctx, level, min_frac), "tgsf_set_dust")
+
     # -- batches --------------------------------------------------------------------------------
     def submit(self, batch) -> None:
         bases = np.ascontiguousarray(batch.bases, dtype=np.uint8)
@@ -268,6 +273,19 @@ def fold_detect(seqs, device: int = 0) -> np.ndarray:
     out = np.zeros(len(recs), dtype=_capi.FOLD_RESULT_DTYPE)
     _capi.check(lib.tgsf_fold_detect(device, buf.ctypes.data, offs.ctypes.data, len(recs), out.ctypes.data),
                 "tgsf_fold_detect")
+    return out
+
+
+def dust_detect(seqs, level: int = 7, device: int = 0) -> np.ndarray:
+    """tgsf_dust_detect on stand-alone pieces (bytes / str): the DUST-masked bases M of each piece (u32)."""
+    lib = _capi.load()
+    recs = [s.encode() if isinstance(s, str) else bytes(s) for s in seqs]
+    offs = np.zeros(len(recs) + 1, dtype=np.uint64)
+    np.cumsum([len(r) for r in recs], out=offs[1:])
+    buf = np.frombuffer(b"".join(recs) + b"\0", dtype=np.uint8)
+    out = np.zeros(len(recs), dtype=np.uint32)
+    _capi.check(lib.tgsf_dust_detect(device, buf.ctypes.data, offs.ctypes.data, len(recs), level, out.ctypes.data),
+                "tgsf_dust_detect")
     return out
 
 
