@@ -189,7 +189,9 @@ int tgsf_collect_gz(tgsf_ctx *ctx, uint8_t *blob, uint64_t blob_cap, uint64_t *b
 /* Waits for the oldest outstanding batch and copies its results out.  reads: n_reads entries;
  * pieces: up to pieces_cap entries, *n_pieces receives the number produced (TGSF_ERR_CAPACITY and
  * no copy if it exceeds pieces_cap; call again with a larger array).  reads/pieces may be NULL to
- * only retire the batch (counters are still updated). */
+ * only retire the batch (counters are still updated).  A batch with a piece that crowds more distinct keys into one
+ * hash pass of the repeat check or the fold-back screen than their pass split can separate fails with
+ * TGSF_ERR_CAPACITY (tgsf_last_error() says so); nothing of it is copied out. */
 int tgsf_collect(tgsf_ctx *ctx, tgsf_read_result *reads, uint32_t n_reads, tgsf_piece *pieces,
                  uint32_t pieces_cap, uint32_t *n_pieces);
 /* Contaminant screen (an extension; the reference has none).  Installs on this context's device the set of every

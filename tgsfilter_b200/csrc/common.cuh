@@ -86,6 +86,7 @@ struct __align__(16) TmpPiece {
 #define DEV_STATUS_OK 0u
 #define DEV_STATUS_POOL_OVERFLOW 1u
 #define DEV_STATUS_BIN_OVERFLOW 2u
+#define DEV_STATUS_HASH_OVERFLOW 3u // a hash pass of k_kmer or k_fold_global overflowed at its most passes
 
 static __device__ __forceinline__ void atomic_add_u64(u64 *p, u64 v) { atomicAdd(p, v); }
 

@@ -15,8 +15,8 @@
 // shared memory and takes pieces of at most FOLD_SMEM_MAX_LEN bases; a piece that is longer, or whose distinct sampled
 // keys fill 3/4 of the table, goes to a list that k_fold_global works through with a per-CTA table and histogram in
 // global memory (L2).  There the key space is split into passes by hash so that each pass fits the table; a pass that
-// overflows doubles the pass count and restarts the piece.  Which table a key lands in does not change which keys are
-// anchors, so both paths give the same result.
+// overflows doubles the pass count and restarts the piece, up to FOLD_MAX_PASSES.  Which table a key lands in does
+// not change which keys are anchors, so both paths give the same result.
 #pragma once
 #include "common.cuh"
 #include "contam.cuh"
@@ -37,6 +37,9 @@
 #define FOLD_SMEM_BYTES (FOLD_SMEM_SLOTS * 16u + FOLD_SMEM_BINS * 16u)
 #define FOLD_GLOBAL_SLOTS 65536u              // 1 MB table per CTA of k_fold_global
 #define FOLD_GLOBAL_WINDOWS_PER_PASS (3u * FOLD_GLOBAL_SLOTS) // ~3/8 of the table sampled per pass
+// fmix32 is a bijection, so a pass over 1/2^14 of the hash range holds at most 2^15 sampled keys and fits: a pass
+// that overflows at this many passes means the constants above were changed, and the batch fails
+#define FOLD_MAX_PASSES (1u << 14)
 
 struct FoldTable {
     u32 *key, *cnt, *p0, *p1;
@@ -301,6 +304,10 @@ k_fold_global(DevBatch B, tgsf_piece *pieces, const u32 *__restrict__ long_list,
         tgsf_fold_result r;
         while (!fold_piece(seq, L, T, passes, Bn, sh, &r)) {
             __syncthreads();
+            if (passes >= FOLD_MAX_PASSES) {
+                if (threadIdx.x == 0) atomicExch(dev_status, DEV_STATUS_HASH_OVERFLOW);
+                return;
+            }
             passes *= 2;
         }
         if (threadIdx.x == 0) fold_apply(pieces, pi, r, min_len, stats, out);

@@ -9,11 +9,17 @@
 // k_kmer: one CTA per piece; the set is an open-addressing hash table in shared memory (atomicCAS).
 // Pieces with more k-mers than half the table are processed in several passes over disjoint
 // hash partitions of the key space, so any piece length is exact with the same 128 KB table.
+// Nothing bounds how many distinct keys one partition gets (a piece can be built to crowd one), so a
+// pass counts its new keys and stops once they pass 3/4 of the table; the pass is then split in two
+// (twice the passes: partition p of P is exactly partitions 2p and 2p + 1 of 2P, so the passes already
+// done stay counted) and the piece goes on from the first half.  A pass that still overflows at
+// KMER_MAX_PASSES fails the batch with DEV_STATUS_HASH_OVERFLOW.
 #pragma once
 #include "common.cuh"
 
 #define KMER_THREADS 512
 #define KMER_SMEM_BYTES (128 * 1024)
+#define KMER_MAX_PASSES (1u << 24) // the partition is taken from 24 hash bits: more passes separate no more keys
 
 static __device__ __forceinline__ u32 mix32(u64 x) {
     x ^= x >> 33;
@@ -31,14 +37,17 @@ static __device__ __forceinline__ u32 base_code(uint8_t b) { // T.cpp:1709-1724
 template <typename KEY>
 __global__ void __launch_bounds__(KMER_THREADS, 1)
 k_kmer(DevBatch B, DevParams P, tgsf_piece *pieces, const u32 *__restrict__ n_pieces_ptr,
-       u64 *__restrict__ counters, const u32 *__restrict__ dev_status,
-       const u32 *__restrict__ piece_list) { // null (k > 16): all pieces; else the long list k_kmer_tag16 left, n_pieces_ptr counts it
+       u64 *__restrict__ counters, u32 *__restrict__ dev_status,
+       const u32 *__restrict__ piece_list, // null (k > 16): all pieces; else the long list k_kmer_tag16 left, n_pieces_ptr counts it
+       u32 fill_cap) { // new keys one pass may hold, below the table's 3/4 (smaller: tests of the split)
     if (*dev_status != DEV_STATUS_OK) return;
     extern __shared__ __align__(16) uint8_t kmem[];
     KEY *table = (KEY *)kmem;
     constexpr u32 SLOTS = KMER_SMEM_BYTES / sizeof(KEY);
     constexpr KEY EMPTY = (KEY)~(KEY)0;
-    __shared__ u32 s_distinct;
+    // At most `limit` + KMER_THREADS keys get in before every thread has seen s_over: the table never fills.
+    const u32 limit = min(SLOTS / 4u * 3u, fill_cap);
+    __shared__ u32 s_distinct, s_fill, s_over;
     const int k = P.kmer;
     const u64 mask = (k >= 32) ? ~0ull : ((1ull << (2 * k)) - 1ull);
     const u32 n_pieces = *n_pieces_ptr;
@@ -54,15 +63,20 @@ k_kmer(DevBatch B, DevParams P, tgsf_piece *pieces, const u32 *__restrict__ n_pi
             repeat = total - 1; // see oracle/tgsf_oracle.c kmer_repeat_len
         } else {
             const uint8_t *seq = B.bases + B.offsets[pc.read] + (u64)pc.start;
-            const u32 passes = ((u32)total + SLOTS / 2 - 1) / (SLOTS / 2);
+            u32 passes = ((u32)total + SLOTS / 2 - 1) / (SLOTS / 2);
             if (threadIdx.x == 0) s_distinct = 0;
             const int per = (total + KMER_THREADS - 1) / KMER_THREADS;
             const int i0 = min((int)threadIdx.x * per, total), i1 = min(i0 + per, total);
             u32 mine = 0;
-            for (u32 pass = 0; pass < passes; ++pass) {
-                __syncthreads();
+            for (u32 pass = 0; pass < passes;) {
+                __syncthreads(); // every thread has read s_over and is done with the table
                 for (u32 i = threadIdx.x; i < SLOTS; i += KMER_THREADS) table[i] = EMPTY;
+                if (threadIdx.x == 0) {
+                    s_fill = 0;
+                    s_over = 0;
+                }
                 __syncthreads();
+                u32 got = 0;
                 if (i0 < i1) {
                     u64 km = 0;
                     for (int j = 0; j < k - 1; ++j) km = (km << 2) | base_code(seq[i0 + j]);
@@ -70,16 +84,33 @@ k_kmer(DevBatch B, DevParams P, tgsf_piece *pieces, const u32 *__restrict__ n_pi
                         km = ((km << 2) | base_code(seq[i + k - 1])) & mask;
                         const u32 h = mix32(km);
                         if (passes > 1 && (u32)(((u64)(h >> 8) * passes) >> 24) != pass) continue;
+                        if (*(volatile u32 *)&s_over) break;
                         u32 slot = h & (SLOTS - 1);
                         const KEY key = (KEY)km;
                         while (true) {
                             const KEY old = atomicCAS(&table[slot], EMPTY, key);
-                            if (old == EMPTY) { ++mine; break; }
+                            if (old == EMPTY) {
+                                ++got;
+                                if (atomicAdd(&s_fill, 1u) >= limit) *(volatile u32 *)&s_over = 1;
+                                break;
+                            }
                             if (old == key) break;
                             slot = (slot + 1) & (SLOTS - 1);
                         }
                     }
                 }
+                __syncthreads();
+                if (!s_over) { // the pass is complete
+                    mine += got;
+                    ++pass;
+                    continue;
+                }
+                if (passes >= KMER_MAX_PASSES) { // every thread takes this branch: the batch fails
+                    if (threadIdx.x == 0) atomicExch(dev_status, DEV_STATUS_HASH_OVERFLOW);
+                    return;
+                }
+                passes *= 2;
+                pass *= 2;
             }
             atomicAdd(&s_distinct, mine);
             __syncthreads();

@@ -210,6 +210,9 @@ struct Scratch {
     }
 };
 
+// what a batch that ended with DEV_STATUS_HASH_OVERFLOW reports
+#define HASH_OVERFLOW_MSG "a piece crowds more distinct keys into one hash pass than the repeat check or the fold-back screen can split"
+
 struct DevHeader { // small block mirrored to the host with every batch
     u32 status;
     u32 tmp_cursor;  // total pieces
@@ -282,6 +285,7 @@ struct tgsf_ctx {
     int res_ctas_per_sm = 6; // grid of the resolve kernels (k_ends, k_mid_count, k_mid_emit) in CTAs per SM; TGSF_RES_CTAS
     bool fork_ends = true; // TGSF_FORK_ENDS=0: k_ends on the batch's main stream after the middle scan (A/B)
     u32 kmer16_list_cap = KMER16_LIST_CAP; // TGSF_KMER16_LIST_CAP=n: smaller pending list (tests of the retry path)
+    u32 kmer_fill_cap = ~0u; // TGSF_KMER_FILL_CAP=n: at most n new keys per k_kmer pass (tests of the pass split)
     float last_kernel_ms = 0, last_total_ms = 0;
     float last_stage_ms[TGSF_N_STAGES] = {};
     int last_chunk_shift = 0; // middle-scan chunk shift of the last collected batch (tgsf_launch_shape)
@@ -661,7 +665,8 @@ int launch_kmer(tgsf_ctx *c, Slot &s, const DevParams &P) {
     u64 *C = c->counters.as<u64>();
     tgsf_piece *pieces = s.pieces.as<tgsf_piece>();
     if (P.kmer > 16) {
-        k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->tmp_cursor, C, &H->status, nullptr);
+        k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->tmp_cursor, C, &H->status, nullptr,
+                                                                       c->kmer_fill_cap);
         c->launches++;
         return check_launch("k_kmer");
     }
@@ -673,9 +678,11 @@ int launch_kmer(tgsf_ctx *c, Slot &s, const DevParams &P) {
         k_kmer_smem<<<c->sm_count, KMER_SB_THREADS, KMER_SB_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status,
                                                                              long_list);
     else if (P.kmer <= 15)
-        k_kmer<u32><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status, long_list);
+        k_kmer<u32><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status, long_list,
+                                                                       c->kmer_fill_cap);
     else
-        k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status, long_list);
+        k_kmer<u64><<<c->sm_count, KMER_THREADS, KMER_SMEM_BYTES, st>>>(s.B, P, pieces, &H->kmer_long, C, &H->status, long_list,
+                                                                       c->kmer_fill_cap);
     c->launches += 2;
     return check_launch("k_kmer");
 }
@@ -989,6 +996,7 @@ struct RecordPieces {
         Slot &s = slot();
         CU(cudaMemcpyAsync(&h, s.header.p, sizeof(h), cudaMemcpyDeviceToHost, s.stream.get()));
         CU(cudaStreamSynchronize(s.stream.get()));
+        if (h.status == DEV_STATUS_HASH_OVERFLOW) { set_err("%s: %s", fn, HASH_OVERFLOW_MSG); return TGSF_ERR_CAPACITY; }
         if (h.status != DEV_STATUS_OK) { set_err("%s: device status %u", fn, h.status); return TGSF_ERR_CUDA; }
         return TGSF_OK;
     }
@@ -1068,6 +1076,7 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
     // [1, real count]), so that tests reach the launch shapes of multi-Gbase batches with small batches
     if (const char *e = getenv("TGSF_SM_COUNT")) c->sm_count = std::max(1, std::min(c->sm_count, atoi(e)));
     if (const char *e = getenv("TGSF_KMER16_LIST_CAP")) c->kmer16_list_cap = (u32)std::min<long>(std::max<long>(atol(e), 32), (long)KMER16_LIST_CAP);
+    if (const char *e = getenv("TGSF_KMER_FILL_CAP")) c->kmer_fill_cap = (u32)std::min<long long>(std::max<long long>(atoll(e), 1), ~0u);
     *out = c.release();
     return TGSF_OK;
 }
@@ -1497,6 +1506,11 @@ int tgsf_collect(tgsf_ctx *c, tgsf_read_result *reads, uint32_t n_reads, tgsf_pi
     if (H->status == DEV_STATUS_BIN_OVERFLOW) {
         retire();
         set_err("a read is longer than max_read_len allows (per-100 bp bins)");
+        return TGSF_ERR_CAPACITY;
+    }
+    if (H->status == DEV_STATUS_HASH_OVERFLOW) {
+        retire();
+        set_err("%s", HASH_OVERFLOW_MSG);
         return TGSF_ERR_CAPACITY;
     }
     if (H->status != DEV_STATUS_OK) {
