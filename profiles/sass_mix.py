@@ -5,7 +5,8 @@ Compiles tgsfilter_b200/csrc/tgsf_cuda.cu for sm_100a to a cubin (nvcc -cubin -X
 k_mid_scan_dyn<NW, AP> instantiation (cuobjdump -sass) and finds its loops that load 16 bases per iteration
 (LDG.E.128): the halo loop and the tracked loop, which is the hot one.  Prints, per adapter-column (one loop
 iteration is 16 columns for each of the AP adapters), the instructions of each such loop by pipe and by opcode,
-and the registers / stack / spills ptxas reports for the kernel.
+and the registers / stack / spills ptxas reports for the kernel.  `--packed` does the same for k_mid_scan_packed,
+which scans a pair of adapters of <= 50 bp as one 96-bit vector (2 adapter-columns per column).
 
 The pipe of an opcode follows NVIDIA's instruction-set notes: LOP3, IADD3, SHF, ISETP, LEA, SEL, PRMT and the
 integer min/max ops issue to the ALU pipe; IMAD in all its forms (.X, .MOV, .SHL, .IADD) to the FMA pipe.  The
@@ -13,6 +14,7 @@ count is static: every instruction of the loop body once, including the few that
 
     python profiles/sass_mix.py                 # k_mid_scan_dyn<1,2>, the benchmark's instantiation
     python profiles/sass_mix.py --nw 4 --ap 1
+    python profiles/sass_mix.py --packed        # k_mid_scan_packed, what the benchmark's adapter pair runs now
     python profiles/sass_mix.py --cubin x.cubin --ptxas-log x.log   # reuse an earlier compile
 """
 from __future__ import annotations
@@ -110,6 +112,7 @@ def main():
     ap = argparse.ArgumentParser(description=__doc__.split("\n\n")[0])
     ap.add_argument("--nw", type=int, default=1, help="Myers words per adapter (template NW)")
     ap.add_argument("--ap", type=int, default=2, help="adapters per thread (template AP)")
+    ap.add_argument("--packed", action="store_true", help="k_mid_scan_packed (a pair in one 96-bit vector)")
     ap.add_argument("--cubin", help="use this cubin instead of compiling")
     ap.add_argument("--ptxas-log", help="with --cubin: the -Xptxas -v output of that compile")
     args = ap.parse_args()
@@ -120,10 +123,14 @@ def main():
             log = open(args.ptxas_log).read() if args.ptxas_log else ""
         else:
             cubin, log = compile_cubin(tmp)
-        name, body = function_sass(cubin, f"_Z14k_mid_scan_dynILi{args.nw}ELi{args.ap}E")
+        if args.packed:
+            args.ap = 2
+            name, body = function_sass(cubin, "_Z17k_mid_scan_packed")
+        else:
+            name, body = function_sass(cubin, f"_Z14k_mid_scan_dynILi{args.nw}ELi{args.ap}E")
 
     cols = 16 * args.ap
-    print(f"k_mid_scan_dyn<{args.nw},{args.ap}>  ({name})")
+    print(f"k_mid_scan_packed  ({name})" if args.packed else f"k_mid_scan_dyn<{args.nw},{args.ap}>  ({name})")
     if log:
         print(f"  ptxas: {ptxas_resources(log, name)}")
     loops = sorted(loops_with_wide_loads(body), key=lambda lp: lp[1] - lp[0])
@@ -142,7 +149,7 @@ def main():
         print(f"\n  {label}: 0x{lo:x}..0x{hi:x}, {len(ins)} instructions = {len(ins) / cols:.2f} per adapter-column "
               f"({cols} adapter-columns per iteration)")
         for pipe, n in sorted(by_pipe.items(), key=lambda kv: -kv[1]):
-            print(f"    {pipe:10s} {n:5d}  {n / cols:6.2f} per adapter-column")
+            print(f"    {pipe:10s} {n:5d}  {n / cols:6.2f} per adapter-column  {n * args.ap / cols:6.2f} per column")
         print("    by opcode: " + ", ".join(f"{op} {n / cols:.2f}" for op, n in by_op.most_common()))
 
 

@@ -307,6 +307,218 @@ k_mid_scan_dyn(DevBatch B, AdapterCtx C, MidScanArgs M, const u32 *__restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------
+// k_mid_scan_packed: the middle scan of a pair of adapters with q <= 50 (one Myers word each) as a FILTER on one
+// 96-bit vector of three 32-bit words (myers_step_pair96): each adapter keeps its last 48 rows (the top 48 bits of
+// its top-padded HW word: wildcard rows, then the query's last min(q, 48) rows), 3 words of recurrence per column
+// instead of the 4 of two 64-bit words.  The score of a query suffix at an end column is a lower bound on the whole
+// query's score there (restricting an alignment to the suffix rows costs no more), so a chunk whose suffix minimum
+// stays above k holds no column <= k and writes 255 exactly like k_mid_scan_dyn.  Every 8 columns each field's
+// score is read off the state; when the group bound of k_mid_scan_dyn (s_0 + s_8 <= 2k + 8) holds for a field, the
+// group is replayed from its saved start state (pair96_replay_group) and a column whose suffix score is <= k flags
+// the adapter for the chunk.  The replay is needed: with 48 rows the bound alone holds somewhere in ~6 % of the chunks
+// (random text), the suffix minimum is <= k in ~0.2 %.  At the chunk's close a flagged adapter is re-scanned exactly
+// (mid_recheck: the 64-bit HW recurrence) from the first group or column that flagged the chunk, after a halo restart,
+// to the chunk's end: no earlier column can score <= k.  That gives the chunk's minimum, count and first column.
+// Starting there instead of at the chunk's start matters: a warp waits for its slowest lane, so whole-chunk re-checks
+// cost more than the narrower vector saved.  Runs, hand-out, halo and outputs are those of k_mid_scan_dyn<1, 2>.
+// ---------------------------------------------------------------------------------------------
+#define MID_PACKED_ROWS 48
+#define MID_PACKED_MAX_Q 50 // longest adapter routed here: more dropped rows would flag too many chunks
+
+// Rare path of k_mid_scan_packed: whether a column of one 8-column group has a field score <= k (bit 0: field a, bit
+// 1: field b), replayed from the state at the group start.  Out of line, like mid_replay_group.
+static __device__ __noinline__ u32 pair96_replay_group(u32 P0, u32 P1, u32 P2, u32 M0, u32 M1, u32 M2, u32 w0, u32 w1,
+                                                       const uint4 *tab, int ka, int kb) {
+    u32 Pv[3] = {P0, P1, P2}, Mv[3] = {M0, M1, M2};
+    const u32 wd[2] = {w0, w1};
+    u32 hits = 0;
+#pragma unroll 1
+    for (int j = 0; j < 8; ++j) {
+        const uint4 e = tab[(wd[j >> 2] >> (8 * (j & 3))) & 0xffu];
+        const u32 eq[3] = {e.x, e.y, e.z};
+        myers_step_pair96(Pv, Mv, eq);
+        int sa, sb;
+        pair96_scores(Pv, Mv, sa, sb);
+        hits |= (sa <= ka ? 1u : 0u) | (sb <= kb ? 2u : 0u);
+    }
+    return hits;
+}
+
+// Exact close of chunk [from, to) of one adapter (halo restart at sb): chunk minimum if <= k (count and first column
+// recorded, best_mid lowered), 255 otherwise.  Out of line: it runs for a small fraction of the chunks.
+static __device__ __noinline__ uint8_t mid_recheck(const u64 *__restrict__ tab, int qlen, int k,
+                                                   const uint8_t *__restrict__ bases, u64 sb, u64 from, u64 to,
+                                                   u64 slot, u32 *__restrict__ chunk_cnt, u64 *__restrict__ chunk_first,
+                                                   u32 *__restrict__ best_mid_ra) {
+    Myers<1> s;
+    myers_init_hw<1>(s, qlen);
+    int best = 0x7fffffff;
+    u32 cnt = 0;
+    u64 first = 0;
+    for (u64 p = sb; p < to; ++p) {
+        myers_step<1, 0, true>(s, tab + __ldg(bases + p), 0);
+        if (p >= from) {
+            if (s.score < best) { best = s.score; cnt = 1; first = p; }
+            else if (s.score == best) ++cnt;
+        }
+    }
+    if (best > k) return 255;
+    atomicMin(best_mid_ra, (u32)best);
+    chunk_cnt[slot] = cnt;
+    chunk_first[slot] = first | ((u64)best << 48);
+    return (uint8_t)min(best, 254);
+}
+
+__global__ void __launch_bounds__(MID_THREADS, 6)
+k_mid_scan_packed(DevBatch B, AdapterCtx C, MidScanArgs M, const u32 *__restrict__ chunk_off,
+                  const ChunkEntry *__restrict__ runs, const u32 *__restrict__ perm,
+                  const u32 *__restrict__ n_runs_ptr, uint8_t *__restrict__ chunk_min,
+                  u32 *__restrict__ chunk_cnt, u64 *__restrict__ chunk_first,
+                  u32 *__restrict__ best_mid, u32 *__restrict__ work_ctr) {
+    const u32 n_runs = *n_runs_ptr;
+    __shared__ uint4 s_tab[256]; // per byte value: the 96-bit pair column in .x .y .z, .w unused (one LDS.128)
+    DevAdapter A[2];
+    const u64 *hw[2];
+#pragma unroll
+    for (int x = 0; x < 2; ++x) {
+        A[x] = C.ad[M.a[x]];
+        hw[x] = C.peq_pool + A[x].peq_off;
+    }
+    for (int i = threadIdx.x; i < 256; i += MID_THREADS) {
+        const u64 fa = hw[0][i] >> (64 - MID_PACKED_ROWS), fb = hw[1][i] >> (64 - MID_PACKED_ROWS);
+        s_tab[i] = make_uint4((u32)fa, (u32)(fa >> 32) | ((u32)fb << 16), (u32)(fb >> 16), 0u);
+    }
+    __syncthreads();
+    const int cs = M.chunk_shift;
+    const u64 chunk_len = 1ull << cs;
+    const int halo = max(A[0].halo_mid, A[1].halo_mid), qmin = min(A[0].qlen, A[1].qlen);
+    const int k[2] = {A[0].k_mid, A[1].k_mid};
+    const int thr0[2] = {2 * k[0] + 8, 2 * k[1] + 8};
+    // state before column 0: the query rows of each field start at +1 (the top 48 bits of myers_init_hw)
+    u32 P0[3];
+    {
+        const u64 ia = ~0ull << (64 - A[0].qlen) >> (64 - MID_PACKED_ROWS);
+        const u64 ib = ~0ull << (64 - A[1].qlen) >> (64 - MID_PACKED_ROWS);
+        P0[0] = (u32)ia;
+        P0[1] = (u32)(ia >> 32) | ((u32)ib << 16);
+        P0[2] = (u32)(ib >> 16);
+    }
+    const uint4 *__restrict__ b16 = (const uint4 *)B.bases;
+
+    const u32 lane = threadIdx.x & 31u;
+    for (;;) { // dynamic hand-out and run geometry as in k_mid_scan_dyn
+        u32 it = 0;
+        if (lane == 0) it = atomicAdd(work_ctr, 32u);
+        it = __shfl_sync(0xffffffffu, it, 0);
+        if (it >= n_runs) break;
+        it += lane;
+        if (it >= n_runs) continue;
+        const ChunkEntry re = runs[perm[it]];
+        const u64 rs = B.offsets[re.read];
+        const i64 tsm = (i64)(B.offsets[re.read + 1] - rs) - 2 * (i64)M.end_len;
+        const u64 mb = rs + (u64)M.end_len, me = B.offsets[re.read + 1] - (u64)M.end_len;
+        const u32 c_first = (u32)(mb >> cs);
+        u32 c = max(re.chunk << M.run_shift, c_first);
+        const u32 c_last = min(((re.chunk + 1) << M.run_shift) - 1u, (u32)((me - 1) >> cs));
+        u32 ci = chunk_off[re.read] + (c - c_first);
+
+        u32 Pv[3] = {P0[0], P0[1], P0[2]}, Mv[3] = {0u, 0u, 0u};
+        bool on[2];
+#pragma unroll
+        for (int x = 0; x < 2; ++x) on[x] = tsm >= (i64)A[x].qlen; // both have k_mid > 0 (routing)
+        const bool scan = tsm >= (i64)qmin;
+        bool flag[2] = {false, false}; // the chunk holds a column whose suffix score is <= k, for adapter x
+        u64 lo = ~0ull;                // no such column of either adapter lies before lo
+        int sa = 0, sb_ = 0;           // field scores at the last group end
+        u64 ob = max((u64)c << cs, mb);
+        u64 sb = ob > (u64)halo ? ob - (u64)halo : 0;
+        if (sb < mb) sb = mb;
+        u64 p = sb;
+        auto column = [&](u32 byte) {
+            const uint4 v = s_tab[byte];
+            const u32 eq[3] = {v.x, v.y, v.z};
+            myers_step_pair96(Pv, Mv, eq);
+        };
+        auto flag_column = [&]() { // one column scored on its own (head and tail)
+            pair96_scores(Pv, Mv, sa, sb_);
+            if (sa <= k[0] || sb_ <= k[1]) lo = min(lo, p);
+            flag[0] |= sa <= k[0];
+            flag[1] |= sb_ <= k[1];
+        };
+        if (scan) {
+            const u64 oe0 = min(((u64)c << cs) + chunk_len, me);
+            while (p < oe0 && (p & 15ull)) {
+                column(B.bases[p]);
+                if (p >= ob) flag_column();
+                ++p;
+            }
+            for (; p < ob; p += 16) {
+                const uint4 v = __ldg(b16 + (p >> 4));
+                const u32 wd[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                for (int j = 0; j < 16; ++j) column((wd[j >> 2] >> (8 * (j & 3))) & 0xffu);
+            }
+            pair96_scores(Pv, Mv, sa, sb_);
+        }
+        for (;;) {
+            const u64 cb = (u64)c << cs;
+            const u64 oe = min(cb + chunk_len, me);
+            if (scan && p < oe) {
+                const uint4 *q = b16 + (p >> 4);
+                for (u32 g = (u32)((oe - p) >> 4); g; --g, ++q) {
+                    const uint4 v = __ldg(q);
+                    const u32 wd[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        const u32 P0g[3] = {Pv[0], Pv[1], Pv[2]}, M0g[3] = {Mv[0], Mv[1], Mv[2]};
+#pragma unroll
+                        for (int j = 8 * h; j < 8 * h + 8; ++j) {
+                            const uint4 e = *(const uint4 *)((const char *)s_tab + mid_row_off(wd, j, M.byte_mul));
+                            const u32 eq[3] = {e.x, e.y, e.z};
+                            myers_step_pair96(Pv, Mv, eq);
+                        }
+                        int ea, eb;
+                        pair96_scores(Pv, Mv, ea, eb);
+                        if (sa + ea <= thr0[0] || sb_ + eb <= thr0[1]) {
+                            const u32 hits = pair96_replay_group(P0g[0], P0g[1], P0g[2], M0g[0], M0g[1], M0g[2],
+                                                                 wd[2 * h], wd[2 * h + 1], s_tab, k[0], k[1]);
+                            if (hits) lo = min(lo, ((u64)(q - b16) << 4) + 8 * h);
+                            flag[0] |= (hits & 1u) != 0;
+                            flag[1] |= (hits & 2u) != 0;
+                        }
+                        sa = ea;
+                        sb_ = eb;
+                    }
+                }
+                p = oe & ~15ull;
+                for (; p < oe; ++p) {
+                    column(B.bases[p]);
+                    flag_column();
+                }
+            }
+            // close chunk ci: columns <= k lie in [lo, oe)
+            const u64 cob = max(max(cb, mb), lo == ~0ull ? 0 : lo);
+            u64 csb = cob > (u64)halo ? cob - (u64)halo : 0;
+            if (csb < mb) csb = mb;
+#pragma unroll
+            for (int x = 0; x < 2; ++x) {
+                const u64 slot = (u64)M.a[x] * M.chunk_stride + ci;
+                uint8_t result = 255;
+                if (on[x] && flag[x])
+                    result = mid_recheck(hw[x], A[x].qlen, k[x], B.bases, csb, cob, oe, slot, chunk_cnt,
+                                         chunk_first, best_mid + (u64)re.read * M.n_adapters + M.a[x]);
+                chunk_min[slot] = result;
+                flag[x] = false;
+            }
+            lo = ~0ull;
+            if (c == c_last) break;
+            ++c;
+            ++ci;
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // Enumerate, in ascending order, the end columns of the middle window of read r whose HW score
 // equals d, visiting only the chunks whose minimum is d.  f(p) is called with the absolute byte
 // offset of each such column; return false from f to stop.

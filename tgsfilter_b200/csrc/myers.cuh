@@ -123,6 +123,53 @@ static __device__ __forceinline__ int myers_score(const u64 (&Pv)[NW], const u64
     return s;
 }
 
+// 96-bit add through the carry flag (IADD3, IADD3.X, and IMAD.X on the FMA pipe for the top word).
+static __device__ __forceinline__ void add96(u32 (&r)[3], const u32 (&a)[3], const u32 (&b)[3]) {
+    asm("add.cc.u32 %0, %3, %6;\n\taddc.cc.u32 %1, %4, %7;\n\taddc.u32 %2, %5, %8;"
+        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2])
+        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(b[0]), "r"(b[1]), "r"(b[2]));
+}
+
+// HW column of a PACKED PAIR (k_mid_scan_packed): two independent 48-row top-padded HW fields in one 96-bit vector of
+// three 32-bit words, field a in bits [0, 48), field b in bits [48, 96).  Field b's top row (bit 48) must see the HW
+// boundary (horizontal delta 0), not field a's bottom row (bit 47 = bit 15 of word 1), so nothing may cross from bit
+// 47 into bit 48:
+//   - bit 47 of Ph and Mh is cleared before the shifts, so 0 comes in at bit 48 (the Mh mask folds into its LOP3);
+//   - the add (Eq & Pv) + Pv runs with bit 47 of both addends cleared, so it carries nothing into bit 48.  Its sum bit
+//     47 is then wrong, and so is Xh's, but bit 47 of Xh only reaches bit 47 of Ph and Mh, which are cleared anyway.
+// Shifts are adds of a vector to itself, so they carry between the words like the add.
+static __device__ __forceinline__ void myers_step_pair96(u32 (&Pv)[3], u32 (&Mv)[3], const u32 (&Eq)[3]) {
+    constexpr u32 H = ~(1u << 15);
+    const u32 Pm[3] = {Pv[0], Pv[1] & H, Pv[2]};
+    const u32 t[3] = {Eq[0] & Pv[0], Eq[1] & Pv[1] & H, Eq[2] & Pv[2]};
+    u32 sum[3], Ph[3], Mh[3];
+    add96(sum, t, Pm);
+#pragma unroll
+    for (int w = 0; w < 3; ++w) {
+        const u32 Xh = (sum[w] ^ Pv[w]) | Eq[w];
+        Ph[w] = Mv[w] | ~(Xh | Pv[w]);
+        Mh[w] = Pv[w] & Xh;
+    }
+    Ph[1] &= H;
+    Mh[1] &= H;
+    add96(Ph, Ph, Ph);
+    add96(Mh, Mh, Mh);
+#pragma unroll
+    for (int w = 0; w < 3; ++w) {
+        const u32 Xv = Eq[w] | Mv[w];
+        Pv[w] = Mh[w] | ~(Xv | Ph[w]);
+        Mv[w] = Ph[w] & Xv;
+    }
+}
+
+// Bottom-row scores of the two fields of a packed pair (vertical deltas of the top-padded rows, as myers_score).
+// Field a's rows in word 1 are counted once and moved from b's sum to a's.
+static __device__ __forceinline__ void pair96_scores(const u32 (&Pv)[3], const u32 (&Mv)[3], int &sa, int &sb) {
+    const int a_hi = __popc(Pv[1] << 16) - __popc(Mv[1] << 16);
+    sa = __popc(Pv[0]) - __popc(Mv[0]) + a_hi;
+    sb = __popc(Pv[1]) - __popc(Mv[1]) + __popc(Pv[2]) - __popc(Mv[2]) - a_hi;
+}
+
 // Measured and rejected (round 1): moving the 64-bit add and the two 1-bit shifts onto the FMA pipe
 // with mad.wide.u32 (IMAD.WIDE) made k_mid_scan 21 % slower (12.0 -> 14.6 ms on config[1]): ALU-pipe
 // instructions fell from 20.2 to 17.5 per column but IMAD.WIDE.U32 issues at about a quarter of the

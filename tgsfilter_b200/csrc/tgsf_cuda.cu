@@ -602,12 +602,16 @@ int launch_head(tgsf_ctx *c, Slot &s) {
                 M.byte_mul[0] = 1u << 24;
                 M.byte_mul[1] = 1u << 16;
                 M.byte_mul[2] = 1u << 8;
+                // a pair of adapters of at most 50 bp runs as one 96-bit filter vector (k_mid_scan_packed): dropping
+                // their first <= 2 rows leaves the filter flagging well under 1 % of the chunks for an exact re-check
+                const bool packed = pair && c->ads.host[(size_t)M.a[0]].qlen <= MID_PACKED_MAX_Q &&
+                                    c->ads.host[(size_t)M.a[1]].qlen <= MID_PACKED_MAX_Q;
                 TRY(for_nw(nw, [&](auto nwc) {
                     constexpr int NW = decltype(nwc)::value;
-                    // AP adapters per thread: the table row of a byte value is AP * NW words, and so is the row
-                    // stride mid_row_off scales by
-                    auto launch = [&](auto kern, size_t smem, int ap) {
-                        M.byte_mul[3] = (u32)(8 * ap * NW);
+                    // row_bytes: the table row of a byte value, the stride mid_row_off scales by (AP * NW words in
+                    // k_mid_scan_dyn, 16 bytes in k_mid_scan_packed)
+                    auto launch = [&](auto kern, size_t smem, u32 row_bytes) {
+                        M.byte_mul[3] = row_bytes;
                         int occ = 0; // persistent grid: exactly the resident CTA count
                         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, MID_THREADS, smem) != cudaSuccess || occ < 1) occ = 4;
                         if (c->mid_ctas_per_sm > 0) occ = std::min(occ, c->mid_ctas_per_sm);
@@ -617,10 +621,11 @@ int launch_head(tgsf_ctx *c, Slot &s) {
                             s.best_mid.as<u32>(), s.mid_work.as<u32>() + mid_launch);
                     };
                     if constexpr (NW <= 4) {
-                        if (pair) launch(k_mid_scan_dyn<NW, 2>, 256 * 2 * NW * sizeof(u64), 2);
-                        else launch(k_mid_scan_dyn<NW, 1>, 256 * NW * sizeof(u64), 1);
+                        if (packed) launch(k_mid_scan_packed, 0, 16);
+                        else if (pair) launch(k_mid_scan_dyn<NW, 2>, 256 * 2 * NW * sizeof(u64), 8 * 2 * NW);
+                        else launch(k_mid_scan_dyn<NW, 1>, 256 * NW * sizeof(u64), 8 * NW);
                     } else {
-                        launch(k_mid_scan_dyn<NW, 1>, 0, 1); // table read from global memory
+                        launch(k_mid_scan_dyn<NW, 1>, 0, 8 * NW); // table read from global memory
                     }
                     c->launches++;
                     ++mid_launch;
