@@ -208,6 +208,41 @@ int tgsf_collect(tgsf_ctx *ctx, tgsf_read_result *reads, uint32_t n_reads, tgsf_
  * kernels are timed in TGSF_STAGE_KMER. */
 int tgsf_set_contaminants(tgsf_ctx *ctx, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs, int32_t k,
                           float min_frac, uint64_t *n_kmers);
+/* Per-record attribution of the contaminant screen.  Installs the set exactly as tgsf_set_contaminants does (same
+ * checks, errors, screen and piece statuses) and also labels every key with the record it came from: records are
+ * r = 0 .. n_seqs - 1 in order; a key gets label r when every valid window of the set that carries it lies in record
+ * r, and label SHARED when it occurs in two or more records (a record and its reverse complement share every key).
+ * record_kmers[r] (r < n_seqs) receives the number of keys labelled r and record_kmers[n_seqs] the number of shared
+ * keys; they add up to *n_kmers.  n_seqs <= TGSF_CONTAM_MAX_RECORDS, otherwise TGSF_ERR_INVALID.
+ * Vote of a screened piece: v_r = its valid windows whose key has label r (each occurrence counts; shared keys vote
+ * for no one).  Its record is the r with the largest v_r >= 1 (smallest r on a tie) with record_hits = v_r; else, when
+ * contam_hits >= 1, the shared row n_seqs with record_hits = 0; else -1.  From the next batch on, every piece that
+ * becomes TGSF_PIECE_CONTAM adds 1 to reads[record] and its len to bases[record] (tgsf_contam_record_stats), so the
+ * rows add up to the contaminant pieces.  The call resets the tallies; a later tgsf_set_contaminants replaces the set
+ * and turns attribution off.  The attribution kernels run after the threshold, only over the pieces it marked, and
+ * are timed in TGSF_STAGE_KMER; the label array costs 4 bytes per table slot (half the table). */
+#define TGSF_CONTAM_MAX_RECORDS 0x7FFFFFFEu
+int tgsf_set_contaminants_labelled(tgsf_ctx *ctx, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs,
+                                   int32_t k, float min_frac, uint64_t *n_kmers, uint64_t *record_kmers);
+/* Cumulative tallies since tgsf_set_contaminants_labelled or tgsf_counters_reset (all batches must have been
+ * collected, else TGSF_ERR_STATE): reads[r] contaminant pieces and bases[r] their bases attributed to record r,
+ * row n_seqs the pieces whose hits all have shared keys.  n must be n_seqs + 1 and the installed set must be
+ * labelled, otherwise TGSF_ERR_INVALID. */
+int tgsf_contam_record_stats(tgsf_ctx *ctx, uint64_t *reads, uint64_t *bases, uint32_t n);
+/* The screen's and the attribution's kernels on n stand-alone pieces seq[offsets[i], offsets[i+1]) (host buffers,
+ * offsets[0] == 0, each piece < 2^31 bases) against the installed labelled set: hits = contam_hits, record and
+ * record_hits as above for every piece with hits >= 1 (not only the contaminant ones; record -1 and record_hits 0
+ * otherwise), contam = 1 when the piece would become TGSF_PIECE_CONTAM.  Touches no counter and no tally.  Bad
+ * arguments give TGSF_ERR_INVALID before the device is touched; TGSF_ERR_STATE while a batch is outstanding or
+ * without a labelled set; n = 0 touches nothing. */
+typedef struct tgsf_contam_class {
+    int32_t hits;
+    int32_t record;
+    int32_t record_hits;
+    int32_t contam;
+} tgsf_contam_class;
+int tgsf_contam_classify(tgsf_ctx *ctx, const uint8_t *seq, const uint64_t *offsets, uint32_t n,
+                         tgsf_contam_class *out);
 
 /* Fold-back screen (an extension; the reference has none).  A piece that reads through a junction without adapter
  * is one strand followed by its own reverse complement, X·rc(X').  Rules, on piece-relative positions of s[0, L):

@@ -74,6 +74,7 @@ struct Params {
     string ContamFile;            // --contam (extension): drop pieces that share k-mers with this FASTA
     int ContamK = 17;             // --contam-k
     float ContamFrac = 0.05f;     // --contam-frac
+    string ContamReport;          // --contam-report: TSV of the contaminant pieces per --contam record
     bool Foldback = false;        // --foldback (extension): cut pieces at a fold-back junction, keep the longer arm
     bool Dust = false;            // --dust (extension): drop pieces dominated by low-complexity sequence
     int DustLevel = 7;            // --dust-level
@@ -128,6 +129,7 @@ int usage() {
                  "   --contam <str>        FASTA[.gz] of contaminant sequences; pieces sharing enough k-mers are discarded\n"
                  "   --contam-k <int>      k-mer size of the contaminant screen, 11-31 [17]\n"
                  "   --contam-frac <float> min fraction of a piece's k-mers found in the set to discard it [0.05]\n"
+                 "   --contam-report <str> write the discarded reads and bases per --contam record to this TSV file\n"
                  " Fold-back screen:\n"
                  "   --foldback            cut reads that fold back onto their own reverse complement, keep the longer arm\n"
                  " Low-complexity screen:\n"
@@ -205,6 +207,7 @@ int parse_cmd(int argc, char **argv, Params *P) {
         else if (flag == "contam") { if (!need()) return 1; P->ContamFile = argv[i]; }
         else if (flag == "contamk") { if (!need()) return 1; P->ContamK = atoi(argv[i]); }
         else if (flag == "contamfrac") { if (!need()) return 1; P->ContamFrac = (float)atof(argv[i]); }
+        else if (flag == "contamreport") { if (!need()) return 1; P->ContamReport = argv[i]; }
         else if (flag == "adapterdenovo") { P->Denovo = true; }
         else if (flag == "foldback") { P->Foldback = true; }
         else if (flag == "dust") { P->Dust = true; }
@@ -221,6 +224,7 @@ int parse_cmd(int argc, char **argv, Params *P) {
         cerr << "Error: --contam-frac must be in (0,1]" << endl;
         exit(-1);
     }
+    if (!P->ContamReport.empty() && P->ContamFile.empty()) { cerr << "Error: --contam-report requires --contam" << endl; exit(-1); }
     if (!P->ContamFile.empty()) {
         if (P->OnlyQC || P->ONLYAD || !P->Filter) {
             cerr << "Error: --contam screens filtered reads and cannot be combined with --qc, -A or -F" << endl;
@@ -274,15 +278,18 @@ int parse_cmd(int argc, char **argv, Params *P) {
     return 0;
 }
 
-// Contaminant FASTA (multi-line, plain or gzip): records back to back in seq, offs[i]..offs[i+1].
-bool load_contam_fasta(const string &path, std::vector<uint8_t> &seq, std::vector<uint64_t> &offs) {
+// Contaminant FASTA (multi-line, plain or gzip): records back to back in seq, offs[i]..offs[i+1]; names[i] is record
+// i's header up to the first space, tab or '\r' (empty for a sequence before the first '>').
+bool load_contam_fasta(const string &path, std::vector<uint8_t> &seq, std::vector<uint64_t> &offs,
+                       std::vector<string> &names) {
     gzFile f = gzopen(path.c_str(), "rb");
     if (!f) return false;
     gzbuffer(f, 1 << 20);
     seq.clear();
     offs.assign(1, 0);
+    names.clear();
     std::vector<char> line(1 << 16);
-    bool in_rec = false, at_bol = true, header = false;
+    bool in_rec = false, at_bol = true, header = false, in_name = false;
     int n;
     while ((n = gzread(f, line.data(), (unsigned)line.size())) > 0) {
         for (int i = 0; i < n; ++i) {
@@ -292,7 +299,14 @@ bool load_contam_fasta(const string &path, std::vector<uint8_t> &seq, std::vecto
                 if (in_rec) offs.push_back(seq.size());
                 in_rec = true;
                 header = true;
-            } else if (!header && ch != '\r' && ch != ' ' && ch != '\t') {
+                in_name = true;
+                names.emplace_back();
+            } else if (header) {
+                if (ch == ' ' || ch == '\t' || ch == '\r') in_name = false;
+                else if (in_name) names.back().push_back(ch);
+            } else if (ch != '\r' && ch != ' ' && ch != '\t') {
+                if (!in_rec) names.emplace_back(); // a sequence before the first '>': a record without a name
+
                 in_rec = true;
                 seq.push_back((uint8_t)ch);
             }
@@ -1020,8 +1034,10 @@ std::vector<string> resolve_adapters(Params &P, bool has_qual, const Sample &S) 
 }
 
 // ---- contexts: one per GPU, with the contaminant set (--contam), the fold-back screen (--foldback) and the DUST screen (--dust) on each
+// --contam-report: the set is installed with labels and record_kmers receives the keys per record (shared keys last).
 std::vector<tgsf_ctx *> create_contexts(const Params &P, int qType, const std::vector<string> &adapters, bool gz_gpu,
-                                        std::vector<uint8_t> &contam_seq, const std::vector<uint64_t> &contam_offs) {
+                                        std::vector<uint8_t> &contam_seq, const std::vector<uint64_t> &contam_offs,
+                                        std::vector<uint64_t> &record_kmers) {
     tgsf_params tp;
     memset(&tp, 0, sizeof(tp));
     tp.min_len = P.MinLen; tp.max_len = P.MaxLen; tp.min_q = P.MinQ; tp.max_q = P.MaxQ;
@@ -1052,10 +1068,18 @@ std::vector<tgsf_ctx *> create_contexts(const Params &P, int qType, const std::v
         if (tgsf_create(g % n_dev, &tp, &ctx[(size_t)g]) != TGSF_OK) die_tgsf("tgsf_create");
     if (!P.ContamFile.empty()) {
         uint64_t n_kmers = 0;
-        for (int g = 0; g < P.gpus; g++)
-            if (tgsf_set_contaminants(ctx[(size_t)g], contam_seq.data(), contam_offs.data(), (uint32_t)(contam_offs.size() - 1),
-                                      P.ContamK, P.ContamFrac, &n_kmers) != TGSF_OK)
-                die_tgsf("tgsf_set_contaminants");
+        const uint32_t n_seqs = (uint32_t)(contam_offs.size() - 1);
+        if (!P.ContamReport.empty()) record_kmers.assign((size_t)n_seqs + 1, 0);
+        for (int g = 0; g < P.gpus; g++) {
+            if (P.ContamReport.empty()) {
+                if (tgsf_set_contaminants(ctx[(size_t)g], contam_seq.data(), contam_offs.data(), n_seqs, P.ContamK,
+                                          P.ContamFrac, &n_kmers) != TGSF_OK)
+                    die_tgsf("tgsf_set_contaminants");
+            } else if (tgsf_set_contaminants_labelled(ctx[(size_t)g], contam_seq.data(), contam_offs.data(), n_seqs,
+                                                      P.ContamK, P.ContamFrac, &n_kmers, record_kmers.data()) != TGSF_OK) {
+                die_tgsf("tgsf_set_contaminants_labelled");
+            }
+        }
         cerr << "INFO: " << n_kmers << " distinct " << P.ContamK << "-mers loaded from " << P.ContamFile << "." << endl;
         std::vector<uint8_t>().swap(contam_seq);
     }
@@ -1620,6 +1644,27 @@ void report_filter(const Params &P, std::vector<tgsf_ctx *> &ctx, const MainPass
     }
 }
 
+// ---- --contam-report: the contaminant pieces per record, summed over the contexts --------------------------------------
+void write_contam_report(FILE *f, const string &path, std::vector<tgsf_ctx *> &ctx, const std::vector<string> &names,
+                         const std::vector<uint64_t> &offs, const std::vector<uint64_t> &record_kmers) {
+    const uint32_t rows = (uint32_t)names.size() + 1;
+    std::vector<uint64_t> reads(rows, 0), bases(rows, 0), r(rows), b(rows);
+    for (tgsf_ctx *c : ctx) {
+        if (tgsf_contam_record_stats(c, r.data(), b.data(), rows) != TGSF_OK) die_tgsf("tgsf_contam_record_stats");
+        for (uint32_t i = 0; i < rows; ++i) { reads[i] += r[i]; bases[i] += b[i]; }
+    }
+    string out = "#record\tname\tlength\tunique_kmers\treads\tbases\n";
+    for (uint32_t i = 0; i + 1 < rows; ++i)
+        out += std::to_string(i) + "\t" + names[i] + "\t" + std::to_string(offs[i + 1] - offs[i]) + "\t" +
+               std::to_string(record_kmers[i]) + "\t" + std::to_string(reads[i]) + "\t" + std::to_string(bases[i]) + "\n";
+    out += "*\tshared\t.\t" + std::to_string(record_kmers[rows - 1]) + "\t" + std::to_string(reads[rows - 1]) + "\t" +
+           std::to_string(bases[rows - 1]) + "\n";
+    if (fwrite(out.data(), 1, out.size(), f) != out.size() || fclose(f) != 0) {
+        cerr << "Error: Failed to write --contam-report " << path << endl;
+        quit(1);
+    }
+}
+
 // ---- downsampling: DownSampleTask (T.cpp:2164-2568) ----------------------------------------------------
 // Selects the reads, writes them in file order from the filtered records (-F: the input) and recomputes the QC tables
 // of the kept reads on the GPU (a QC-only context: its "raw" tables are the report's "after" column).
@@ -1760,10 +1805,16 @@ int main(int argc, char **argv) {
     if (const char *e = getenv("TGSF_GPUS")) P.gpus = std::max(1, atoi(e));
     if (parse_cmd(argc, argv, &P) == 1) return 1;
     std::vector<uint8_t> contam_seq;
-    std::vector<uint64_t> contam_offs;
+    std::vector<uint64_t> contam_offs, record_kmers;
+    std::vector<string> contam_names;
+    FILE *contam_report = nullptr;
     if (!P.ContamFile.empty()) {
-        if (!load_contam_fasta(P.ContamFile, contam_seq, contam_offs)) { cerr << "Error: Failed to read --contam " << P.ContamFile << endl; return 1; }
+        if (!load_contam_fasta(P.ContamFile, contam_seq, contam_offs, contam_names)) { cerr << "Error: Failed to read --contam " << P.ContamFile << endl; return 1; }
         if (contam_offs.size() < 2 || contam_seq.empty()) { cerr << "Error: no sequence in --contam " << P.ContamFile << endl; return 1; }
+        if (!P.ContamReport.empty() && !(contam_report = fopen(P.ContamReport.c_str(), "w"))) {
+            cerr << "Error: Failed to open file for --contam-report " << P.ContamReport << endl;
+            return 1;
+        }
     }
     for (int i = 0; i < 256; i++) g_comp[i] = 'N';
     const char *pairs[] = {"AT", "GC", "CG", "TA", "at", "gc", "cg", "ta", "MK", "RY", "WW", "SS", "YR", "KM",
@@ -1787,7 +1838,7 @@ int main(int argc, char **argv) {
         tlog("gpu prepass + resolve", T_ph.lap());
         // .gz output: the deflate blocks of every record are produced on the GPU (TGSF_GZ_HOST=1: host zlib instead)
         const bool gz_gpu = P.OUTGZ && !P.Downsample && !P.OnlyQC && !getenv("TGSF_GZ_HOST");
-        std::vector<tgsf_ctx *> ctx = create_contexts(P, qType, adapters, gz_gpu, contam_seq, contam_offs);
+        std::vector<tgsf_ctx *> ctx = create_contexts(P, qType, adapters, gz_gpu, contam_seq, contam_offs, record_kmers);
         tlog("tgsf_create", T_ph.lap());
         w.reset(new Writer(P, in->pool));
         const MainPass M = feed(*in, ctx, *w, has_qual, gz_gpu, has_qual && P.Outfq == 1 ? 1.0 : 0.5, clean_exit);
@@ -1798,6 +1849,7 @@ int main(int argc, char **argv) {
         tlog("main pass total", T_ph.lap());
         in->close();
         report_filter(P, ctx, M, *w, has_qual, rawSide, cleanSide);
+        if (contam_report) write_contam_report(contam_report, P.ContamReport, ctx, contam_names, contam_offs, record_kmers);
         if (clean_exit) for (tgsf_ctx *c : ctx) tgsf_destroy(c);
     }
     if (P.Downsample) downsample(P, qType, w ? std::move(w->kept) : Filtered(), cleanSide);

@@ -111,6 +111,8 @@ ALIGN_RESULT_DTYPE = [("edit_distance", "<i4"), ("n_locations", "<i4"), ("align_
                       ("first_start", "<i4"), ("first_end", "<i4"), ("last_start", "<i4"),
                       ("last_end", "<i4"), ("loc_hash", "<u4")]
 FOLD_RESULT_DTYPE = [("fold", "<i4"), ("anchors", "<i4"), ("centre", "<i4"), ("min_gap", "<i4")]
+CONTAM_CLASS_DTYPE = [("hits", "<i4"), ("record", "<i4"), ("record_hits", "<i4"), ("contam", "<i4")]
+CONTAM_MAX_RECORDS = 0x7FFFFFFE
 
 # every symbol include/tgsf.h declares; tests check the built library exports all of them
 EXPORTED_SYMBOLS = (
@@ -119,7 +121,7 @@ EXPORTED_SYMBOLS = (
     "tgsf_counter_layout_get", "tgsf_counters", "tgsf_counters_reset", "tgsf_counters_device",
     "tgsf_launch_count", "tgsf_launch_shape", "tgsf_mid_run_shift", "tgsf_allreduce", "tgsf_prepass", "tgsf_align_hw", "tgsf_set_contaminants",
     "tgsf_end_kmer_counts", "tgsf_set_foldback", "tgsf_foldback_stats", "tgsf_fold_detect", "tgsf_set_dust",
-    "tgsf_dust_detect",
+    "tgsf_dust_detect", "tgsf_set_contaminants_labelled", "tgsf_contam_record_stats", "tgsf_contam_classify",
 )
 
 _lib = None
@@ -174,6 +176,10 @@ def load() -> C.CDLL:
     lib.tgsf_fold_detect.argtypes = [C.c_int, u8p, u64p, C.c_uint32, vp]
     lib.tgsf_set_dust.argtypes = [vp, C.c_int32, C.c_float]
     lib.tgsf_dust_detect.argtypes = [C.c_int, u8p, u64p, C.c_uint32, C.c_int32, vp]
+    lib.tgsf_set_contaminants_labelled.argtypes = [vp, u8p, u64p, C.c_uint32, C.c_int32, C.c_float,
+                                                   C.POINTER(C.c_uint64), u64p]
+    lib.tgsf_contam_record_stats.argtypes = [vp, u64p, u64p, C.c_uint32]
+    lib.tgsf_contam_classify.argtypes = [vp, u8p, u64p, C.c_uint32, vp]
     for name in EXPORTED_SYMBOLS:
         fn = getattr(lib, name)
         if fn.restype is C.c_int and name not in ("tgsf_version", "tgsf_last_error",

@@ -75,11 +75,23 @@ static __device__ __forceinline__ bool contam_lookup(const u64 *__restrict__ tab
     }
 }
 
+#define CONTAM_LABEL_EMPTY 0xFFFFFFFFu  // label array (tgsf_set_contaminants_labelled): slot without a key
+#define CONTAM_LABEL_SHARED 0xFFFFFFFEu // the key occurs in two or more records
+
+// Label of the key at slot i seen in record r: the first record wins the CAS, any other record makes it SHARED.
+// Once a label is not EMPTY it only ever becomes SHARED, so the result does not depend on the order of the atomics.
+static __device__ __forceinline__ void contam_label_set(u32 *label, u32 r) {
+    const u32 old = atomicCAS(label, CONTAM_LABEL_EMPTY, r);
+    if (old != CONTAM_LABEL_EMPTY && old != r) *label = CONTAM_LABEL_SHARED;
+}
+
 // Build: thread t owns the window END positions [t*SEG, (t+1)*SEG) of the concatenated records and rolls in from k - 1
-// bytes before (clamped to its record); windows never span two records.  *n_inserted += successful inserts.
+// bytes before (clamped to its record); windows never span two records.  *n_inserted += successful inserts.  LABELS:
+// also label every key's slot with its record in labels[] (parallel to the table).
+template <bool LABELS>
 __global__ void __launch_bounds__(256)
 k_contam_build(const uint8_t *__restrict__ seq, const u64 *__restrict__ offs, u32 n_seqs, int k, u64 *table, u64 mask,
-               unsigned long long *n_inserted) {
+               unsigned long long *n_inserted, u32 *labels) {
     const u64 n_bytes = offs[n_seqs];
     const u64 kmask = (1ull << (2 * k)) - 1ull;
     unsigned long long mine = 0;
@@ -104,8 +116,15 @@ k_contam_build(const uint8_t *__restrict__ seq, const u64 *__restrict__ offs, u3
             const u64 key = roll.key();
             for (u64 i = contam_mix(key) & mask;; i = (i + 1) & mask) {
                 const u64 old = atomicCAS((unsigned long long *)(table + i), CONTAM_EMPTY, key);
-                if (old == CONTAM_EMPTY) { ++mine; break; }
-                if (old == key) break;
+                if (old == CONTAM_EMPTY) {
+                    ++mine;
+                    if (LABELS) contam_label_set(labels + i, r);
+                    break;
+                }
+                if (old == key) {
+                    if (LABELS) contam_label_set(labels + i, r);
+                    break;
+                }
             }
         }
     }
@@ -199,13 +218,17 @@ k_contam_screen(const uint8_t *__restrict__ bases, const ContamChunk *__restrict
     }
 }
 
-// Threshold: contaminant iff hits * 10^6 >= ppm * windows (u64).
+// Threshold: contaminant iff hits * 10^6 >= ppm * windows (u64).  LIST: also append the index of every piece it marks
+// (with `all`, of every screened piece with hits >= 1) to list[*list_n++], the attribution's work list.
+template <bool LIST>
 __global__ void k_contam_decide(tgsf_piece *pieces, const u32 *__restrict__ n_pieces_ptr, u32 cap, int k, u64 ppm,
-                                const u32 *__restrict__ dev_status) {
+                                const u32 *__restrict__ dev_status, u32 *list, u32 *list_n, bool all) {
     const u32 i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= cap || *dev_status != DEV_STATUS_OK || i >= *n_pieces_ptr) return;
     const tgsf_piece p = pieces[i];
     if (p.status != TGSF_PIECE_EMIT || p.len < k) return;
     const u64 windows = (u64)(p.len - k + 1);
-    if ((u64)p.contam_hits * 1000000ull >= ppm * windows) pieces[i].status = TGSF_PIECE_CONTAM;
+    const bool contam = (u64)p.contam_hits * 1000000ull >= ppm * windows;
+    if (contam) pieces[i].status = TGSF_PIECE_CONTAM;
+    if (LIST && (contam || (all && p.contam_hits >= 1))) list[atomicAdd(list_n, 1u)] = i;
 }

@@ -18,6 +18,7 @@
 #include "adapters.cuh"
 #include "common.cuh"
 #include "contam.cuh"
+#include "contam_attr.cuh"
 #include "dust.cuh"
 #include "foldback.cuh"
 #include "kmer.cuh"
@@ -222,6 +223,7 @@ struct DevHeader { // small block mirrored to the host with every batch
     u32 kmer_work;   // k_kmer_tag16: next piece to take
     u32 kmer_long;   // pieces it left for k_kmer_smem (too long for 16-bit positions)
     u32 fold_work, fold_long, fold_long_work; // fold-back screen: next piece, long-list size, next long piece
+    u32 contam_list_n, contam_work;           // contaminant attribution: listed pieces, next listed piece
 };
 
 struct Slot {
@@ -244,6 +246,7 @@ struct Slot {
     DBuf best_mid, mid_n, mid_off, end_n, end_pos, pool, sortbuf, tmp, pieces, res, header;
     DBuf scan_tmp, kmer_long_list, mid_work, gz_blob, gz_spans;
     DBuf contam_cnt, contam_off, contam_chunks; // chunk lists of the contaminant and the DUST screen (only while on)
+    DBuf contam_list;                            // contaminant attribution: pieces to attribute (labelled sets only)
     DBuf dust_masked;                            // DUST screen: masked bases per piece (only while on)
     DBuf fold_long_list, fold_ws;                // fold-back screen (only while enabled)
     Scratch scratch, scratch2; // traceback stores: main stream (k_mid_count) / side stream (k_ends)
@@ -257,11 +260,14 @@ struct Slot {
 // Contaminant k-mer set (tgsf_set_contaminants).
 struct ContamSet {
     DBuf table, pf_bits; // pf_bits: prefilter bitmap, only for sets of <= CONTAM_PF_MAX_KEYS keys
+    DBuf labels, tally;  // labelled sets only: u32 label per table slot; u64 reads[n_records + 1], bases[n_records + 1]
     u64 mask = 0;        // table capacity - 1
     u64 n_keys = 0;
     u64 ppm = 0;
     int k = 0;
+    u32 n_records = 0;
     bool installed() const { return table.p != nullptr; }
+    bool labelled() const { return labels.p != nullptr; }
 };
 
 }  // namespace
@@ -281,6 +287,7 @@ struct tgsf_ctx {
     u32 head = 0, tail = 0, outstanding = 0; // ring: submit at head, collect at tail
     u64 launches = 0;
     int kmer16_ctas_per_sm = 2;
+    int attr_ctas_per_sm = 1; // k_contam_attr<false> CTAs per SM (occupancy): more probes in flight
     int mid_ctas_per_sm = 0; // TGSF_MID_CTAS=n: cap on resident k_mid_scan CTAs per SM (0 = as many as fit)
     int res_ctas_per_sm = 6; // grid of the resolve kernels (k_ends, k_mid_count, k_mid_emit) in CTAs per SM; TGSF_RES_CTAS
     bool fork_ends = true; // TGSF_FORK_ENDS=0: k_ends on the batch's main stream after the middle scan (A/B)
@@ -692,10 +699,11 @@ int launch_kmer(tgsf_ctx *c, Slot &s, const DevParams &P) {
     return check_launch("k_kmer");
 }
 
-// Contaminant screen over the pieces still emitted after K4; writes piece fields only.
-int launch_contam(tgsf_ctx *c, Slot &s) {
+// Contaminant screen of set cs over the pieces still emitted after K4; writes piece fields only.  A labelled set also
+// attributes the pieces: the contaminant ones into the set's tallies, or, with attr_out (tgsf_contam_classify), every
+// piece with a hit into attr_out[piece].
+int launch_contam(tgsf_ctx *c, Slot &s, const ContamSet &cs, int2 *attr_out) {
     cudaStream_t st = s.stream.get();
-    const ContamSet &cs = c->contam;
     DevHeader *H = s.header.as<DevHeader>();
     const u32 cap = s.pieces_cap;
     // pieces are disjoint parts of the reads: at most n_bases / CHUNK full chunks plus one partial chunk per piece
@@ -720,9 +728,27 @@ int launch_contam(tgsf_ctx *c, Slot &s) {
             s.B.bases, s.contam_chunks.as<ContamChunk>(), s.contam_off.as<u32>() + cap, cs.k, cs.table.as<u64>(), cs.mask,
             nullptr, s.pieces.as<tgsf_piece>(), &H->status);
     c->launches++;
-    k_contam_decide<<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap, cs.k, cs.ppm,
-                                                    &H->status);
-    c->launches++;
+    if (!cs.labelled()) {
+        k_contam_decide<false><<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap, cs.k,
+                                                               cs.ppm, &H->status, nullptr, nullptr, false);
+        c->launches++;
+        return check_launch("contam");
+    }
+    TRY(s.contam_list.ensure((size_t)std::max<u32>(cap, 1) * sizeof(u32)));
+    k_contam_decide<true><<<cdiv(cap, 256), 256, 0, st>>>(s.pieces.as<tgsf_piece>(), &H->tmp_cursor, cap, cs.k, cs.ppm,
+                                                          &H->status, s.contam_list.as<u32>(), &H->contam_list_n,
+                                                          attr_out != nullptr);
+    unsigned long long *tally = attr_out ? nullptr : cs.tally.as<unsigned long long>();
+    if (cs.pf_bits.p)
+        k_contam_attr<true><<<c->sm_count, ATTR_THREADS, CONTAM_PF_SMEM_BYTES, st>>>(
+            s.B, s.pieces.as<tgsf_piece>(), s.contam_list.as<u32>(), &H->contam_list_n, &H->contam_work, cs.k,
+            cs.table.as<u64>(), cs.mask, cs.labels.as<u32>(), cs.pf_bits.as<u32>(), cs.n_records, tally, attr_out,
+            &H->status);
+    else
+        k_contam_attr<false><<<c->sm_count * c->attr_ctas_per_sm, ATTR_THREADS, 0, st>>>(
+            s.B, s.pieces.as<tgsf_piece>(), s.contam_list.as<u32>(), &H->contam_list_n, &H->contam_work, cs.k,
+            cs.table.as<u64>(), cs.mask, cs.labels.as<u32>(), nullptr, cs.n_records, tally, attr_out, &H->status);
+    c->launches += 2;
     return check_launch("contam");
 }
 
@@ -837,7 +863,7 @@ int launch_tail(tgsf_ctx *c, Slot &s) {
         if (c->foldback)
             TRY(launch_fold(c, s, s.pieces.as<tgsf_piece>(), &H->tmp_cursor, H, nullptr, P.L.max_bins * SCAN_BIN));
         if (P.min_repeat > 0) TRY(launch_kmer(c, s, P));
-        if (c->contam.installed()) TRY(launch_contam(c, s));
+        if (c->contam.installed()) TRY(launch_contam(c, s, c->contam, nullptr));
         if (c->dust_level) TRY(launch_dust(c, s, c->dust_level, c->dust_ppm));
         CU(cudaEventRecord(s.ev_stage[6].get(), st));
         // clean pass over the kept pieces (T.cpp:1991-2009); piece count is device-side, the
@@ -1070,10 +1096,13 @@ int tgsf_create(int device, const tgsf_params *params, tgsf_ctx **out) {
     CU(smem(k_kmer_smem, KMER_SB_SMEM_BYTES));
     CU(smem(k_kmer_tag16, KMER16_SMEM_BYTES));
     CU(smem(k_contam_screen<true>, CONTAM_PF_SMEM_BYTES));
+    CU(smem(k_contam_attr<true>, CONTAM_PF_SMEM_BYTES));
     CU(smem(k_fold_smem, FOLD_SMEM_BYTES));
     int occ = 0;
     if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_kmer_tag16, KMER16_THREADS, KMER16_SMEM_BYTES) == cudaSuccess && occ >= 1)
         c->kmer16_ctas_per_sm = occ;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_contam_attr<false>, ATTR_THREADS, 0) == cudaSuccess && occ >= 1)
+        c->attr_ctas_per_sm = occ;
     if (const char *e = getenv("TGSF_MID_CTAS")) c->mid_ctas_per_sm = atoi(e);
     if (const char *e = getenv("TGSF_FORK_ENDS")) c->fork_ends = atoi(e) != 0;
     if (const char *e = getenv("TGSF_RES_CTAS")) c->res_ctas_per_sm = std::max(1, std::min(16, atoi(e)));
@@ -1094,10 +1123,14 @@ int tgsf_destroy(tgsf_ctx *c) {
     return TGSF_OK;
 }
 
-int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs, int32_t k,
-                          float min_frac, uint64_t *n_kmers) {
-    if (!c || !offsets || !n_kmers || n_seqs == 0) { set_err("tgsf_set_contaminants: missing argument"); return TGSF_ERR_INVALID; }
-    if (c->outstanding) { set_err("tgsf_set_contaminants with %u batch(es) outstanding", c->outstanding); return TGSF_ERR_STATE; }
+// tgsf_set_contaminants, and with record_kmers tgsf_set_contaminants_labelled: the labels, their key counts and zeroed
+// tallies besides the table.
+static int install_contaminants(const char *fn, tgsf_ctx *c, const uint8_t *seq, const uint64_t *offsets,
+                                uint32_t n_seqs, int32_t k, float min_frac, uint64_t *n_kmers, uint64_t *record_kmers) {
+    const bool labelled = record_kmers != nullptr;
+    if (!c || !offsets || !n_kmers || n_seqs == 0) { set_err("%s: missing argument", fn); return TGSF_ERR_INVALID; }
+    if (c->outstanding) { set_err("%s with %u batch(es) outstanding", fn, c->outstanding); return TGSF_ERR_STATE; }
+    if (labelled && n_seqs > TGSF_CONTAM_MAX_RECORDS) { set_err("%s: more than %u records", fn, TGSF_CONTAM_MAX_RECORDS); return TGSF_ERR_INVALID; }
     if (k < CONTAM_K_MIN || k > CONTAM_K_MAX) { set_err("contaminant k must be in [%d,%d], got %d", CONTAM_K_MIN, CONTAM_K_MAX, k); return TGSF_ERR_INVALID; }
     const double fd = (double)min_frac;
     const long long ppm = fd == fd && fd >= 0.0 && fd <= 2.0 ? llround(fd * 1e6) : -1;
@@ -1116,6 +1149,10 @@ int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offse
     ContamSet next;
     DBuf d_seq, d_off, d_cnt;
     TRY(next.table.ensure(cap * sizeof(u64)));
+    if (labelled) {
+        TRY(next.labels.ensure(cap * sizeof(u32)));
+        CU(cudaMemsetAsync(next.labels.p, 0xFF, cap * sizeof(u32), st));
+    }
     TRY(d_seq.ensure(n_bytes));
     TRY(d_off.ensure(((size_t)n_seqs + 1) * sizeof(u64)));
     TRY(d_cnt.ensure(sizeof(unsigned long long)));
@@ -1125,8 +1162,12 @@ int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offse
     CU(cudaMemcpyAsync(d_off.p, offsets, ((size_t)n_seqs + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
     const u64 threads = (n_bytes + CONTAM_BUILD_SEG - 1) / CONTAM_BUILD_SEG;
     const u32 grid = (u32)std::min<u64>((threads + 255) / 256, (u64)c->sm_count * 16);
-    k_contam_build<<<grid, 256, 0, st>>>(d_seq.as<uint8_t>(), d_off.as<u64>(), n_seqs, k, next.table.as<u64>(),
-                                         cap - 1, d_cnt.as<unsigned long long>());
+    if (labelled)
+        k_contam_build<true><<<grid, 256, 0, st>>>(d_seq.as<uint8_t>(), d_off.as<u64>(), n_seqs, k, next.table.as<u64>(),
+                                                   cap - 1, d_cnt.as<unsigned long long>(), next.labels.as<u32>());
+    else
+        k_contam_build<false><<<grid, 256, 0, st>>>(d_seq.as<uint8_t>(), d_off.as<u64>(), n_seqs, k, next.table.as<u64>(),
+                                                    cap - 1, d_cnt.as<unsigned long long>(), nullptr);
     c->launches++;
     TRY(check_launch("k_contam_build"));
     unsigned long long n = 0;
@@ -1143,11 +1184,83 @@ int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offse
         TRY(check_launch("k_contam_bitmap"));
         CU(cudaStreamSynchronize(st));
     }
+    std::vector<u64> rk;
+    if (labelled) {
+        const size_t rows = (size_t)n_seqs + 1;
+        DBuf d_rk;
+        TRY(d_rk.ensure(rows * sizeof(u64)));
+        TRY(next.tally.ensure(2 * rows * sizeof(u64)));
+        CU(cudaMemsetAsync(d_rk.p, 0, rows * sizeof(u64), st));
+        CU(cudaMemsetAsync(next.tally.p, 0, next.tally.cap, st));
+        k_contam_label_count<<<(u32)std::min<u64>(cap / 256, (u64)c->sm_count * 8), 256, 0, st>>>(
+            next.table.as<u64>(), next.labels.as<u32>(), cap, n_seqs, d_rk.as<unsigned long long>());
+        c->launches++;
+        TRY(check_launch("k_contam_label_count"));
+        rk.resize(rows);
+        CU(cudaMemcpyAsync(rk.data(), d_rk.p, rows * sizeof(u64), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        next.n_records = n_seqs;
+    }
     next.mask = cap - 1;
     next.ppm = (u64)ppm;
     next.k = k;
     c->contam = std::move(next); // frees the set it replaces
     *n_kmers = c->contam.n_keys;
+    if (labelled) memcpy(record_kmers, rk.data(), rk.size() * sizeof(u64));
+    return TGSF_OK;
+}
+
+int tgsf_set_contaminants(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs, int32_t k,
+                          float min_frac, uint64_t *n_kmers) {
+    return install_contaminants("tgsf_set_contaminants", c, seq, offsets, n_seqs, k, min_frac, n_kmers, nullptr);
+}
+
+int tgsf_set_contaminants_labelled(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offsets, uint32_t n_seqs,
+                                   int32_t k, float min_frac, uint64_t *n_kmers, uint64_t *record_kmers) {
+    if (!record_kmers) { set_err("tgsf_set_contaminants_labelled: missing argument"); return TGSF_ERR_INVALID; }
+    return install_contaminants("tgsf_set_contaminants_labelled", c, seq, offsets, n_seqs, k, min_frac, n_kmers,
+                                record_kmers);
+}
+
+int tgsf_contam_record_stats(tgsf_ctx *c, uint64_t *reads, uint64_t *bases, uint32_t n) {
+    if (!c || !reads || !bases) { set_err("tgsf_contam_record_stats: NULL argument"); return TGSF_ERR_INVALID; }
+    if (!c->contam.labelled()) { set_err("tgsf_contam_record_stats: the installed contaminant set has no labels"); return TGSF_ERR_INVALID; }
+    if ((u64)n != (u64)c->contam.n_records + 1) {
+        set_err("tgsf_contam_record_stats: n must be n_seqs + 1 = %llu, got %u", (unsigned long long)c->contam.n_records + 1, n);
+        return TGSF_ERR_INVALID;
+    }
+    if (c->outstanding) { set_err("collect all batches first"); return TGSF_ERR_STATE; }
+    CU(cudaSetDevice(c->device));
+    const u64 *T = c->contam.tally.as<u64>();
+    CU(cudaMemcpy(reads, T, (size_t)n * sizeof(u64), cudaMemcpyDeviceToHost));
+    CU(cudaMemcpy(bases, T + n, (size_t)n * sizeof(u64), cudaMemcpyDeviceToHost));
+    return TGSF_OK;
+}
+
+int tgsf_contam_classify(tgsf_ctx *c, const uint8_t *seq, const uint64_t *offsets, uint32_t n, tgsf_contam_class *out) {
+    if (!c) { set_err("tgsf_contam_classify: ctx is NULL"); return TGSF_ERR_INVALID; }
+    if (c->outstanding) { set_err("tgsf_contam_classify with %u batch(es) outstanding", c->outstanding); return TGSF_ERR_STATE; }
+    if (!c->contam.labelled()) { set_err("tgsf_contam_classify: no labelled contaminant set installed"); return TGSF_ERR_STATE; }
+    if (n == 0) return TGSF_OK;
+    if (!offsets || !out) { set_err("tgsf_contam_classify: NULL argument"); return TGSF_ERR_INVALID; }
+    RecordPieces R;
+    TRY(R.setup("tgsf_contam_classify", c->device, seq, offsets, n));
+    Slot &s = R.slot();
+    DBuf d_out;
+    TRY(d_out.ensure((size_t)n * sizeof(int2)));
+    CU(cudaMemsetAsync(d_out.p, 0xFF, (size_t)n * sizeof(int2), s.stream.get())); // record -1: not attributed
+    TRY(launch_contam(R.c.get(), s, c->contam, d_out.as<int2>()));
+    std::vector<tgsf_piece> pc((size_t)n);
+    std::vector<int2> attr((size_t)n);
+    CU(cudaMemcpyAsync(pc.data(), s.pieces.p, (size_t)n * sizeof(tgsf_piece), cudaMemcpyDeviceToHost, s.stream.get()));
+    CU(cudaMemcpyAsync(attr.data(), d_out.p, (size_t)n * sizeof(int2), cudaMemcpyDeviceToHost, s.stream.get()));
+    TRY(R.finish("tgsf_contam_classify"));
+    for (uint32_t i = 0; i < n; ++i) {
+        out[i].hits = pc[i].contam_hits;
+        out[i].record = attr[i].x;
+        out[i].record_hits = attr[i].x < 0 ? 0 : attr[i].y;
+        out[i].contam = pc[i].status == TGSF_PIECE_CONTAM ? 1 : 0;
+    }
     return TGSF_OK;
 }
 
@@ -1582,6 +1695,7 @@ int tgsf_counters_reset(tgsf_ctx *c) {
     CU(cudaSetDevice(c->device));
     CU(cudaMemset(c->counters.p, 0, (size_t)c->P.L.n_u64 * sizeof(u64)));
     if (c->fold_stats.p) CU(cudaMemset(c->fold_stats.p, 0, 4 * sizeof(u64)));
+    if (c->contam.labelled()) CU(cudaMemset(c->contam.tally.p, 0, c->contam.tally.cap));
     return TGSF_OK;
 }
 

@@ -86,6 +86,43 @@ class FilterEngine:
                                                      min_frac, C.byref(n)), "tgsf_set_contaminants")
         return int(n.value)
 
+    def set_contaminants_labelled(self, seqs, k: int = 17, min_frac: float = 0.05) -> Tuple[int, np.ndarray]:
+        """tgsf_set_contaminants_labelled: set_contaminants that also attributes every later contaminant piece to the
+        record it matches.  Returns (distinct canonical k-mers, keys per record with the shared keys last: u64[n + 1])."""
+        recs = [s.encode() if isinstance(s, str) else bytes(s) for s in seqs]
+        offs = np.zeros(len(recs) + 1, dtype=np.uint64)
+        np.cumsum([len(r) for r in recs], out=offs[1:])
+        buf = np.frombuffer(b"".join(recs) + b"\0", dtype=np.uint8)
+        n = C.c_uint64(0)
+        rk = np.zeros(len(recs) + 1, dtype=np.uint64)
+        _capi.check(self._lib.tgsf_set_contaminants_labelled(self._ctx, buf.ctypes.data, offs.ctypes.data, len(recs),
+                                                              k, min_frac, C.byref(n), rk.ctypes.data),
+                    "tgsf_set_contaminants_labelled")
+        self._contam_records = len(recs)
+        return int(n.value), rk
+
+    def contam_record_stats(self, n_records: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """tgsf_contam_record_stats: (reads, bases) u64[n + 1] of the contaminant pieces per record, shared row last,
+        cumulative since the labelled set was installed or the counters were reset."""
+        n = (getattr(self, "_contam_records", 0) if n_records is None else n_records) + 1
+        reads = np.zeros(n, dtype=np.uint64)
+        bases = np.zeros(n, dtype=np.uint64)
+        _capi.check(self._lib.tgsf_contam_record_stats(self._ctx, reads.ctypes.data, bases.ctypes.data, n),
+                    "tgsf_contam_record_stats")
+        return reads, bases
+
+    def contam_classify(self, seqs) -> np.ndarray:
+        """tgsf_contam_classify on stand-alone pieces (bytes / str) against the installed labelled set: one
+        (hits, record, record_hits, contam) row per piece."""
+        recs = [s.encode() if isinstance(s, str) else bytes(s) for s in seqs]
+        offs = np.zeros(len(recs) + 1, dtype=np.uint64)
+        np.cumsum([len(r) for r in recs], out=offs[1:])
+        buf = np.frombuffer(b"".join(recs) + b"\0", dtype=np.uint8)
+        out = np.zeros(len(recs), dtype=_capi.CONTAM_CLASS_DTYPE)
+        _capi.check(self._lib.tgsf_contam_classify(self._ctx, buf.ctypes.data, offs.ctypes.data, len(recs),
+                                                    out.ctypes.data), "tgsf_contam_classify")
+        return out
+
     # -- fold-back screen ------------------------------------------------------------------------
     def set_foldback(self, enable: bool = True) -> None:
         """tgsf_set_foldback: cut every later batch's pieces at a fold-back junction (keep the longer arm)."""
